@@ -2,10 +2,21 @@
 """Benchmark of the hot path: land-sea mask -> RCB boxes + pid labels + neighbours / halos.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one complete decomposition (ddc_partition with pid + neighbour tables) of the
 workload's synthetic mask.  With N > 1 (torchrun, one rank per GPU) the SAME mask is row-sharded
 over the ranks (strong scaling) and the histograms are combined with NCCL inside the step.
+Every timed loop runs K steps.
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (float32 where that is
+exact, else float64): boxes [P, 4] (x0, y0, ext_x, ext_y), part_loads [P], neighbour_counts
+[2, 4, P] (periodic, edge in the order left, right, bottom, top, part), neighbours [n, 6] with one row
+(periodic, edge, part, neighbour id, halo, halo start) per entry of the neighbour tables, in the order of
+the metadata file, and the pid map: whole as pid [ny, nx] up to PID_DUMP_CELLS cells, else a fixed
+seeded sample pid_sample at the flat indices y * nx + x in pid_sample_index.  (One array for all tables:
+the tables of an edge without periodic neighbours are empty.)  The mask comes from the workload's seed,
+so two builds run with the same arguments can be compared array for array.
 
   value       whole-job mask cells partitioned per second, mask already resident in HBM
   e2e         same metric through the C ABI with HOST buffers: pinned-host -> device copy of the
@@ -16,7 +27,8 @@ over the ranks (strong scaling) and the histograms are combined with NCCL inside
 
 `--impl reference` times the reference algorithm's CPU port (oracle/, OpenMP tasks over all host
 cores) on a bounded sample of the same workload; the reference binary itself needs MPI + Zoltan +
-parallel netCDF + Boost, none of which exist in this image (see DESIGN.md).
+parallel netCDF + Boost, none of which exist in this image (see DESIGN.md).  It runs K steps too, and
+one step of the whole default workload takes tens of seconds: pass --steps 1 for a quick number.
 """
 from __future__ import annotations
 
@@ -47,6 +59,9 @@ GOLDEN_DIGESTS = os.path.join(ROOT, "tests", "golden", "bench_digests.json")
 DEFAULT_WORKLOAD = "C5_32768x32768_p16384"
 L2_BYTES = 126 * 1000 * 1000
 ALGO_BYTES_PER_CELL = 8  # 4 B int32 mask read + 4 B int32 pid write (SURVEY 8d)
+PID_DUMP_CELLS = 1 << 20  # --dump-outputs: pid maps larger than this are sampled (12 B per sampled cell)
+DUMP_SEED = 20251020
+DUMP_MAX_BYTES = 64 * 1000 * 1000
 
 
 def measured_peak_gbs():
@@ -136,6 +151,55 @@ class _DevArray:
                                          "version": 2, "strides": None}
 
 
+def _exact_float(a):
+    """int array -> float32 when every value is exact in it, else float64"""
+    import numpy as np
+    a = np.asarray(a)
+    return a.astype(np.float32 if a.size == 0 or int(np.abs(a).max()) < (1 << 24) else np.float64)
+
+
+def dump_outputs(h, out_dir, d_pid, nx, ny, y_begin, y_count, dev, world, rank):
+    """--dump-outputs: the results of the handle's last decomposition as DIR/<name>.npy (see the module doc).
+    Every rank calls the same getters; the pid rows of all ranks are combined, rank 0 writes."""
+    import numpy as np
+    import torch
+    from domain_decomp_b200 import capi
+    out = {"boxes": h.boxes(), "part_loads": h.part_loads()}
+    counts, rows = np.zeros((2, 4, h.nparts), dtype=np.int64), []
+    for per in range(2):
+        for e in range(len(capi.EDGE_NAMES)):
+            counts[per, e] = h.neighbour_counts(e, per)
+            ids, halos, starts = h.neighbours(e, per)
+            part = np.repeat(np.arange(h.nparts), counts[per, e])
+            rows.append(np.stack([np.full(ids.size, per), np.full(ids.size, e), part, ids, halos, starts], axis=1))
+    out["neighbour_counts"], out["neighbours"] = counts, np.concatenate(rows)
+    cells = nx * ny
+    whole = cells <= PID_DUMP_CELLS
+    idx = (np.arange(cells, dtype=np.int64) if whole else
+           np.unique(np.random.default_rng(DUMP_SEED).integers(0, cells, size=PID_DUMP_CELLS)))
+    g = torch.from_numpy(idx).to(dev)
+    lo = y_begin * nx
+    mine = (g >= lo) & (g < lo + y_count * nx)
+    vals = torch.zeros(idx.size, dtype=torch.int64, device=dev)
+    vals[mine] = d_pid.reshape(-1)[g[mine] - lo].long()
+    if world > 1:
+        torch.distributed.all_reduce(vals)  # every sampled cell lies in the rows of exactly one rank
+    if whole:
+        out["pid"] = vals.cpu().numpy().reshape(ny, nx)
+    else:
+        out["pid_sample"], out["pid_sample_index"] = vals.cpu().numpy(), idx
+    if rank != 0:
+        return
+    # the sample's flat indices exceed float32's exact range: float64, exact below 2**53
+    arrays = {k: v.astype(np.float64) if k == "pid_sample_index" else _exact_float(v) for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def plugin_e2e(mask, expect_pid, expect_boxes_soa, nx, ny, P, px, py, gpus, reps):
     """CudaRcbPartitioner::partition through libdomain_decomp.so's ddc_plugin_bench (host/PluginBench.cpp)"""
     import ctypes as C
@@ -208,12 +272,9 @@ def reference_arm(args):
     whole = args.sample == "whole" or (args.sample == "auto" and avail > need)
     t0 = time.perf_counter()
     mask, sp, px, py, desc = cpu_sample(args.workload, threads, whole=whole)
-    # keep the whole run within a few minutes whatever K is: the first decomposition is timed and sizes the rest
-    # (a CPU pass over a fresh mask has nothing to warm up: every step counts)
-    first = run_cpu(mask, sp, px, py, threads, 1, 0)
-    budget = 120.0
-    steps, warmup = max(1, min(args.steps, int(budget / max(first, 1e-3)))), 0
-    sec = first if steps == 1 else (first + run_cpu(mask, sp, px, py, threads, steps - 1, 0) * (steps - 1)) / steps
+    # a CPU pass over a fresh mask has nothing to warm up: every step counts
+    steps, warmup = args.steps, 0
+    sec = run_cpu(mask, sp, px, py, threads, steps, warmup)
     value = mask.size / sec
     same_config = mask.shape == (ny, nx) and sp == P
     line = {
@@ -236,7 +297,8 @@ def reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every timed loop (--impl reference: tens of seconds per step on the default workload)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -247,7 +309,13 @@ def main():
                     help="--impl reference: the whole workload (when the host memory allows: auto) or the bounded window")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="multi-GPU exchange: stores into the peers' memory from inside the kernels (default) or NCCL collectives")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -286,7 +354,7 @@ def main():
 
     nx, ny, P, land, seed, px, py = WORKLOADS[args.workload]
     cells = nx * ny
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     h = capi.Handle(local_rank, rank, world, nccl_id)
     if world > 1 and args.exchange == "peer":
         handles = [None] * world
@@ -338,6 +406,10 @@ def main():
     ms_per_step = max_over_ranks(total_ms / K)
     value = cells / (ms_per_step * 1e-3)
     st = h.stats()
+    if args.dump_outputs:
+        d_pid = torch.as_tensor(_DevArray(h.pid_device(), (max(y_count, 1), nx)), device=dev)[:y_count]
+        dump_outputs(h, args.dump_outputs, d_pid, nx, ny, y_begin, y_count, dev, world, rank)
+        del d_pid
 
     # ---- per-kernel timing (CUDA events on the launching stream, inside ddc_partition) --------
     stage = {k: 0.0 for k in capi.STAGE_NAMES}
@@ -405,7 +477,6 @@ def main():
         h_pid = torch.empty((max(y_count, 1), nx), dtype=torch.int32, pin_memory=True)
         h_mask.copy_(d_mask)  # the same synthetic mask, now living in pinned host memory
         torch.cuda.synchronize()
-        ke = max(1, min(K, 10))
 
         def e2e_step():
             h.set_mask_host_ptr(h_mask.data_ptr(), nx, ny, y_begin, y_count)  # H2D
@@ -425,15 +496,15 @@ def main():
         t0 = time.perf_counter()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        for _ in range(ke):
+        for _ in range(K):
             e2e_step()
         e1.record(stream)
         torch.cuda.synchronize()
-        wall = (time.perf_counter() - t0) * 1e3 / ke
-        ev_ms = e0.elapsed_time(e1) / ke
+        wall = (time.perf_counter() - t0) * 1e3 / K
+        ev_ms = e0.elapsed_time(e1) / K
         barrier()
         e2e_ms = max_over_ranks(max(wall, ev_ms))
-        e2e = {"value": cells / (e2e_ms * 1e-3), "unit": "cells/s", "ms_per_step": e2e_ms, "steps": ke,
+        e2e = {"value": cells / (e2e_ms * 1e-3), "unit": "cells/s", "ms_per_step": e2e_ms, "steps": K,
                "h2d_bytes_per_step": shard_bytes * world if world > 1 else shard_bytes,
                "d2h_bytes_per_step": (shard_bytes + small) * world if world > 1 else shard_bytes + small,
                "path": "C ABI (ddc_set_mask_host, ddc_partition, ddc_get_pid_host, table getters), one process per GPU",
@@ -462,7 +533,7 @@ def main():
         if rank == 0:
             try:
                 plugin = plugin_e2e(np.ascontiguousarray(g_mask), np.ascontiguousarray(g_pid), boxes_soa, nx, ny, P, px, py,
-                                    world, max(1, min(ke, 5)))
+                                    world, K)
             except Exception as exc:  # the C ABI number stands
                 plugin = {"error": str(exc)}
         if world > 1:

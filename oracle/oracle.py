@@ -22,13 +22,17 @@ EDGES = ("left", "right", "bottom", "top")  # DomainUtils.hpp:15 enum order L,R,
 
 
 def build(force: bool = False) -> str:
-    """Compile the C restatement (and oracle/_ref when the reference checkout exists)."""
+    """Compile the C restatement, the emulation libraries and the host-layer test binaries; with
+    DDC_REFERENCE_DIR naming a checkout of the reference, also its own sources into oracle/_ref."""
     src = os.path.join(_HERE, "ddc_oracle.c")
     if force or not os.path.exists(_LIB) or os.path.getmtime(_LIB) < os.path.getmtime(src):
         subprocess.check_call(["make", "-s", "-C", _HERE, "libddc_oracle.so"])
-    subprocess.check_call(["make", "-s", "-j4", "-C", _HERE, "libddc_median_emu.so", "libddc_emu.so", "libddc_cuda_emu.so"])  # make decides what is stale
-    if os.path.isdir("/root/reference"):  # make decides what is stale
-        subprocess.check_call(["make", "-s", "-j4", "-C", _HERE, "ref"] + (["-B"] if force else []))
+    # make decides what is stale
+    subprocess.check_call(["make", "-s", "-j4", "-C", _HERE, "libddc_median_emu.so", "libddc_emu.so", "libddc_cuda_emu.so", "hostcpu"]
+                          + (["-B"] if force else []))
+    ref = os.environ.get("DDC_REFERENCE_DIR")
+    if ref:
+        subprocess.check_call(["make", "-s", "-j4", "-C", _HERE, "ref", "REF=" + os.path.abspath(ref)] + (["-B"] if force else []))
     return _LIB
 
 
@@ -226,7 +230,7 @@ def ref_host_run(mask: np.ndarray, P: int, px: bool = False, py: bool = False, *
       files[name] = {dims: [(name, len)], atts: {..}, vars: {(group, name): (dims, values)}, unwritten: {..}}"""
     L = ref_host_lib()
     if L is None:
-        raise RuntimeError("oracle/_ref/libref_hostpath.so is not built (needs /root/reference)")
+        raise RuntimeError("oracle/_ref/libref_hostpath.so is not built (needs DDC_REFERENCE_DIR)")
     mask = np.ascontiguousarray(mask, dtype=np.int32)
     ny, nx = mask.shape
     b = None if boxes is None else np.ascontiguousarray(boxes, dtype=np.int32)

@@ -9,7 +9,9 @@ arbitrary inputs, not only on the five goldens:
   the code around the Zoltan call: P == 1 shortcut, box clamp, labels (ZoltanPartitioner.cpp:96-121,172-219)
   discover_neighbours / is_neighbour / halo_start / domain_overlap   (Partitioner.cpp:20-80,329-435)
   get_neighbour_info[_periodic], save_mask, save_metadata            (Partitioner.cpp:98-318)
-CPU only.  Skipped where the reference checkout (hence oracle/_ref) is absent."""
+CPU only.  Where the reference checkout (hence oracle/_ref) is absent, the comparisons run against the answers stored
+in tests/golden/reference_answers.json (tests/reference_answers.py); the tests whose subject is the reference's
+code itself skip."""
 import os
 import subprocess
 
@@ -17,6 +19,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, golden_mask
+from reference_answers import Answers
 
 EDGES = ("left", "right", "bottom", "top")
 
@@ -26,6 +29,12 @@ def ref(oracle):
     if oracle.ref_host_lib() is None:
         pytest.skip("oracle/_ref/libref_hostpath.so not built (no reference checkout here)")
     return oracle
+
+
+@pytest.fixture(scope="module")
+def live(oracle):
+    """True where oracle/_ref is built: the live comparison with the reference's code runs beside the stored answers"""
+    return oracle.ref_host_lib() is not None
 
 
 def boxes_of(md):
@@ -60,9 +69,11 @@ def sane_blocks(oracle, P, nx, ny):
     return all(b[2] >= 1 and b[3] >= 1 for b in (oracle.naive_block(P, nx, ny, r) for r in range(P)))
 
 
-def test_grid_against_reference_grid(ref):
+def test_grid_against_reference_grid(oracle, live):
     """Grid::create on P ranks: block, counts, slab, global ids -- the reference vs the oracle's naive
     blocks vs plain numpy"""
+    ref = oracle
+    answers = Answers("test_reference_hostpath::test_grid_against_reference_grid", live)
     rng = np.random.default_rng(17)
     checked = 0
     while checked < 60:
@@ -70,6 +81,10 @@ def test_grid_against_reference_grid(ref):
         if not sane_blocks(ref, P, nx, ny):
             continue
         mask = (rng.random((ny, nx)) < rng.random()).astype(np.int32) * rng.integers(1, 4, size=(ny, nx)).astype(np.int32)
+        answers.check([ref.naive_block(P, nx, ny, rank) for rank in range(P)], (nx, ny, P))
+        checked += 1
+        if not live:
+            continue
         r = ref.ref_host_run(mask, P)
         for rank, got in enumerate(r["ranks"]):
             x0, y0, ex, ey = ref.naive_block(P, nx, ny, rank)
@@ -79,7 +94,7 @@ def test_grid_against_reference_grid(ref):
             assert got["mask"] == slab.ravel().tolist()
             yy, xx = np.nonzero(slab > 0)
             assert got["ids"] == ((yy + y0) * nx + xx + x0).tolist()
-        checked += 1
+    answers.finish()
 
 
 def test_grid_dimension_names_order_and_group(ref):
@@ -107,13 +122,19 @@ def per_part(nbr, P, per, e):
     return [[(int(ids[k]), int(halos[k]), int(starts[k])) for k in range(off[p], off[p + 1])] for p in range(P)]
 
 
-def check_against_oracle(ref, mask, P, px, py):
+def check_against_oracle(ref, mask, P, px, py, answers, live):
+    """the oracle's decomposition is the stored answer of this case and, where oracle/_ref is built (`live`), what the
+    reference's own neighbour discovery and writers give back for its boxes and owners"""
     ny, nx = mask.shape
     o = ref.partition(mask, P, px, py, use_hist=True)
     boxes = o.boxes if o.changes else np.asarray([ref.naive_block(P, nx, ny, r) for r in range(P)], dtype=np.int32)
     assert o.boxes.tolist() == boxes.tolist()  # the oracle already reports the naive blocks when nothing moved
-    r = ref.ref_host_run(mask, P, px, py, boxes=o.boxes, pid=o.pid, changes=o.changes)
     ctx = (nx, ny, P, px, py)
+    answers.check({"boxes": o.boxes, "pid": o.pid, "changes": o.changes, "counts": o.nbr.counts, "ids": o.nbr.ids,
+                   "halos": o.nbr.halos, "starts": o.nbr.starts}, ctx)
+    if not live:
+        return
+    r = ref.ref_host_run(mask, P, px, py, boxes=o.boxes, pid=o.pid, changes=o.changes)
     for p in range(P):
         assert r["ranks"][p]["box"] == o.boxes[p].tolist(), ctx
         for per in range(2):
@@ -141,9 +162,11 @@ def check_against_oracle(ref, mask, P, px, py):
     assert not r["files"]["mask"]["unwritten"]
 
 
-def test_neighbours_and_files_against_reference_code_random(ref):
+def test_neighbours_and_files_against_reference_code_random(oracle, live):
     """random coastlines, 1 .. 24 parts, all periodic combinations: the oracle's boxes / owners go through the
     reference's own neighbour discovery and writers and must come back as the oracle's tables"""
+    ref = oracle
+    answers = Answers("test_reference_hostpath::test_neighbours_and_files_against_reference_code_random", live)
     rng = np.random.default_rng(23)
     done = 0
     while done < 120:
@@ -153,20 +176,25 @@ def test_neighbours_and_files_against_reference_code_random(ref):
         land = rng.random() * 0.8
         mask = (rng.random((ny, nx)) >= land).astype(np.int32)
         px, py = bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
-        check_against_oracle(ref, mask, P, px, py)
+        check_against_oracle(ref, mask, P, px, py, answers, live)
         done += 1
+    answers.finish()
 
 
-def test_nothing_moved_and_all_land_against_reference_code(ref):
+def test_nothing_moved_and_all_land_against_reference_code(oracle, live):
     """`changes == 0`: the reference reports the naive blocks and finds THEIR neighbours"""
+    answers = Answers("test_reference_hostpath::test_nothing_moved_and_all_land_against_reference_code", live)
     for (n, P) in [(64, 4), (60, 6), (96, 16)]:
-        check_against_oracle(ref, np.ones((n, n), dtype=np.int32), P, True, True)
-    check_against_oracle(ref, np.zeros((12, 18), dtype=np.int32), 6, False, True)
-    check_against_oracle(ref, np.zeros((4, 6), dtype=np.int32), 2, False, False)  # test_zoltan_partitioner_0.cpp:39-66
+        check_against_oracle(oracle, np.ones((n, n), dtype=np.int32), P, True, True, answers, live)
+    check_against_oracle(oracle, np.zeros((12, 18), dtype=np.int32), 6, False, True, answers, live)
+    check_against_oracle(oracle, np.zeros((4, 6), dtype=np.int32), 2, False, False, answers, live)  # test_zoltan_partitioner_0.cpp:39-66
+    answers.finish()
 
 
-def test_host_library_grid_matches_reference_grid(ref, tmp_path):
+def test_host_library_grid_matches_reference_grid(oracle, live, tmp_path):
     """this repository's Grid (host library, through nc_tool on a classic netCDF file) == the reference's Grid"""
+    ref = oracle
+    answers = Answers("test_reference_hostpath::test_host_library_grid_matches_reference_grid", live)
     scipy_io = pytest.importorskip("scipy.io")
     from domain_decomp_b200 import build
     build.build_all()
@@ -181,22 +209,28 @@ def test_host_library_grid_matches_reference_grid(ref, tmp_path):
         f.createDimension("y", ny)
         f.createVariable("mask", "i4", ("y", "x"))[:] = mask
         f.close()
-        r = ref.ref_host_run(mask, P)
+        r = ref.ref_host_run(mask, P) if live else None
         for rank in range(P):
             out = subprocess.run([tool, "grid", path, "x", "y", "yx", "mask", "ranks", str(P), str(rank)],
                                  capture_output=True, text=True, timeout=60)
             assert out.returncode == 0, out.stderr
             lines = dict(l.split(" ", 1) for l in out.stdout.strip().splitlines())
+            answers.check({k: lines[k] for k in ("block", "objects", "mask")}, (nx, ny, P, rank))
+            if not live:
+                continue
             got = r["ranks"][rank]
             assert list(map(int, lines["block"].split())) == got["block"]
             assert lines["objects"] == "%d nonzero %d" % (got["objects"], got["nonzero"])
             assert list(map(int, lines["mask"].split())) == got["mask"]
+    answers.finish()
 
 
 @pytest.mark.parametrize("px,py", [(0, 0), (1, 1)])
-def test_arctic25km_64_parts_against_reference_code(ref, px, py):
+def test_arctic25km_64_parts_against_reference_code(oracle, live, px, py):
     """BASELINE config 2 (528 x 522 synthetic coastline, 64 parts) on 64 thread-ranks of reference code"""
+    answers = Answers("test_reference_hostpath::test_arctic25km_64_parts_against_reference_code[%d-%d]" % (px, py), live)
     from domain_decomp_b200 import capi
     mask = capi.generate_mask_host(528, 522, 25, 0.45)
-    assert sane_blocks(ref, 64, 528, 522)
-    check_against_oracle(ref, mask, 64, bool(px), bool(py))
+    assert sane_blocks(oracle, 64, 528, 522)
+    check_against_oracle(oracle, mask, 64, bool(px), bool(py), answers, live)
+    answers.finish()

@@ -30,6 +30,8 @@ SYMBOLS = (
     "ddc_get_neighbour_total", "ddc_get_neighbours", "ddc_get_part_loads", "ddc_get_stats",
     "ddc_neighbours_from_boxes", "ddc_generate_mask_device", "ddc_generate_mask_host", "ddc_version",
     "ddc_peer_export", "ddc_peer_import", "ddc_peer_close", "ddc_host_alloc", "ddc_host_free", "ddc_peer_connect", "ddc_halo_tile_offsets", "ddc_halo_exchange_f64",
+    "ddc_shard_parts", "ddc_halo_shard_offsets", "ddc_halo_export", "ddc_halo_import", "ddc_halo_connect",
+    "ddc_halo_exchange_shards_f64", "ddc_halo_close",
 )
 
 
@@ -96,6 +98,14 @@ def load() -> C.CDLL:
     L.ddc_neighbours_from_boxes.argtypes = [vp, i32, i32, i32, vp, vp, vp, vp, i32, i32]
     L.ddc_halo_tile_offsets.argtypes = [vp, vp]
     L.ddc_halo_exchange_f64.argtypes = [vp, vp, i32]
+    L.ddc_shard_parts.argtypes = [i32, i32, i32, C.POINTER(i32), C.POINTER(i32)]
+    L.ddc_shard_parts.restype = None
+    L.ddc_halo_shard_offsets.argtypes = [vp, vp]
+    L.ddc_halo_export.argtypes = [vp, C.c_int64, C.POINTER(vp), vp]
+    L.ddc_halo_import.argtypes = [vp, vp]
+    L.ddc_halo_connect.argtypes = [C.POINTER(vp), i32, C.c_int64, C.POINTER(vp)]
+    L.ddc_halo_exchange_shards_f64.argtypes = [vp, i32]
+    L.ddc_halo_close.argtypes = [vp]
     L.ddc_generate_mask_device.argtypes = [vp, vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     L.ddc_generate_mask_host.argtypes = [vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     _lib = L
@@ -106,6 +116,26 @@ def shard_rows(ny: int, nranks: int, rank: int):
     b, c = C.c_int(), C.c_int()
     load().ddc_shard_rows(ny, nranks, rank, C.byref(b), C.byref(c))
     return b.value, c.value
+
+
+def shard_parts(nparts: int, nranks: int, rank: int):
+    """(p_begin, p_count): the parts whose tiles `rank` holds in the sharded halo exchange"""
+    b, c = C.c_int(), C.c_int()
+    load().ddc_shard_parts(nparts, nranks, rank, C.byref(b), C.byref(c))
+    return b.value, c.value
+
+
+def halo_connect(handles: list["Handle"], elems: int) -> list[int]:
+    """join the halo buffers of handles that live in this process (handles[q] = rank q); returns each rank's tiles
+    pointer (device memory for up to `elems` doubles)"""
+    n = len(handles)
+    hs = (C.c_void_p * n)(*[h.h.value for h in handles])
+    out = (C.c_void_p * n)()
+    L = load()
+    if L.ddc_halo_connect(hs, n, elems, out):
+        err = [L.ddc_last_error(h.h).decode() for h in handles]
+        raise DdcError("ddc_halo_connect: %s" % (next((e for e in err if e), None) or L.ddc_last_error(None).decode()))
+    return [int(p) for p in out]
 
 
 def nccl_unique_id() -> bytes:
@@ -240,6 +270,30 @@ class Handle:
 
     def halo_exchange_f64(self, tiles_dev_ptr: int, periodic: bool = False):
         self._ck(self.L.ddc_halo_exchange_f64(self.h, tiles_dev_ptr, int(periodic)), "ddc_halo_exchange_f64")
+
+    def halo_shard_offsets(self) -> np.ndarray:
+        """element offsets of this rank's framed tiles in its own halo buffer (ddc_halo_shard_offsets)"""
+        _, count = shard_parts(self.nparts, self.nranks, self.rank)
+        out = np.empty(count + 1, dtype=np.int64)
+        self._ck(self.L.ddc_halo_shard_offsets(self.h, out.ctypes.data), "ddc_halo_shard_offsets")
+        return out
+
+    def halo_export(self, elems: int):
+        """allocate this rank's halo buffer for up to `elems` doubles; returns (tiles device pointer, CUDA IPC handle)"""
+        ptr = C.c_void_p()
+        buf = C.create_string_buffer(IPC_HANDLE_BYTES)
+        self._ck(self.L.ddc_halo_export(self.h, elems, C.byref(ptr), buf), "ddc_halo_export")
+        return int(ptr.value), buf.raw
+
+    def halo_import(self, handles: list[bytes]):
+        """handles: the halo_export() IPC handle of every rank, in rank order"""
+        self._ck(self.L.ddc_halo_import(self.h, b"".join(handles)), "ddc_halo_import")
+
+    def halo_exchange_shards_f64(self, periodic: bool = False):
+        self._ck(self.L.ddc_halo_exchange_shards_f64(self.h, int(periodic)), "ddc_halo_exchange_shards_f64")
+
+    def halo_close(self):
+        self._ck(self.L.ddc_halo_close(self.h), "ddc_halo_close")
 
     def neighbour_counts(self, edge: int, periodic: int) -> np.ndarray:
         out = np.empty(self.nparts, dtype=np.int32)

@@ -238,6 +238,16 @@ struct ddc_handle_s {
     size_t x_flagcap = 0; // per-block flags of the row-count kernel, per rank
     bool p2p = false, peer_local = false; // peer_local: the peers are handles of this process (ddc_peer_connect)
     unsigned step = 0; // decompositions enqueued so far (the flag value of the exchange barriers)
+    // halo exchange across ranks (ddc_halo_*): one buffer per rank, [HALO_HEAD_BYTES head][tiles of this rank's parts]
+    char* halo_buf = nullptr; // this rank's buffer
+    char* halo_peer[MAX_PEERS] = {}; // every rank's buffer as mapped here (halo_peer[rank] == halo_buf)
+    int64_t halo_elems = 0; // capacity for tiles, in doubles
+    bool halo_mapped = false, halo_local = false; // halo_local: the peers are handles of this process (ddc_halo_connect)
+    bool halo_shard_ok = false; // ddc_halo_shard_offsets ran for the current decomposition
+    long long halo_shard_max = 0; // the largest rank's tile total of that decomposition
+    unsigned halo_step = 0; // exchanges enqueued since the buffers were joined
+    int* halo_err = nullptr; // pinned, device-mapped: set by a halo kernel whose wait timed out
+    int* halo_err_dev = nullptr;
     int h_totals[8] = { 0 };
     bool totals_valid = false;
     // Page-locked copy of the small results (boxes, neighbour counts, part loads; the neighbour lists on demand): the
@@ -482,6 +492,73 @@ int fetch_lists(ddc_handle_t h)
     h->lists_cached = true;
     return DDC_OK;
 }
+
+// ---- CUDA IPC and peer access, shared by the histogram exchange (ddc_peer_*) and the halo exchange (ddc_halo_*) ----
+// the IPC handle of `buf` (the base of a cudaMalloc allocation) into out[DDC_IPC_HANDLE_BYTES]
+int ipc_export(ddc_handle_t h, void* buf, void* out)
+{
+    cudaIpcMemHandle_t ipc;
+    CUDA_TRY(h, cudaIpcGetMemHandle(&ipc, buf));
+    static_assert(sizeof(cudaIpcMemHandle_t) == DDC_IPC_HANDLE_BYTES, "IPC handle size");
+    memcpy(out, &ipc, sizeof ipc);
+    return DDC_OK;
+}
+// map every other rank's buffer (all_handles: nranks IPC handles in rank order); mapped[rank] = own
+template <typename T>
+int ipc_import(ddc_handle_t h, const void* all_handles, T* own, T** mapped)
+{
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    for (int q = 0; q < h->nranks; q++) {
+        if (q == h->rank) {
+            mapped[q] = own;
+            continue;
+        }
+        cudaIpcMemHandle_t ipc;
+        memcpy(&ipc, (const char*)all_handles + (size_t)q * DDC_IPC_HANDLE_BYTES, sizeof ipc);
+        void* p = nullptr;
+        CUDA_TRY(h, cudaIpcOpenMemHandle(&p, ipc, cudaIpcMemLazyEnablePeerAccess));
+        mapped[q] = (T*)p;
+    }
+    return DDC_OK;
+}
+// unmap what ipc_import mapped (local: the peers are handles of this process, nothing was IPC-mapped); the first error
+template <typename T>
+cudaError_t ipc_unmap(ddc_handle_t h, T** mapped, bool local)
+{
+    cudaError_t first = cudaSuccess;
+    for (int q = 0; q < h->nranks && q < MAX_PEERS; q++) {
+        if (mapped[q] && q != h->rank && !local) {
+            const cudaError_t e = cudaIpcCloseMemHandle(mapped[q]);
+            if (first == cudaSuccess)
+                first = e;
+        }
+        mapped[q] = nullptr;
+    }
+    return first;
+}
+// handles of one process: every device may access the memory of every other one
+int enable_peer_access(ddc_handle_t* handles, int n)
+{
+    for (int q = 0; q < n; q++) {
+        ddc_handle_t h = handles[q];
+        CUDA_TRY(h, cudaSetDevice(h->device));
+        for (int r = 0; r < n; r++) {
+            if (handles[r]->device == h->device)
+                continue;
+            int can = 0;
+            CUDA_TRY(h, cudaDeviceCanAccessPeer(&can, h->device, handles[r]->device));
+            if (!can)
+                return fail(h, DDC_ERR_CUDA, "device %d cannot access the memory of device %d", h->device, handles[r]->device);
+            cudaError_t e = cudaDeviceEnablePeerAccess(handles[r]->device, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled)
+                cudaGetLastError(); // not an error
+            else if (e != cudaSuccess)
+                return fail(h, DDC_ERR_CUDA, "cudaDeviceEnablePeerAccess(%d -> %d): %s", h->device, handles[r]->device,
+                    cudaGetErrorString(e));
+        }
+    }
+    return DDC_OK;
+}
 } // namespace
 
 // ------------------------------------------------------------------------------------------------
@@ -603,11 +680,14 @@ int ddc_destroy(ddc_handle_t h)
         cudaStreamSynchronize(h->side_stream);
     if (h->comm)
         g_nccl.CommDestroy(h->comm);
-    for (int q = 0; q < h->nranks && q < MAX_PEERS; q++)
-        if (h->xpeer[q] && q != h->rank && !h->peer_local)
-            cudaIpcCloseMemHandle(h->xpeer[q]);
+    ipc_unmap(h, h->xpeer, h->peer_local);
     if (h->xbuf)
         cudaFree(h->xbuf);
+    ipc_unmap(h, h->halo_peer, h->halo_local);
+    if (h->halo_buf)
+        cudaFree(h->halo_buf);
+    if (h->halo_err)
+        cudaFreeHost(h->halo_err);
     h->mask_own.release();
     h->bits.release();
     h->colcount.release();
@@ -687,11 +767,7 @@ int ddc_peer_export(ddc_handle_t h, int nx, int ny, int nparts, void* ipc_handle
     const size_t words = peer_words(h->nranks, h->x_colcap, h->x_rowcap, h->x_flagcap);
     CUDA_TRY(h, cudaMalloc((void**)&h->xbuf, words * sizeof(unsigned)));
     CUDA_TRY(h, cudaMemset(h->xbuf, 0, words * sizeof(unsigned)));
-    cudaIpcMemHandle_t ipc;
-    CUDA_TRY(h, cudaIpcGetMemHandle(&ipc, h->xbuf));
-    static_assert(sizeof(cudaIpcMemHandle_t) == DDC_IPC_HANDLE_BYTES, "IPC handle size");
-    memcpy(ipc_handle_out, &ipc, sizeof ipc);
-    return DDC_OK;
+    return ipc_export(h, h->xbuf, ipc_handle_out);
 }
 
 int ddc_peer_import(ddc_handle_t h, const void* all_handles)
@@ -700,18 +776,8 @@ int ddc_peer_import(ddc_handle_t h, const void* all_handles)
         return fail(h, DDC_ERR_ARG, "ddc_peer_import: bad arguments");
     if (!h->xbuf)
         return fail(h, DDC_ERR_STATE, "ddc_peer_import: call ddc_peer_export() first");
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    for (int q = 0; q < h->nranks; q++) {
-        if (q == h->rank) {
-            h->xpeer[q] = h->xbuf;
-            continue;
-        }
-        cudaIpcMemHandle_t ipc;
-        memcpy(&ipc, (const char*)all_handles + (size_t)q * DDC_IPC_HANDLE_BYTES, sizeof ipc);
-        void* p = nullptr;
-        CUDA_TRY(h, cudaIpcOpenMemHandle(&p, ipc, cudaIpcMemLazyEnablePeerAccess));
-        h->xpeer[q] = (unsigned*)p;
-    }
+    if (int rc = ipc_import(h, all_handles, h->xbuf, h->xpeer))
+        return rc;
     h->p2p = true;
     return DDC_OK;
 }
@@ -723,23 +789,11 @@ int ddc_peer_connect(ddc_handle_t* handles, int n, int nx, int ny, int nparts)
     for (int q = 0; q < n; q++)
         if (!handles[q] || handles[q]->nranks != n || handles[q]->rank != q || handles[q]->xbuf)
             return fail(handles[q], DDC_ERR_ARG, "ddc_peer_connect: handle %d must be rank %d of %d and not yet exported", q, q, n);
+    if (int rc = enable_peer_access(handles, n))
+        return rc;
     for (int q = 0; q < n; q++) {
         ddc_handle_t h = handles[q];
         CUDA_TRY(h, cudaSetDevice(h->device));
-        for (int r = 0; r < n; r++) {
-            if (handles[r]->device == h->device)
-                continue;
-            int can = 0;
-            CUDA_TRY(h, cudaDeviceCanAccessPeer(&can, h->device, handles[r]->device));
-            if (!can)
-                return fail(h, DDC_ERR_CUDA, "device %d cannot access the memory of device %d", h->device, handles[r]->device);
-            cudaError_t e = cudaDeviceEnablePeerAccess(handles[r]->device, 0);
-            if (e == cudaErrorPeerAccessAlreadyEnabled)
-                cudaGetLastError(); // not an error
-            else if (e != cudaSuccess)
-                return fail(h, DDC_ERR_CUDA, "cudaDeviceEnablePeerAccess(%d -> %d): %s", h->device, handles[r]->device,
-                    cudaGetErrorString(e));
-        }
         peer_capacity(nx, ny, nparts, n, &h->x_colcap, &h->x_rowcap, &h->x_flagcap);
         const size_t words = peer_words(n, h->x_colcap, h->x_rowcap, h->x_flagcap);
         CUDA_TRY(h, cudaMalloc((void**)&h->xbuf, words * sizeof(unsigned)));
@@ -765,11 +819,7 @@ int ddc_peer_close(ddc_handle_t h)
         return DDC_ERR_ARG;
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    for (int q = 0; q < h->nranks && q < MAX_PEERS; q++) {
-        if (h->xpeer[q] && q != h->rank && !h->peer_local)
-            CUDA_TRY(h, cudaIpcCloseMemHandle(h->xpeer[q]));
-        h->xpeer[q] = nullptr;
-    }
+    CUDA_TRY(h, ipc_unmap(h, h->xpeer, h->peer_local));
     h->p2p = false;
     return DDC_OK;
 }
@@ -816,6 +866,19 @@ void ddc_shard_rows(int ny, int nranks, int rank, int* y_begin, int* y_count)
         *y_begin = b;
     if (y_count)
         *y_count = e - b;
+}
+
+void ddc_shard_parts(int nparts, int nranks, int rank, int* p_begin, int* p_count)
+{
+    int b = 0, e = 0;
+    if (nparts > 0 && nranks > 0 && rank >= 0 && rank < nranks) {
+        b = (int)((long long)rank * nparts / nranks);
+        e = (int)((long long)(rank + 1) * nparts / nranks);
+    }
+    if (p_begin)
+        *p_begin = b;
+    if (p_count)
+        *p_count = e - b;
 }
 
 static int check_shard(ddc_handle_t h, int nx, int ny, int y_begin, int y_count)
@@ -882,9 +945,16 @@ int ddc_synchronize(ddc_handle_t h)
     if (!h)
         return DDC_ERR_ARG;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    if (h->partitioned && h->pending)
-        return validate(h); // waits for the step and settles the plan
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    if (h->partitioned && h->pending) {
+        if (int rc = validate(h)) // waits for the step and settles the plan
+            return rc;
+    } else
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    if (h->halo_err && *(volatile int*)h->halo_err) { // a halo exchange kernel gave up waiting for a rank
+        *(volatile int*)h->halo_err = 0;
+        return fail(h, DDC_ERR_PEER, "halo exchange timed out: a rank did not reach the exchange within %.1f s",
+            (double)PEER_TIMEOUT_NS * 1e-9);
+    }
     return DDC_OK;
 }
 
@@ -945,6 +1015,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     h->totals_valid = false;
     h->small_cached = h->lists_cached = false;
     h->halo_parts = 0;
+    h->halo_shard_ok = false;
     memset(&h->stats, 0, sizeof h->stats);
     int launches = 0;
     // stage i begins: a CUDA event when profiling, and an NVTX range (the host-side enqueue of the stage; Nsight
@@ -1676,6 +1747,7 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
     h->px = px;
     h->py = py;
     h->mask_set = false; // the mask (if any) has to be set again before the next ddc_partition
+    h->halo_shard_ok = false;
     h->d_mask = nullptr;
     h->pending = false;
     int rc = run_neighbours(h, P, nx, ny, px, py);
@@ -1694,17 +1766,15 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
 // ------------------------------------------------------------------------------------------------
 // halo exchange (a consumer of the neighbour tables)
 // ------------------------------------------------------------------------------------------------
-int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
+// the tile offsets of all parts in one buffer (offsets[P] = total), also left on the device for the exchange kernels
+static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
 {
-    NEED_PARTITION(h);
-    if (!offsets)
-        return fail(h, DDC_ERR_ARG, "ddc_halo_tile_offsets: null output");
     const int P = h->nparts;
     std::vector<int32_t> ex(P), ey(P);
     int rc = ddc_get_boxes(h, nullptr, nullptr, ex.data(), ey.data());
     if (rc)
         return rc;
-    std::vector<long long> off((size_t)P + 1);
+    off.assign((size_t)P + 1, 0);
     long long run = 0;
     for (int p = 0; p < P; p++) {
         off[p] = run;
@@ -1715,7 +1785,18 @@ int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
     CUDA_TRY(h, cudaMemcpyAsync(h->halo_off.p, off.data(), sizeof(long long) * ((size_t)P + 1), cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->halo_parts = P;
-    for (int p = 0; p <= P; p++)
+    return DDC_OK;
+}
+
+int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
+{
+    NEED_PARTITION(h);
+    if (!offsets)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_tile_offsets: null output");
+    std::vector<long long> off;
+    if (int rc = tile_offsets(h, off))
+        return rc;
+    for (size_t p = 0; p < off.size(); p++)
         offsets[p] = off[p];
     return DDC_OK;
 }
@@ -1739,6 +1820,164 @@ int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic)
         h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, tiles_dev,
         periodic ? 0xffu : 0x0fu));
     CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// halo exchange across ranks (parts sharded over the ranks, ghost cells pushed over peer memory)
+// ------------------------------------------------------------------------------------------------
+int ddc_halo_shard_offsets(ddc_handle_t h, int64_t* offsets)
+{
+    NEED_PARTITION(h);
+    if (!offsets)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_shard_offsets: null output");
+    std::vector<long long> off;
+    if (int rc = tile_offsets(h, off))
+        return rc;
+    // every rank's total from the replicated boxes: the exchange refuses on every rank alike when one does not fit
+    const int P = h->nparts, G = h->nranks;
+    long long most = 0;
+    for (int r = 0; r < G; r++) {
+        int b, c;
+        ddc_shard_parts(P, G, r, &b, &c);
+        most = std::max(most, off[(size_t)b + c] - off[b]);
+    }
+    int b, c;
+    ddc_shard_parts(P, G, h->rank, &b, &c);
+    for (int i = 0; i <= c; i++)
+        offsets[i] = off[(size_t)b + i] - off[b];
+    h->halo_shard_max = most;
+    h->halo_shard_ok = true;
+    return DDC_OK;
+}
+
+constexpr int HALO_PUSH_BLOCKS = 4 * 148; // k_halo_push's grid at most: a few waves of B200's 148 SMs
+// this rank's halo buffer: zeroed head (flags, block counter) + room for `elems` doubles; the error word beside it
+static int halo_alloc(ddc_handle_t h, int64_t elems)
+{
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    const size_t bytes = HALO_HEAD_BYTES + (size_t)elems * sizeof(double);
+    CUDA_TRY(h, cudaMalloc((void**)&h->halo_buf, bytes));
+    CUDA_TRY(h, cudaMemsetAsync(h->halo_buf, 0, bytes, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream)); // zero before any peer can see the buffer
+    if (!h->halo_err) {
+        CUDA_TRY(h, cudaHostAlloc((void**)&h->halo_err, sizeof(int), cudaHostAllocMapped));
+        CUDA_TRY(h, cudaHostGetDevicePointer((void**)&h->halo_err_dev, h->halo_err, 0));
+        *h->halo_err = 0;
+    }
+    // Load the exchange kernels now.  Loaded lazily at its first launch (CUDA_MODULE_LOADING=LAZY, the default), a kernel
+    // can wait for the kernels running on the device -- and those can be other ranks' k_halo_open, spinning until this
+    // rank's arrives (measured: the first exchange of handles sharing a B200 timed out).
+    cudaFuncAttributes fa;
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_open));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_push));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_close));
+    h->halo_elems = elems;
+    h->halo_step = 0;
+    return DDC_OK;
+}
+
+int ddc_halo_export(ddc_handle_t h, int64_t elems, double** tiles_dev, void* ipc_handle_out)
+{
+    if (!h || elems < 0 || !tiles_dev || !ipc_handle_out)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_export: bad arguments");
+    if (h->nranks > MAX_PEERS)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_export: at most %d ranks", MAX_PEERS);
+    if (h->halo_buf)
+        return fail(h, DDC_ERR_STATE, "ddc_halo_export: already exported");
+    if (int rc = halo_alloc(h, elems))
+        return rc;
+    *tiles_dev = (double*)(h->halo_buf + HALO_HEAD_BYTES);
+    return ipc_export(h, h->halo_buf, ipc_handle_out);
+}
+
+int ddc_halo_import(ddc_handle_t h, const void* all_handles)
+{
+    if (!h || !all_handles)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_import: bad arguments");
+    if (!h->halo_buf || h->halo_local)
+        return fail(h, DDC_ERR_STATE, "ddc_halo_import: call ddc_halo_export() first");
+    if (h->halo_mapped)
+        return fail(h, DDC_ERR_STATE, "ddc_halo_import: already imported (ddc_halo_close() first)");
+    if (int rc = ipc_import(h, all_handles, h->halo_buf, h->halo_peer))
+        return rc;
+    h->halo_mapped = true;
+    return DDC_OK;
+}
+
+int ddc_halo_connect(ddc_handle_t* handles, int n, int64_t elems, double** tiles_dev)
+{
+    if (!handles || n < 1 || n > MAX_PEERS || elems < 0 || !tiles_dev)
+        return fail(nullptr, DDC_ERR_ARG, "ddc_halo_connect: bad arguments");
+    for (int q = 0; q < n; q++)
+        if (!handles[q] || handles[q]->nranks != n || handles[q]->rank != q || handles[q]->halo_buf)
+            return fail(handles[q], DDC_ERR_ARG, "ddc_halo_connect: handle %d must be rank %d of %d and not yet exported", q, q,
+                n);
+    if (int rc = enable_peer_access(handles, n))
+        return rc;
+    for (int q = 0; q < n; q++) {
+        if (int rc = halo_alloc(handles[q], elems))
+            return rc;
+        tiles_dev[q] = (double*)(handles[q]->halo_buf + HALO_HEAD_BYTES);
+    }
+    for (int q = 0; q < n; q++) {
+        for (int r = 0; r < n; r++)
+            handles[q]->halo_peer[r] = handles[r]->halo_buf;
+        handles[q]->halo_mapped = true;
+        handles[q]->halo_local = true;
+    }
+    return DDC_OK;
+}
+
+int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
+{
+    NEED_PARTITION(h);
+    // every check below has the same outcome on every rank (replicated tables, the same calls): no rank is left waiting
+    if (!h->halo_buf || !h->halo_mapped)
+        return fail(h, DDC_ERR_STATE, "ddc_halo_exchange_shards_f64: no halo buffers (ddc_halo_export + ddc_halo_import, or "
+                                      "ddc_halo_connect)");
+    if (!h->halo_shard_ok || h->halo_parts != h->nparts)
+        return fail(h, DDC_ERR_STATE, "ddc_halo_exchange_shards_f64: call ddc_halo_shard_offsets() for this decomposition first");
+    if (h->halo_shard_max > h->halo_elems)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_exchange_shards_f64: a rank's tiles need %lld doubles, the buffers hold %lld",
+            h->halo_shard_max, (long long)h->halo_elems);
+    if (!h->have_nbr)
+        return DDC_OK; // one part (or no tables asked for): nothing to exchange
+    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
+        return rc;
+    const int P = h->nparts, G = h->nranks;
+    Tables t = tables(h, P);
+    HaloShards hs {};
+    hs.ps.rank = h->rank;
+    hs.ps.G = G;
+    hs.ps.enabled = 1;
+    hs.ps.step = ++h->halo_step;
+    for (int q = 0; q < G; q++) {
+        hs.ps.flags[q] = (unsigned*)h->halo_peer[q];
+        hs.tiles[q] = (double*)(h->halo_peer[q] + HALO_HEAD_BYTES);
+    }
+    hs.done = (unsigned*)h->halo_buf + 2 * MAX_PEERS;
+    hs.opened = hs.done + 1;
+    hs.err = h->halo_err_dev;
+    hs.P = P;
+    ddc_shard_parts(P, G, h->rank, &hs.p_begin, &hs.p_count);
+    const unsigned lists = periodic ? 0xffu : 0x0fu;
+    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
+    CUDA_TRY(h, launch_k(k_halo_push, dim3((unsigned)std::max(1, std::min(hs.p_count, HALO_PUSH_BLOCKS))), dim3(256), 0, h->stream, false, hs, t.bx,
+        h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, lists));
+    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
+    CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+
+int ddc_halo_close(ddc_handle_t h)
+{
+    if (!h)
+        return DDC_ERR_ARG;
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    CUDA_TRY(h, ipc_unmap(h, h->halo_peer, h->halo_local));
+    h->halo_mapped = false;
     return DDC_OK;
 }
 

@@ -2529,6 +2529,138 @@ __global__ void __launch_bounds__(256) k_halo_exchange(BoxTable bx, int P, const
 }
 
 // ------------------------------------------------------------------------------------------------
+// Halo exchange across ranks: parts sharded over the ranks, ghost cells pushed over peer memory
+// ------------------------------------------------------------------------------------------------
+// Rank r owns parts [r P / G, (r + 1) P / G) and holds their framed tiles, in the layout of k_halo_exchange restricted
+// to those parts and rebased to 0, behind a head of HALO_HEAD_BYTES in a buffer of its own that every rank maps.  One
+// exchange is three plain launches with halo step k:
+//   k_halo_open   one block: R = k into slot [0][rank] of every rank's flags, then wait for R >= k of every rank
+//                 (nothing earlier on any rank's stream still reads the ghosts that are about to be overwritten);
+//   k_halo_push   every ghost cell whose SOURCE part this rank owns, read locally and stored into the receiving
+//                 part's tile wherever it lives (posted remote stores: no NVLink round trip per access); the last
+//                 block stores D = k into slot [1][rank] of every rank's flags;
+//   k_halo_close  one block: wait for D >= k of every rank (every ghost of this rank's tiles has arrived).
+// The flags are PeerSync flags ([stage][MAX_PEERS], value 2 k), never reset.  A wait that times out sets the
+// handle's error word (host memory, read by ddc_synchronize); a push whose open timed out stores nothing and raises
+// no flag, so the ranks that wait for it time out too instead of reading stale ghosts.
+constexpr size_t HALO_HEAD_BYTES = 256; // [flags: 2 x MAX_PEERS u32][block counter][opened step] ... tiles
+struct HaloShards {
+    PeerSync ps; // flags[q] = rank q's head as mapped here; step = the exchange number k
+    double* tiles[MAX_PEERS]; // rank q's tiles as mapped here (tiles[rank]: this rank's)
+    unsigned* done; // this rank's block counter of k_halo_push, zero between exchanges
+    unsigned* opened; // this rank's word: the last step whose k_halo_open saw every rank
+    int* err; // host-mapped error word (1: a rank did not reach the exchange in time)
+    int P, p_begin, p_count; // all parts; this rank's range
+};
+__device__ __forceinline__ void halo_timed_out(const HaloShards& hs)
+{
+#ifndef DDC_HOST_EMU
+    *(volatile int*)hs.err = 1;
+    __threadfence_system();
+#else
+    *hs.err = 1;
+#endif
+}
+// phases: 1 signal, 2 wait, 3 both (the device always runs both; the CPU emulation runs its ranks phase by phase)
+__global__ void __launch_bounds__(32) k_halo_open(HaloShards hs, int phases)
+{
+    const int q = threadIdx.x;
+    if (phases & 1) {
+        __threadfence_system(); // everything this rank did before is complete (plain launch) and performed
+        if (q < hs.ps.G)
+            peer_signal(hs.ps, 0, 0u);
+    }
+    if (phases & 2) {
+        unsigned seen = 0;
+        const bool ok = q >= hs.ps.G || peer_wait(hs.ps, 0, &seen);
+        if (!__syncthreads_or(!ok)) {
+            if (q == 0)
+                *hs.opened = hs.ps.step;
+        } else if (q == 0)
+            halo_timed_out(hs);
+    }
+}
+
+// One warp per (list l, owned part q): q's neighbours p in list l receive q's cells in their ghosts on the opposite
+// edge.  The lists are symmetric (p is in q's edge-e list iff q is in p's opposite-edge list, same periodic flag), so
+// q's entry in p's list -- found by binary search, the lists are id-ascending -- gives the halo size and start that
+// k_halo_exchange uses for that ghost run, and the cells and values written are exactly the ones it writes.
+__global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, const int* __restrict__ counts,
+    const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
+    const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists)
+{
+    __shared__ int s_last;
+    const int P = hs.P, G = hs.ps.G;
+    const bool go = *(volatile unsigned*)hs.opened == hs.ps.step;
+    // grid-stride over the warps: few enough blocks that the system fence each one pays below stays cheap
+    const long long nw = go ? 8LL * hs.p_count : 0, stride = (long long)gridDim.x * (blockDim.x >> 5);
+    for (long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < nw; w += stride) {
+        const int l = (int)(w / hs.p_count), q = hs.p_begin + (int)(w % hs.p_count);
+        if ((lists >> l) & 1u) {
+            const int lane = lane_id();
+            const int lp = (l & 4) | ((l & 3) ^ 1); // the list of p that holds q
+            const int edge = lp & 3; // p's edge that faces q
+            const int qw = bx.ex[q];
+            const double* theirs = hs.tiles[hs.ps.rank] + (off[q] - off[hs.p_begin]);
+            const int n = counts[l * P + q], first = offsets[l * (P + 1) + q];
+            for (int k = 0; k < n; k++) {
+                const int p = ids[(size_t)l * cap + first + k];
+                const int m = counts[lp * P + p];
+                const size_t base = (size_t)lp * cap + offsets[lp * (P + 1) + p];
+                int lo = 0, hi = m;
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (ids[base + mid] < q)
+                        lo = mid + 1;
+                    else
+                        hi = mid;
+                }
+                if (lo == m || ids[base + lo] != q)
+                    continue; // (not symmetric: k_halo_exchange would write nothing for this pair either)
+                const int h = halos[base + lo], st = starts[base + lo];
+                const int owner = (int)(((long long)(p + 1) * G - 1) / P), pb = (int)((long long)owner * P / G);
+                double* mine = hs.tiles[owner] + (off[p] - off[pb]);
+                const int px0 = bx.x0[p], py0 = bx.y0[p], pex = bx.ex[p], pey = bx.ey[p];
+                const bool lr = edge < 2;
+                const int along = lr ? max(py0, bx.y0[q]) - py0 : max(px0, bx.x0[q]) - px0;
+                for (int i = lane; i < h; i += 32) {
+                    const int s = st + (lr ? i * qw : i);
+                    const double v = theirs[(size_t)(s / qw + 1) * (qw + 2) + (s % qw + 1)];
+                    const int row = lr ? along + i + 1 : (edge == 2 ? 0 : pey + 1);
+                    const int col = lr ? (edge == 0 ? 0 : pex + 1) : along + i + 1;
+                    mine[(size_t)row * (pex + 2) + col] = v;
+                }
+            }
+        }
+    }
+    if (!go)
+        return; // (block-uniform) k_halo_open timed out: no stores, no flag
+    __syncthreads(); // every thread's stores are issued ...
+    if (threadIdx.x == 0) {
+        __threadfence_system(); // ... and performed at the peers before the block is counted
+        s_last = atomicAdd(hs.done, 1u) == gridDim.x - 1u;
+    }
+    __syncthreads();
+    if (s_last) {
+        if ((int)threadIdx.x < G)
+            peer_signal(hs.ps, 1, 0u);
+        if (threadIdx.x == 0)
+            *hs.done = 0u;
+    }
+}
+
+__global__ void __launch_bounds__(32) k_halo_close(HaloShards hs)
+{
+    if (*(volatile unsigned*)hs.opened != hs.ps.step)
+        return; // k_halo_open timed out and said so
+    const int q = threadIdx.x;
+    unsigned seen = 0;
+    const bool ok = q >= hs.ps.G || peer_wait(hs.ps, 1, &seen);
+    if (__syncthreads_or(!ok) && q == 0)
+        halo_timed_out(hs);
+}
+
+// ------------------------------------------------------------------------------------------------
 // synthetic land-sea mask: two octaves of integer value noise (bit-identical on host and device)
 // ------------------------------------------------------------------------------------------------
 __host__ __device__ inline uint64_t splitmix64(uint64_t z)

@@ -188,6 +188,35 @@ DDC_API int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny
 DDC_API int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets /* nparts + 1 */);
 DDC_API int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic);
 
+/* The same exchange with the parts SHARDED over the ranks (nranks >= 1, one GPU each; several ranks of one process may
+   share a device).  Rank r owns parts [p_begin, p_begin + p_count) of ddc_shard_parts and holds their tiles in ONE
+   library-owned device buffer, in the ddc_halo_tile_offsets layout restricted to those parts and rebased to 0
+   (ddc_halo_shard_offsets: offsets[p_count] = this rank's total), so the ranks' buffers concatenated in rank order ARE
+   the single-buffer layout.  ddc_halo_exchange_shards_f64 then does what ddc_halo_exchange_f64 does on that
+   concatenation, bit for bit: each rank's kernels store the ghost cells its parts are the source of straight into the
+   receiving part's tile, on whichever GPU it lives (posted stores over NVLink), between two flag barriers.
+   Set-up: one process per GPU -- ddc_halo_export allocates this rank's buffer for up to `elems` doubles (every rank
+   passes the same elems) and returns its CUDA IPC handle; the host gathers the handles (MPI_Allgather /
+   torch.distributed) and hands them, in rank order, to ddc_halo_import.  One process -- ddc_halo_connect(handles, n,
+   elems, tiles_dev): handles[q] is rank q of n; ranks that share a device must run on different streams.  These
+   buffers are independent of the ddc_peer_* exchange buffers: decompositions may use NCCL or peer memory alike.
+   The flags of the exchange carry the number of the exchange: after the buffers are joined every rank makes the same
+   number of ddc_halo_exchange_shards_f64 calls, as every rank makes the same ddc_partition calls for the peer
+   buffers above.  The call only enqueues (on the handle's stream) and returns, so one host thread can drive several
+   handles in turn; ddc_synchronize reports a rank that did not reach an exchange within the timeout as DDC_ERR_PEER.
+   Errors are the same on every rank and come before anything is enqueued: DDC_ERR_STATE without buffers or without
+   ddc_halo_shard_offsets for the current decomposition, DDC_ERR_ARG when some rank's tiles exceed `elems`.  Without
+   neighbour tables (one part, or no DDC_WANT_NEIGHBOURS) the exchange does nothing on every rank. */
+DDC_API void ddc_shard_parts(int nparts, int nranks, int rank, int* p_begin, int* p_count); /* p_begin = rank * nparts / nranks */
+DDC_API int ddc_halo_shard_offsets(ddc_handle_t h, int64_t* offsets /* p_count + 1 */);
+DDC_API int ddc_halo_export(ddc_handle_t h, int64_t elems, double** tiles_dev, void* ipc_handle_out /* DDC_IPC_HANDLE_BYTES */);
+DDC_API int ddc_halo_import(ddc_handle_t h, const void* all_handles /* nranks * DDC_IPC_HANDLE_BYTES, rank order */);
+DDC_API int ddc_halo_connect(ddc_handle_t* handles, int n, int64_t elems, double** tiles_dev /* n */);
+DDC_API int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic);
+/* unmap the other ranks' halo buffers.  Shutdown order as for ddc_peer_close: every rank calls ddc_halo_close(), the
+   host synchronises the ranks, then every rank calls ddc_destroy(), which frees its own halo buffer. */
+DDC_API int ddc_halo_close(ddc_handle_t h);
+
 /* ---- synthetic masks (SURVEY 8d): deterministic value-noise land-sea mask, generated directly
    into device memory so that no 4 GiB file is needed for the large configurations.
    land_frac in [0,1] is the target land fraction; rows as in ddc_set_mask_device. */

@@ -32,6 +32,7 @@ SYMBOLS = (
     "ddc_peer_export", "ddc_peer_import", "ddc_peer_close", "ddc_host_alloc", "ddc_host_free", "ddc_peer_connect", "ddc_halo_tile_offsets", "ddc_halo_exchange_f64",
     "ddc_shard_parts", "ddc_halo_shard_offsets", "ddc_halo_export", "ddc_halo_import", "ddc_halo_connect",
     "ddc_halo_exchange_shards_f64", "ddc_halo_close",
+    "ddc_halo_scatter_f64", "ddc_halo_gather_f64", "ddc_halo_scatter_shards_f64", "ddc_halo_gather_shards_f64",
 )
 
 
@@ -106,6 +107,10 @@ def load() -> C.CDLL:
     L.ddc_halo_connect.argtypes = [C.POINTER(vp), i32, C.c_int64, C.POINTER(vp)]
     L.ddc_halo_exchange_shards_f64.argtypes = [vp, i32]
     L.ddc_halo_close.argtypes = [vp]
+    L.ddc_halo_scatter_f64.argtypes = [vp, vp, vp]
+    L.ddc_halo_gather_f64.argtypes = [vp, vp, vp]
+    L.ddc_halo_scatter_shards_f64.argtypes = [vp, vp]
+    L.ddc_halo_gather_shards_f64.argtypes = [vp, vp]
     L.ddc_generate_mask_device.argtypes = [vp, vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     L.ddc_generate_mask_host.argtypes = [vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     _lib = L
@@ -294,6 +299,22 @@ class Handle:
 
     def halo_close(self):
         self._ck(self.L.ddc_halo_close(self.h), "ddc_halo_close")
+
+    def halo_scatter_f64(self, field_ptr: int, tiles_ptr: int):
+        """tile interiors <- the field (device double [ny][nx]), one buffer in the halo_tile_offsets() layout"""
+        self._ck(self.L.ddc_halo_scatter_f64(self.h, field_ptr, tiles_ptr), "ddc_halo_scatter_f64")
+
+    def halo_gather_f64(self, tiles_ptr: int, field_ptr: int):
+        """the field (device double [ny][nx]) <- tile interiors, one buffer in the halo_tile_offsets() layout"""
+        self._ck(self.L.ddc_halo_gather_f64(self.h, tiles_ptr, field_ptr), "ddc_halo_gather_f64")
+
+    def halo_scatter_shards_f64(self, rows_ptr: int):
+        """every rank's tile interiors <- this rank's rows (device double [y_count][nx] of shard_rows)"""
+        self._ck(self.L.ddc_halo_scatter_shards_f64(self.h, rows_ptr), "ddc_halo_scatter_shards_f64")
+
+    def halo_gather_shards_f64(self, rows_ptr: int):
+        """this rank's rows (device double [y_count][nx] of shard_rows) <- every rank's tile interiors"""
+        self._ck(self.L.ddc_halo_gather_shards_f64(self.h, rows_ptr), "ddc_halo_gather_shards_f64")
 
     def neighbour_counts(self, edge: int, periodic: int) -> np.ndarray:
         out = np.empty(self.nparts, dtype=np.int32)

@@ -187,6 +187,10 @@ struct ddc_handle_s {
     DevBuf<DevScalars> sc;
     DevBuf<long long> halo_off; // tile offsets of the halo exchange (ddc_halo_tile_offsets)
     int halo_parts = 0;
+    // the (part, row) ranges of halo scatter / gather (HaloItems): [0] every field row, [1] this rank's ddc_shard_rows
+    DevBuf<int> halo_items; // [2][4 P + 1]
+    DevBuf<long long> halo_item_base; // [2][P]
+    int halo_items_n[2] = { 0, 0 }, halo_items_total[2] = { 0, 0 };
     DevBuf<unsigned> gate; // the word the gate kernel of the second stream waits for (see BoxGate)
     int use_gate = 1; // DDC_GATE: 0 never, 1 unless the shard is tiny, 2 always
     bool side_pdl = true; // DDC_SIDE_PDL: the scan of the neighbour counts launched programmatically behind the count kernel
@@ -700,6 +704,8 @@ int ddc_destroy(ddc_handle_t h)
     h->sc.release();
     h->gate.release();
     h->halo_off.release();
+    h->halo_items.release();
+    h->halo_item_base.release();
     h->plan.release();
     h->strips.release();
     h->boxes.release();
@@ -1766,12 +1772,13 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
 // ------------------------------------------------------------------------------------------------
 // halo exchange (a consumer of the neighbour tables)
 // ------------------------------------------------------------------------------------------------
-// the tile offsets of all parts in one buffer (offsets[P] = total), also left on the device for the exchange kernels
+// the tile offsets of all parts in one buffer (offsets[P] = total), also left on the device for the exchange kernels,
+// and beside them the (part, row) ranges of scatter and gather: every field row, and this rank's ddc_shard_rows
 static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
 {
     const int P = h->nparts;
-    std::vector<int32_t> ex(P), ey(P);
-    int rc = ddc_get_boxes(h, nullptr, nullptr, ex.data(), ey.data());
+    std::vector<int32_t> y0(P), ex(P), ey(P);
+    int rc = ddc_get_boxes(h, nullptr, y0.data(), ex.data(), ey.data());
     if (rc)
         return rc;
     off.assign((size_t)P + 1, 0);
@@ -1781,8 +1788,23 @@ static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
         run += (long long)(std::max(ex[p], 0) + 2) * (std::max(ey[p], 0) + 2);
     }
     off[P] = run;
+    const size_t per = (size_t)4 * P + 1;
+    std::vector<int> items(2 * per);
+    std::vector<long long> base((size_t)2 * P);
+    int yb, yc;
+    ddc_shard_rows(h->ny, h->nranks, h->rank, &yb, &yc);
+    for (int s = 0; s < 2; s++) {
+        int* t = items.data() + s * per;
+        h->halo_items_n[s] = halo_item_ranges(P, s ? h->nranks : 1, y0.data(), ex.data(), ey.data(), off.data(), s ? yb : 0,
+            s ? yb + yc : h->ny, t, base.data() + (size_t)s * P);
+        h->halo_items_total[s] = t[3 * P + h->halo_items_n[s]];
+    }
     CUDA_TRY(h, h->halo_off.ensure((size_t)P + 1));
+    CUDA_TRY(h, h->halo_items.ensure(2 * per));
+    CUDA_TRY(h, h->halo_item_base.ensure((size_t)2 * P));
     CUDA_TRY(h, cudaMemcpyAsync(h->halo_off.p, off.data(), sizeof(long long) * ((size_t)P + 1), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->halo_items.p, items.data(), sizeof(int) * 2 * per, cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->halo_item_base.p, base.data(), sizeof(long long) * 2 * P, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->halo_parts = P;
     return DDC_OK;
@@ -1821,6 +1843,44 @@ int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic)
         periodic ? 0xffu : 0x0fu));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;
+}
+
+// halo scatter / gather: the field rows <-> the tile interiors (k_halo_field, k_halo_field_shards)
+constexpr int HALO_FIELD_BLOCKS = 8 * 148; // at most: 8 blocks of 256 threads on each of B200's 148 SMs, grid-stride
+static HaloItems halo_items_of(ddc_handle_t h, int s) // s: 0 every field row, 1 this rank's shard rows
+{
+    const size_t P = h->nparts, per = 4 * P + 1;
+    const int* t = h->halo_items.p + s * per;
+    return HaloItems { t, t + P, t + 2 * P, t + 3 * P, h->halo_item_base.p + s * P, h->halo_items_n[s] };
+}
+static unsigned halo_field_grid(ddc_handle_t h, int s) // one warp per item, 8 per block
+{
+    return (unsigned)std::max(1, std::min((h->halo_items_total[s] + 7) / 8, HALO_FIELD_BLOCKS));
+}
+
+static int halo_field(ddc_handle_t h, bool scatter, double* field_dev, double* tiles_dev, const char* name)
+{
+    if (!field_dev || !tiles_dev)
+        return fail(h, DDC_ERR_ARG, "%s: null pointer", name);
+    if (h->halo_parts != h->nparts)
+        return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_tile_offsets() for this decomposition first", name);
+    Tables t = tables(h, h->nparts);
+    CUDA_TRY(h, launch_k(scatter ? k_halo_field<true> : k_halo_field<false>, dim3(halo_field_grid(h, 0)), dim3(256), 0, h->stream,
+        false, halo_items_of(h, 0), t.bx, tiles_dev, field_dev, h->nx));
+    CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+
+int ddc_halo_scatter_f64(ddc_handle_t h, const double* field_dev, double* tiles_dev)
+{
+    NEED_PARTITION(h);
+    return halo_field(h, true, const_cast<double*>(field_dev), tiles_dev, "ddc_halo_scatter_f64");
+}
+
+int ddc_halo_gather_f64(ddc_handle_t h, const double* tiles_dev, double* field_dev)
+{
+    NEED_PARTITION(h);
+    return halo_field(h, false, field_dev, const_cast<double*>(tiles_dev), "ddc_halo_gather_f64");
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1872,6 +1932,8 @@ static int halo_alloc(ddc_handle_t h, int64_t elems)
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_open));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_push));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_close));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<true>));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<false>));
     h->halo_elems = elems;
     h->halo_step = 0;
     return DDC_OK;
@@ -1929,38 +1991,51 @@ int ddc_halo_connect(ddc_handle_t* handles, int n, int64_t elems, double** tiles
     return DDC_OK;
 }
 
-int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
+// the checks of every sharded halo call (exchange, scatter, gather).  Each has the same outcome on every rank
+// (replicated tables, the same calls), so no rank is left waiting for one that refused.
+static int halo_shards_ready(ddc_handle_t h, const char* name)
 {
-    NEED_PARTITION(h);
-    // every check below has the same outcome on every rank (replicated tables, the same calls): no rank is left waiting
     if (!h->halo_buf || !h->halo_mapped)
-        return fail(h, DDC_ERR_STATE, "ddc_halo_exchange_shards_f64: no halo buffers (ddc_halo_export + ddc_halo_import, or "
-                                      "ddc_halo_connect)");
+        return fail(h, DDC_ERR_STATE, "%s: no halo buffers (ddc_halo_export + ddc_halo_import, or ddc_halo_connect)", name);
     if (!h->halo_shard_ok || h->halo_parts != h->nparts)
-        return fail(h, DDC_ERR_STATE, "ddc_halo_exchange_shards_f64: call ddc_halo_shard_offsets() for this decomposition first");
+        return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_shard_offsets() for this decomposition first", name);
     if (h->halo_shard_max > h->halo_elems)
-        return fail(h, DDC_ERR_ARG, "ddc_halo_exchange_shards_f64: a rank's tiles need %lld doubles, the buffers hold %lld",
-            h->halo_shard_max, (long long)h->halo_elems);
-    if (!h->have_nbr)
-        return DDC_OK; // one part (or no tables asked for): nothing to exchange
-    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
-        return rc;
-    const int P = h->nparts, G = h->nranks;
-    Tables t = tables(h, P);
+        return fail(h, DDC_ERR_ARG, "%s: a rank's tiles need %lld doubles, the buffers hold %lld", name, h->halo_shard_max,
+            (long long)h->halo_elems);
+    return DDC_OK;
+}
+
+// the kernels' view of the buffers for the next sharded halo call: it takes the next step number
+static HaloShards halo_shards_next(ddc_handle_t h)
+{
     HaloShards hs {};
     hs.ps.rank = h->rank;
-    hs.ps.G = G;
+    hs.ps.G = h->nranks;
     hs.ps.enabled = 1;
     hs.ps.step = ++h->halo_step;
-    for (int q = 0; q < G; q++) {
+    for (int q = 0; q < h->nranks; q++) {
         hs.ps.flags[q] = (unsigned*)h->halo_peer[q];
         hs.tiles[q] = (double*)(h->halo_peer[q] + HALO_HEAD_BYTES);
     }
     hs.done = (unsigned*)h->halo_buf + 2 * MAX_PEERS;
     hs.opened = hs.done + 1;
     hs.err = h->halo_err_dev;
-    hs.P = P;
-    ddc_shard_parts(P, G, h->rank, &hs.p_begin, &hs.p_count);
+    hs.P = h->nparts;
+    ddc_shard_parts(h->nparts, h->nranks, h->rank, &hs.p_begin, &hs.p_count);
+    return hs;
+}
+
+int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
+{
+    NEED_PARTITION(h);
+    if (int rc = halo_shards_ready(h, "ddc_halo_exchange_shards_f64"))
+        return rc;
+    if (!h->have_nbr)
+        return DDC_OK; // one part (or no tables asked for): nothing to exchange
+    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
+        return rc;
+    Tables t = tables(h, h->nparts);
+    const HaloShards hs = halo_shards_next(h);
     const unsigned lists = periodic ? 0xffu : 0x0fu;
     CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
     CUDA_TRY(h, launch_k(k_halo_push, dim3((unsigned)std::max(1, std::min(hs.p_count, HALO_PUSH_BLOCKS))), dim3(256), 0, h->stream, false, hs, t.bx,
@@ -1968,6 +2043,36 @@ int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
     CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;
+}
+
+static int halo_field_shards(ddc_handle_t h, bool scatter, double* rows_dev, const char* name)
+{
+    if (int rc = halo_shards_ready(h, name))
+        return rc;
+    int yb, yc;
+    ddc_shard_rows(h->ny, h->nranks, h->rank, &yb, &yc);
+    if (!rows_dev && yc > 0) // (this rank only: its peers time out waiting for it and report DDC_ERR_PEER)
+        return fail(h, DDC_ERR_ARG, "%s: null rows (this rank holds rows %d..%d)", name, yb, yb + yc - 1);
+    Tables t = tables(h, h->nparts);
+    const HaloShards hs = halo_shards_next(h);
+    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
+    CUDA_TRY(h, launch_k(scatter ? k_halo_field_shards<true> : k_halo_field_shards<false>, dim3(halo_field_grid(h, 1)), dim3(256), 0,
+        h->stream, false, hs, halo_items_of(h, 1), t.bx, rows_dev, h->nx, yb));
+    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
+    CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+
+int ddc_halo_scatter_shards_f64(ddc_handle_t h, const double* rows_dev)
+{
+    NEED_PARTITION(h);
+    return halo_field_shards(h, true, const_cast<double*>(rows_dev), "ddc_halo_scatter_shards_f64");
+}
+
+int ddc_halo_gather_shards_f64(ddc_handle_t h, double* rows_dev)
+{
+    NEED_PARTITION(h);
+    return halo_field_shards(h, false, rows_dev, "ddc_halo_gather_shards_f64");
 }
 
 int ddc_halo_close(ddc_handle_t h)

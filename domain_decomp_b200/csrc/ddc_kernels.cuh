@@ -2581,6 +2581,25 @@ __global__ void __launch_bounds__(32) k_halo_open(HaloShards hs, int phases)
     }
 }
 
+// The end of every middle kernel of the sharded protocol (all threads of the block): once every block has counted
+// itself, the last one stores D = k into slot [1][rank] of every rank's flags, for k_halo_close, and resets the counter.
+__device__ __forceinline__ void halo_block_done(const HaloShards& hs)
+{
+    __shared__ int s_last;
+    __syncthreads(); // every thread's accesses are issued ...
+    if (threadIdx.x == 0) {
+        __threadfence_system(); // ... and performed at the peers before the block is counted
+        s_last = atomicAdd(hs.done, 1u) == gridDim.x - 1u;
+    }
+    __syncthreads();
+    if (s_last) {
+        if ((int)threadIdx.x < hs.ps.G)
+            peer_signal(hs.ps, 1, 0u);
+        if (threadIdx.x == 0)
+            *hs.done = 0u;
+    }
+}
+
 // One warp per (list l, owned part q): q's neighbours p in list l receive q's cells in their ghosts on the opposite
 // edge.  The lists are symmetric (p is in q's edge-e list iff q is in p's opposite-edge list, same periodic flag), so
 // q's entry in p's list -- found by binary search, the lists are id-ascending -- gives the halo size and start that
@@ -2589,7 +2608,6 @@ __global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, c
     const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
     const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists)
 {
-    __shared__ int s_last;
     const int P = hs.P, G = hs.ps.G;
     const bool go = *(volatile unsigned*)hs.opened == hs.ps.step;
     // grid-stride over the warps: few enough blocks that the system fence each one pays below stays cheap
@@ -2635,18 +2653,7 @@ __global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, c
     }
     if (!go)
         return; // (block-uniform) k_halo_open timed out: no stores, no flag
-    __syncthreads(); // every thread's stores are issued ...
-    if (threadIdx.x == 0) {
-        __threadfence_system(); // ... and performed at the peers before the block is counted
-        s_last = atomicAdd(hs.done, 1u) == gridDim.x - 1u;
-    }
-    __syncthreads();
-    if (s_last) {
-        if ((int)threadIdx.x < G)
-            peer_signal(hs.ps, 1, 0u);
-        if (threadIdx.x == 0)
-            *hs.done = 0u;
-    }
+    halo_block_done(hs);
 }
 
 __global__ void __launch_bounds__(32) k_halo_close(HaloShards hs)
@@ -2658,6 +2665,131 @@ __global__ void __launch_bounds__(32) k_halo_close(HaloShards hs)
     const bool ok = q >= hs.ps.G || peer_wait(hs.ps, 1, &seen);
     if (__syncthreads_or(!ok) && q == 0)
         halo_timed_out(hs);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Halo scatter / gather: a field between its rows (double [ny][nx], x fastest) and the parts' tile interiors
+// ------------------------------------------------------------------------------------------------
+// Scatter stores field[y0 + j][x0 + i] into row j + 1, column i + 1 of part p's tile; gather is the inverse.  The work
+// is (part, interior row) items, one warp each: at C5 a part row is ~256 cells, so every warp instruction moves 256
+// contiguous bytes on both sides, and there are millions of items for 148 SMs instead of one long walk per part.
+// The host lists, per part, the interior rows that meet the field rows at hand (all of them for one buffer, the rank's
+// ddc_shard_rows block when sharded): range k is part[k]'s rows j0[k] ... for first[k + 1] - first[k] items, and its
+// tile is at element base[k] of the buffer of rank owner[k] (one buffer: owner 0, base = the ddc_halo_tile_offsets
+// offset; sharded: rebased to the owner's first part).  The host computes both: in a kernel, the 64-bit divisions that
+// find the owner are a subroutine call, and the registers saved around it spill.
+// Only non-empty ranges are listed, so first[] is strictly increasing.
+struct HaloItems {
+    const int* part; // [n]
+    const int* j0; // [n]
+    const int* owner; // [n]
+    const int* first; // [n + 1], first[0] = 0, first[n] = all items
+    const long long* base; // [n]
+    int n;
+};
+// the ranges of the field rows [lo, hi) with the parts sharded over G ranks (G = 1: one buffer) into
+// out[4 P + 1] = [part: P][j0: P][owner: P][first: P + 1] and base[P]; y0 / ex / ey: the boxes, off: the
+// ddc_halo_tile_offsets offsets.  Returns n.  Host code, shared by ddc_api.cu and the emulation harness of the tests.
+inline int halo_item_ranges(int P, int G, const int* y0, const int* ex, const int* ey, const long long* off, int lo, int hi,
+    int* out, long long* base)
+{
+    int n = 0, run = 0;
+    for (int p = 0; p < P; p++) {
+        const int a = (y0[p] > lo ? y0[p] : lo) - y0[p], b = (y0[p] + ey[p] < hi ? y0[p] + ey[p] : hi) - y0[p];
+        if (ex[p] > 0 && b > a) {
+            const int owner = (int)(((long long)(p + 1) * G - 1) / P);
+            out[n] = p;
+            out[P + n] = a;
+            out[2 * P + n] = owner;
+            out[3 * P + n] = run;
+            base[n] = off[p] - off[(long long)owner * P / G];
+            run += b - a;
+            n++;
+        }
+    }
+    out[3 * P + n] = run;
+    return n;
+}
+
+constexpr int HALO_ROW_LOADS = 8; // loads in flight per lane: a 256-cell row in one round
+// n cells between a tile row and a field row, as 64-bit words (no arithmetic: NaN payloads, -0.0, subnormals stay).
+// Every load of a round is issued before its stores: over NVLink (the sharded gather) a load is a round trip, and
+// 8 independent ones per lane keep the link busy where one dependent load at a time would not.
+template <bool kScatter>
+__device__ __forceinline__ void halo_copy_row(unsigned long long* tile, unsigned long long* row, int n, int lane)
+{
+    const unsigned long long* __restrict__ src = kScatter ? row : tile;
+    unsigned long long* __restrict__ dst = kScatter ? tile : row;
+    for (int c0 = 0; c0 < n; c0 += 32 * HALO_ROW_LOADS) {
+        unsigned long long v[HALO_ROW_LOADS];
+#pragma unroll
+        for (int u = 0; u < HALO_ROW_LOADS; u++) {
+            const int c = c0 + 32 * u + lane;
+            if (c < n)
+                v[u] = src[c];
+        }
+#pragma unroll
+        for (int u = 0; u < HALO_ROW_LOADS; u++) {
+            const int c = c0 + 32 * u + lane;
+            if (c < n)
+                dst[c] = v[u];
+        }
+    }
+}
+// every item of `it`.  Warp g takes the contiguous items [g c, (g + 1) c), c = ceil(items / warps): one binary search
+// for its first range, then row after row -- the next row's addresses are arithmetic, so its loads issue right behind
+// the previous row's stores, and a part's box and tile are looked up only when the walk enters the part (DESIGN.md 7).
+// tile_of(k): the tile of range k; field: the row y_base of the field
+template <bool kScatter, typename TileOf>
+__device__ __forceinline__ void halo_copy_items(const HaloItems& it, BoxTable bx, TileOf tile_of, double* field, int nx, int y_base)
+{
+    const unsigned total = (unsigned)it.first[it.n], warps = gridDim.x * (blockDim.x >> 5);
+    const unsigned chunk = total / warps + (total % warps != 0u);
+    const unsigned g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const unsigned long long w0 = (unsigned long long)g * chunk;
+    if (w0 >= total)
+        return;
+    const int end = (int)min((unsigned long long)total, w0 + chunk), lane = lane_id();
+    int w = (int)w0, k = 0, hi = it.n - 1; // k: the range with first[k] <= w < first[k + 1]
+    while (k < hi) {
+        const int mid = (k + hi + 1) >> 1;
+        if (it.first[mid] <= w)
+            k = mid;
+        else
+            hi = mid - 1;
+    }
+    while (w < end) {
+        const int p = it.part[k], ex = bx.ex[p], stop = min(end, it.first[k + 1]);
+        int j = it.j0[k] + (w - it.first[k]);
+        unsigned long long* tile = reinterpret_cast<unsigned long long*>(tile_of(k)) + (size_t)(j + 1) * (ex + 2) + 1;
+        unsigned long long* row = reinterpret_cast<unsigned long long*>(field) + (size_t)(bx.y0[p] + j - y_base) * nx + bx.x0[p];
+        for (; w < stop; w++, tile += ex + 2, row += nx)
+            halo_copy_row<kScatter>(tile, row, ex, lane);
+        k++;
+    }
+}
+
+// one buffer with every part's tile at tiles + off[p] (ddc_halo_tile_offsets); field: the whole double [ny][nx]
+template <bool kScatter>
+__global__ void __launch_bounds__(256) k_halo_field(HaloItems it, BoxTable bx, double* tiles, double* field, int nx)
+{
+    halo_copy_items<kScatter>(it, bx, [&](int k) { return tiles + it.base[k]; }, field, nx, 0);
+}
+
+// The sharded scatter / gather: the middle kernel between k_halo_open and k_halo_close.  rows: this rank's
+// ddc_shard_rows block, starting at field row y_begin; `it` lists the parts' rows inside it, whoever owns the part.
+// Scatter reads the rows locally and stores into the owners' tiles (posted remote stores, as k_halo_push); gather
+// loads from the owners' tiles and stores into the rows, which only this rank maps (they are the caller's memory).
+// Its D flag therefore also says "this rank has finished reading every rank's tiles": after k_halo_close no kernel a
+// caller runs next on any rank can overwrite a cell that is still being read.
+template <bool kScatter>
+__global__ void __launch_bounds__(256) k_halo_field_shards(HaloShards hs, HaloItems it, BoxTable bx, double* rows, int nx,
+    int y_begin)
+{
+    if (*(volatile unsigned*)hs.opened != hs.ps.step)
+        return; // (grid-uniform) k_halo_open timed out: nothing touched, no flag
+    halo_copy_items<kScatter>(it, bx, [&](int k) { return hs.tiles[it.owner[k]] + it.base[k]; }, rows, nx, y_begin);
+    halo_block_done(hs);
 }
 
 // ------------------------------------------------------------------------------------------------

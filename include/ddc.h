@@ -217,6 +217,32 @@ DDC_API int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic);
    host synchronises the ranks, then every rank calls ddc_destroy(), which frees its own halo buffer. */
 DDC_API int ddc_halo_close(ddc_handle_t h);
 
+/* Halo scatter and gather: a field between its rows and the parts' tiles.  A field is double [ny][nx], x fastest, the
+   layout of the mask and the pid map; rank r of a sharded run holds rows [y_begin, y_begin + y_count) of
+   ddc_shard_rows(ny, nranks, r).  Scatter writes the INTERIOR of every tile from the field: row j + 1, column i + 1 of
+   part p's tile gets field[y0[p] + j][x0[p] + i].  Gather is the inverse: it reads interiors only and writes every
+   cell of the field (or of this rank's rows) exactly once -- the boxes tile the whole domain, land included.  Neither
+   reads nor writes a ghost frame.  Values are copied bit for bit (NaN payloads, -0.0, subnormals): no arithmetic.
+   Single buffer (the ddc_halo_exchange_f64 layout, all parts): field_dev is the whole field.  Needs
+   ddc_halo_tile_offsets for the current decomposition (else DDC_ERR_STATE) and non-null pointers (else DDC_ERR_ARG);
+   it does NOT need neighbour tables: with one part, or without DDC_WANT_NEIGHBOURS, the whole field still moves.
+   Sharded (the ddc_halo_exchange_shards_f64 buffers): rows_dev is this rank's row block; scatter stores every cell of
+   it into its part's tile on whichever rank owns the part (posted stores), gather loads every cell of it from there.
+   The buffers, shard offsets and capacity are checked as for the exchange, with the same status codes, from
+   replicated data and before anything is enqueued, so they come out the same on every rank.  One check is this
+   rank's alone: rows_dev == NULL on a rank whose block has rows is DDC_ERR_ARG on that rank (NULL is fine for an empty
+   block: ddc_shard_rows' ceil rule leaves the last ranks empty when ny is small).  Its peers then wait for it in vain
+   and ddc_synchronize reports DDC_ERR_PEER on them, as for a rank that never makes the call.
+   Scatter and gather are sharded halo calls like the exchange: each takes the next halo step number, behind the same
+   two flag barriers, so every rank must make the same sequence of sharded halo calls; exchanges, scatters and gathers
+   may be mixed freely as long as the order is the same on every rank.  After a sharded gather returns on the stream,
+   no rank still reads this rank's tiles.  The calls only enqueue (on the handle's stream), so one host thread can
+   drive several handles. */
+DDC_API int ddc_halo_scatter_f64(ddc_handle_t h, const double* field_dev, double* tiles_dev);
+DDC_API int ddc_halo_gather_f64(ddc_handle_t h, const double* tiles_dev, double* field_dev);
+DDC_API int ddc_halo_scatter_shards_f64(ddc_handle_t h, const double* rows_dev);
+DDC_API int ddc_halo_gather_shards_f64(ddc_handle_t h, double* rows_dev);
+
 /* ---- synthetic masks (SURVEY 8d): deterministic value-noise land-sea mask, generated directly
    into device memory so that no 4 GiB file is needed for the large configurations.
    land_frac in [0,1] is the target land fraction; rows as in ddc_set_mask_device. */

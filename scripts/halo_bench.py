@@ -1,16 +1,20 @@
 #!/usr/bin/env python
-"""Time the halo exchanges on the BASELINE decompositions C4 (8192^2 -> 4096 parts) and C5 (32768^2 -> 16384, px).
+"""Time the halo exchanges, scatters and gathers on the BASELINE decompositions C4 (8192^2 -> 4096 parts) and C5
+(32768^2 -> 16384, px).
 
     python scripts/halo_bench.py --out result.json                   # one GPU
     torchrun --nproc-per-node G scripts/halo_bench.py --out r.json    # G GPUs, one process each
 
 One GPU: ddc_halo_exchange_f64 on one buffer against ddc_halo_exchange_shards_f64 with one rank (the same ghost
-cells, plus the open / close barriers of the sharded protocol), alternated in rounds.  G GPUs: the sharded exchange
-over CUDA IPC, time per exchange = the slowest rank's.  Times are CUDA events around `--iters` back-to-back
-exchanges after `--warmup` (enqueue included: it is what a caller pays).  Exchanges are periodic (the periodic lists
-are used where the decomposition has them).  Ghost cells moved come from the neighbour tables: a cell is read once
-(8 B) and written once (8 B); "cross-rank" cells are written into another rank's buffer.  The GPU name and power
-limit are read in the same run.  Writes JSON to --out (and prints it); nothing in the tree."""
+cells, plus the open / close barriers of the sharded protocol), and ddc_halo_scatter_f64 / ddc_halo_gather_f64 against
+their sharded forms with one rank, all alternated in rounds.  G GPUs: the sharded calls over CUDA IPC, time per call =
+the slowest rank's.  Times are CUDA events around `--iters` back-to-back calls after `--warmup` (enqueue included: it
+is what a caller pays).  Exchanges are periodic (the periodic lists are used where the decomposition has them).  Ghost
+cells moved come from the neighbour tables: a cell is read once (8 B) and written once (8 B); "cross-rank" cells are
+written into another rank's buffer.  Scatter and gather move every cell of the field (nx ny cells, 8 B read + 8 B
+written each); their "cross-rank" cells are those whose row (ddc_shard_rows) and part (ddc_shard_parts) belong to
+different ranks.  Rates are compared with the 6546.9 GB/s of a read+write copy measured on a B200 (DESIGN.md 4).  The
+GPU name and power limit are read in the same run.  Writes JSON to --out (and prints it); nothing in the tree."""
 import argparse
 import json
 import os
@@ -25,6 +29,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from domain_decomp_b200 import capi  # noqa: E402
 
+COPY_GBPS = 6546.9  # a read+write device copy on a B200 (MEASURED_PEAKS.json:hbm_gbs, DESIGN.md 4)
 CONFIGS = {  # tests/golden/bench_digests.json
     "C4": dict(nx=8192, ny=8192, parts=4096, seed=1, land_frac=0.6, px=0, py=0),
     "C5": dict(nx=32768, ny=32768, parts=16384, seed=32, land_frac=0.45, px=1, py=0),
@@ -54,6 +59,28 @@ def ghost_counts(h, P, G, periodic):
             total += int(halos.sum())
             cross += int(halos[owner(recv) != owner(ids.astype(np.int64))].sum())
     return total, cross
+
+
+def field_counts(boxes, ny, P, G):
+    """cells a scatter / gather moves: (all, those whose row block and part belong to different ranks)"""
+    b = np.asarray(boxes, dtype=np.int64)
+    y0, ex, ey = b[:, 1], np.maximum(b[:, 2], 0), np.maximum(b[:, 3], 0)
+    owner = ((np.arange(P, dtype=np.int64) + 1) * G - 1) // P
+    local = np.zeros(P, dtype=np.int64)  # rows of each part inside its owner's row block
+    for r in range(G):
+        yb, yc = capi.shard_rows(ny, G, r)
+        mine = owner == r
+        local[mine] = np.clip(np.minimum(y0 + ey, yb + yc) - np.maximum(y0, yb), 0, None)[mine]
+    return int((ex * ey).sum()), int((ex * (ey - local)).sum())
+
+
+def field_row(name, cfg, G, variant, ms, cells, cross):
+    bytes_moved = 16 * cells  # 8 B read + 8 B written per cell
+    gbps = bytes_moved / (ms * 1e-3) / 1e9
+    return dict(config=name, nx=cfg["nx"], ny=cfg["ny"], parts=cfg["parts"], ranks=G, variant=variant,
+                ms_per_call=round(ms, 5), cells=cells, cells_cross_rank=cross, bytes_read=8 * cells,
+                bytes_written=8 * cells, bytes_cross_rank=16 * cross, achieved_GBps=round(gbps, 1),
+                share_of_copy_rate=round(gbps / COPY_GBPS, 4))
 
 
 def timed(fn, stream, iters):
@@ -101,23 +128,32 @@ def one_gpu(args):
         (ptr,) = capi.halo_connect([h], int(off[-1]))
         h.halo_shard_offsets()
         cells, cross = ghost_counts(h, P, 1, True)
+        fcells, fcross = field_counts(h.boxes(), cfg["ny"], P, 1)
+        field = torch.zeros((cfg["ny"], cfg["nx"]), dtype=torch.float64, device=dev)
+        back = torch.zeros_like(field)
         variants = {"single_buffer": lambda: h.halo_exchange_f64(single.data_ptr(), True),
-                    "sharded_G1": lambda: h.halo_exchange_shards_f64(True)}
+                    "sharded_G1": lambda: h.halo_exchange_shards_f64(True),
+                    "scatter_single_buffer": lambda: h.halo_scatter_f64(field.data_ptr(), single.data_ptr()),
+                    "gather_single_buffer": lambda: h.halo_gather_f64(single.data_ptr(), back.data_ptr()),
+                    "scatter_sharded_G1": lambda: h.halo_scatter_shards_f64(field.data_ptr()),
+                    "gather_sharded_G1": lambda: h.halo_gather_shards_f64(back.data_ptr())}
         for fn in variants.values():
             timed(fn, stream, args.warmup)
         samples = {k: [] for k in variants}
-        for _ in range(args.rounds):  # alternated: the two share whatever else the machine does
+        for _ in range(args.rounds):  # alternated: the variants share whatever else the machine does
             for k, fn in variants.items():
                 samples[k].append(timed(fn, stream, args.iters))
         h.synchronize()
         for k in variants:
-            r = row(name, cfg, 1, float(np.median(samples[k])), cells, cross)
+            ms = float(np.median(samples[k]))
+            r = row(name, cfg, 1, ms, cells, cross) if k in ("single_buffer", "sharded_G1") else \
+                field_row(name, cfg, 1, k, ms, fcells, fcross)
             r.update(variant=k, samples_ms=[round(s, 5) for s in samples[k]], iters=args.iters)
             results.append(r)
             print(json.dumps(r), flush=True)
         h.halo_close()
         h.close()
-        del single
+        del single, field, back
         torch.cuda.empty_cache()
     return results
 
@@ -149,19 +185,29 @@ def multi_gpu(args):
         h.halo_import(handles)
         h.halo_shard_offsets()
         cells, cross = ghost_counts(h, P, world, True)
-        fn = lambda: h.halo_exchange_shards_f64(True)
-        timed(fn, stream, args.warmup)
-        samples = []
+        fcells, fcross = field_counts(h.boxes(), cfg["ny"], P, world)
+        yb, yc = capi.shard_rows(cfg["ny"], world, rank)
+        rows = torch.zeros((max(yc, 1), cfg["nx"]), dtype=torch.float64, device=dev)
+        variants = {"sharded": lambda: h.halo_exchange_shards_f64(True),
+                    "scatter_sharded": lambda: h.halo_scatter_shards_f64(rows.data_ptr()),
+                    "gather_sharded": lambda: h.halo_gather_shards_f64(rows.data_ptr())}
+        for fn in variants.values():
+            timed(fn, stream, args.warmup)
+        samples = {k: [] for k in variants}
         for _ in range(args.rounds):
-            dist.barrier()
-            samples.append(timed(fn, stream, args.iters))
-        t = torch.tensor(samples, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)  # per round: the slowest rank
-        r = row(name, cfg, world, float(np.median(t.cpu().numpy())), cells, cross)
-        r.update(variant="sharded", samples_ms=[round(float(s), 5) for s in t.cpu()], iters=args.iters)
-        results.append(r)
-        if rank == 0:
-            print(json.dumps(r), flush=True)
+            for k, fn in variants.items():
+                dist.barrier()
+                samples[k].append(timed(fn, stream, args.iters))
+        for k in variants:
+            t = torch.tensor(samples[k], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)  # per round: the slowest rank
+            ms = float(np.median(t.cpu().numpy()))
+            r = row(name, cfg, world, ms, cells, cross) if k == "sharded" else field_row(name, cfg, world, k, ms, fcells, fcross)
+            r.update(variant=k, samples_ms=[round(float(s), 5) for s in t.cpu()], iters=args.iters)
+            results.append(r)
+            if rank == 0:
+                print(json.dumps(r), flush=True)
+        del rows
         h.halo_close()
         h.peer_close()
         dist.barrier()

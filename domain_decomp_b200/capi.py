@@ -16,6 +16,8 @@ LIB_PATH = os.path.join(_PKG, "libddc_cuda.so")
 
 LEFT, RIGHT, BOTTOM, TOP = 0, 1, 2, 3
 EDGE_NAMES = ("left", "right", "bottom", "top")
+BOTTOM_LEFT, BOTTOM_RIGHT, TOP_LEFT, TOP_RIGHT = 0, 1, 2, 3
+CORNER_NAMES = ("bottom_left", "bottom_right", "top_left", "top_right")
 WANT_PID, WANT_NEIGHBOURS, PROFILE, ASYNC = 1, 2, 4, 8
 NCCL_ID_BYTES = 128
 IPC_HANDLE_BYTES = 64
@@ -33,6 +35,7 @@ SYMBOLS = (
     "ddc_shard_parts", "ddc_halo_shard_offsets", "ddc_halo_export", "ddc_halo_import", "ddc_halo_connect",
     "ddc_halo_exchange_shards_f64", "ddc_halo_close",
     "ddc_halo_scatter_f64", "ddc_halo_gather_f64", "ddc_halo_scatter_shards_f64", "ddc_halo_gather_shards_f64",
+    "ddc_get_corner_neighbours", "ddc_halo_exchange_full_f64", "ddc_halo_exchange_full_shards_f64",
 )
 
 
@@ -111,6 +114,9 @@ def load() -> C.CDLL:
     L.ddc_halo_gather_f64.argtypes = [vp, vp, vp]
     L.ddc_halo_scatter_shards_f64.argtypes = [vp, vp]
     L.ddc_halo_gather_shards_f64.argtypes = [vp, vp]
+    L.ddc_get_corner_neighbours.argtypes = [vp, i32, i32, vp, vp]
+    L.ddc_halo_exchange_full_f64.argtypes = [vp, vp, i32]
+    L.ddc_halo_exchange_full_shards_f64.argtypes = [vp, i32]
     L.ddc_generate_mask_device.argtypes = [vp, vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     L.ddc_generate_mask_host.argtypes = [vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     _lib = L
@@ -315,6 +321,22 @@ class Handle:
     def halo_gather_shards_f64(self, rows_ptr: int):
         """this rank's rows (device double [y_count][nx] of shard_rows) <- every rank's tile interiors"""
         self._ck(self.L.ddc_halo_gather_shards_f64(self.h, rows_ptr), "ddc_halo_gather_shards_f64")
+
+    def corner_neighbours(self, corner: int, periodic: int):
+        """(ids, starts), int32[nparts] each: the source part of every part's corner `corner` (-1: none) and the
+        source cell's index in that part's flattened box (ddc_get_corner_neighbours)"""
+        ids, starts = np.empty(self.nparts, dtype=np.int32), np.empty(self.nparts, dtype=np.int32)
+        self._ck(self.L.ddc_get_corner_neighbours(self.h, corner, int(periodic), ids.ctypes.data, starts.ctypes.data),
+                 "ddc_get_corner_neighbours")
+        return ids, starts
+
+    def halo_exchange_full_f64(self, tiles_dev_ptr: int, periodic: bool = False):
+        """halo_exchange_f64 plus the corner ghosts: the whole frame of every tile"""
+        self._ck(self.L.ddc_halo_exchange_full_f64(self.h, tiles_dev_ptr, int(periodic)), "ddc_halo_exchange_full_f64")
+
+    def halo_exchange_full_shards_f64(self, periodic: bool = False):
+        """halo_exchange_shards_f64 plus the corner ghosts"""
+        self._ck(self.L.ddc_halo_exchange_full_shards_f64(self.h, int(periodic)), "ddc_halo_exchange_full_shards_f64")
 
     def neighbour_counts(self, edge: int, periodic: int) -> np.ndarray:
         out = np.empty(self.nparts, dtype=np.int32)

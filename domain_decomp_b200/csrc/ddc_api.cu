@@ -191,6 +191,12 @@ struct ddc_handle_s {
     DevBuf<int> halo_items; // [2][4 P + 1]
     DevBuf<long long> halo_item_base; // [2][P]
     int halo_items_n[2] = { 0, 0 }, halo_items_total[2] = { 0, 0 };
+    // the corner items of the full-frame exchange (HaloCorners), built with them: [0] one buffer, [1] the items whose
+    // source part this rank owns; each [src 4 P][dst 4 P] (+ [4 P] destination ranks), the interior set first
+    DevBuf<long long> halo_corner_ix; // [2][8 P]
+    DevBuf<int> halo_corner_rank; // [2][4 P]
+    int halo_corner_n[2][2] = {}; // [view][0: interior set, 1: both sets]
+    bool halo_corner_ok = false; // built for the current boxes and periodic flags
     DevBuf<unsigned> gate; // the word the gate kernel of the second stream waits for (see BoxGate)
     int use_gate = 1; // DDC_GATE: 0 never, 1 unless the shard is tiny, 2 always
     bool side_pdl = true; // DDC_SIDE_PDL: the scan of the neighbour counts launched programmatically behind the count kernel
@@ -704,6 +710,8 @@ int ddc_destroy(ddc_handle_t h)
     h->sc.release();
     h->gate.release();
     h->halo_off.release();
+    h->halo_corner_ix.release();
+    h->halo_corner_rank.release();
     h->halo_items.release();
     h->halo_item_base.release();
     h->plan.release();
@@ -1022,6 +1030,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     h->small_cached = h->lists_cached = false;
     h->halo_parts = 0;
     h->halo_shard_ok = false;
+    h->halo_corner_ok = false;
     memset(&h->stats, 0, sizeof h->stats);
     int launches = 0;
     // stage i begins: a CUDA event when profiling, and an NVTX range (the host-side enqueue of the stage; Nsight
@@ -1754,6 +1763,7 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
     h->py = py;
     h->mask_set = false; // the mask (if any) has to be set again before the next ddc_partition
     h->halo_shard_ok = false;
+    h->halo_corner_ok = false;
     h->d_mask = nullptr;
     h->pending = false;
     int rc = run_neighbours(h, P, nx, ny, px, py);
@@ -1772,15 +1782,35 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
 // ------------------------------------------------------------------------------------------------
 // halo exchange (a consumer of the neighbour tables)
 // ------------------------------------------------------------------------------------------------
+// the corner source table of the current boxes (halo_corner_sources): ids / starts [2][4][P]
+static int corner_sources(ddc_handle_t h, std::vector<int32_t> box[4], std::vector<int>& ids, std::vector<int>& starts)
+{
+    const int P = h->nparts;
+    for (int i = 0; i < 4; i++)
+        box[i].resize(P);
+    if (int rc = ddc_get_boxes(h, box[0].data(), box[1].data(), box[2].data(), box[3].data()))
+        return rc;
+    ids.resize((size_t)8 * P);
+    starts.resize((size_t)8 * P);
+    halo_corner_sources(P, h->nx, h->ny, h->px, h->py, box[0].data(), box[1].data(), box[2].data(), box[3].data(),
+        ids.data(), starts.data());
+    return DDC_OK;
+}
+
 // the tile offsets of all parts in one buffer (offsets[P] = total), also left on the device for the exchange kernels,
-// and beside them the (part, row) ranges of scatter and gather: every field row, and this rank's ddc_shard_rows
+// and beside them the (part, row) ranges of scatter and gather (every field row, and this rank's ddc_shard_rows) and
+// the corner items of the full-frame exchange.  Everything is built here, where the host may wait for the stream: a
+// sharded call must not wait (one host thread may drive several ranks, whose open kernels wait for each other).
 static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
 {
     const int P = h->nparts;
-    std::vector<int32_t> y0(P), ex(P), ey(P);
-    int rc = ddc_get_boxes(h, nullptr, y0.data(), ex.data(), ey.data());
-    if (rc)
+    std::vector<int32_t> box[4];
+    std::vector<int> cids, cstarts;
+    if (int rc = corner_sources(h, box, cids, cstarts))
         return rc;
+    const std::vector<int32_t>& y0 = box[1];
+    const std::vector<int32_t>& ex = box[2];
+    const std::vector<int32_t>& ey = box[3];
     off.assign((size_t)P + 1, 0);
     long long run = 0;
     for (int p = 0; p < P; p++) {
@@ -1805,9 +1835,28 @@ static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
     CUDA_TRY(h, cudaMemcpyAsync(h->halo_off.p, off.data(), sizeof(long long) * ((size_t)P + 1), cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaMemcpyAsync(h->halo_items.p, items.data(), sizeof(int) * 2 * per, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaMemcpyAsync(h->halo_item_base.p, base.data(), sizeof(long long) * 2 * P, cudaMemcpyHostToDevice, h->stream));
+    const size_t cp = (size_t)4 * P;
+    std::vector<long long> cix(4 * cp);
+    std::vector<int> crank(2 * cp);
+    for (int s = 0; s < 2; s++)
+        halo_corner_items(P, s ? h->nranks : 1, s ? h->rank : 0, cids.data(), cstarts.data(), ex.data(), ey.data(), off.data(),
+            cix.data() + 2 * s * cp, cix.data() + (2 * s + 1) * cp, crank.data() + s * cp, h->halo_corner_n[s]);
+    CUDA_TRY(h, h->halo_corner_ix.ensure(4 * cp));
+    CUDA_TRY(h, h->halo_corner_rank.ensure(2 * cp));
+    CUDA_TRY(h, cudaMemcpyAsync(h->halo_corner_ix.p, cix.data(), sizeof(long long) * 4 * cp, cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->halo_corner_rank.p, crank.data(), sizeof(int) * 2 * cp, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->halo_parts = P;
+    h->halo_corner_ok = true;
     return DDC_OK;
+}
+
+// the corner items of view s (0 one buffer, 1 this rank's sources); periodic: both sets, else the interior set
+static HaloCorners halo_corners_of(ddc_handle_t h, int s, int periodic)
+{
+    const size_t cp = (size_t)4 * h->nparts;
+    return HaloCorners { h->halo_corner_ix.p + 2 * s * cp, h->halo_corner_ix.p + (2 * s + 1) * cp,
+        s ? h->halo_corner_rank.p + cp : nullptr, h->halo_corner_n[s][periodic ? 1 : 0] };
 }
 
 int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
@@ -1823,13 +1872,32 @@ int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
     return DDC_OK;
 }
 
-int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic)
+// the source part and cell of one corner of every part (computed on the host from the boxes)
+int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, int32_t* ids, int32_t* starts)
 {
     NEED_PARTITION(h);
+    if (corner < 0 || corner >= DDC_N_CORNER || periodic < 0 || periodic > 1)
+        return fail(h, DDC_ERR_ARG, "ddc_get_corner_neighbours: corner must be 0..3 and periodic 0/1");
+    std::vector<int32_t> box[4];
+    std::vector<int> cids, cstarts;
+    if (int rc = corner_sources(h, box, cids, cstarts))
+        return rc;
+    const size_t P = h->nparts, at = ((size_t)periodic * 4 + corner) * P;
+    if (ids)
+        memcpy(ids, cids.data() + at, P * sizeof(int32_t));
+    if (starts)
+        memcpy(starts, cstarts.data() + at, P * sizeof(int32_t));
+    return DDC_OK;
+}
+
+constexpr int HALO_CORNER_BLOCKS = 4 * 148; // k_halo_corners' grid at most (grid-stride): 4 P items, 64 K at C5
+// one buffer: the edge ghosts (k_halo_exchange), and with `full` the corner ghosts after them (k_halo_corners)
+static int halo_exchange(ddc_handle_t h, double* tiles_dev, int periodic, bool full, const char* name)
+{
     if (!tiles_dev)
-        return fail(h, DDC_ERR_ARG, "ddc_halo_exchange_f64: null tiles");
-    if (h->halo_parts != h->nparts)
-        return fail(h, DDC_ERR_STATE, "ddc_halo_exchange_f64: call ddc_halo_tile_offsets() for this decomposition first");
+        return fail(h, DDC_ERR_ARG, "%s: null tiles", name);
+    if (h->halo_parts != h->nparts || (full && !h->halo_corner_ok))
+        return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_tile_offsets() for this decomposition first", name);
     if (!h->have_nbr)
         return DDC_OK; // one part (or no tables asked for): nothing to exchange
     int rc = fetch_totals(h); // (re-runs the fill pass with the exact capacity if the bounded one overflowed)
@@ -1841,8 +1909,24 @@ int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic)
     CUDA_TRY(h, launch_k(k_halo_exchange<double>, dim3((unsigned)((warps * 32 + 255) / 256)), dim3(256), 0, h->stream, false, t.bx, P,
         h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, tiles_dev,
         periodic ? 0xffu : 0x0fu));
+    const HaloCorners corners = halo_corners_of(h, 0, periodic);
+    if (full && corners.n > 0) // (corners read interiors only: no order with the edges is needed)
+        CUDA_TRY(h, launch_k(k_halo_corners, dim3((unsigned)std::min((corners.n + 255) / 256, HALO_CORNER_BLOCKS)), dim3(256), 0,
+            h->stream, false, corners, tiles_dev));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;
+}
+
+int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic)
+{
+    NEED_PARTITION(h);
+    return halo_exchange(h, tiles_dev, periodic, false, "ddc_halo_exchange_f64");
+}
+
+int ddc_halo_exchange_full_f64(ddc_handle_t h, double* tiles_dev, int periodic)
+{
+    NEED_PARTITION(h);
+    return halo_exchange(h, tiles_dev, periodic, true, "ddc_halo_exchange_full_f64");
 }
 
 // halo scatter / gather: the field rows <-> the tile interiors (k_halo_field, k_halo_field_shards)
@@ -1931,6 +2015,7 @@ static int halo_alloc(ddc_handle_t h, int64_t elems)
     cudaFuncAttributes fa;
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_open));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_push));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_push_full));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_close));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<true>));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<false>));
@@ -2040,6 +2125,28 @@ int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
     CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
     CUDA_TRY(h, launch_k(k_halo_push, dim3((unsigned)std::max(1, std::min(hs.p_count, HALO_PUSH_BLOCKS))), dim3(256), 0, h->stream, false, hs, t.bx,
         h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, lists));
+    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
+    CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+
+int ddc_halo_exchange_full_shards_f64(ddc_handle_t h, int periodic)
+{
+    NEED_PARTITION(h);
+    if (int rc = halo_shards_ready(h, "ddc_halo_exchange_full_shards_f64")) // (halo_shard_ok: the corner items are current)
+        return rc;
+    if (!h->have_nbr)
+        return DDC_OK; // as ddc_halo_exchange_shards_f64: nothing to exchange, no step taken
+    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
+        return rc;
+    Tables t = tables(h, h->nparts);
+    const HaloShards hs = halo_shards_next(h);
+    const HaloCorners corners = halo_corners_of(h, 1, periodic);
+    const int grid = std::max(1, std::min(std::max(hs.p_count, (corners.n + 255) / 256), HALO_PUSH_BLOCKS));
+    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
+    CUDA_TRY(h, launch_k(k_halo_push_full, dim3((unsigned)grid), dim3(256), 0, h->stream, false, hs, t.bx, h->nbr_counts.p,
+        h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, periodic ? 0xffu : 0x0fu,
+        corners));
     CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;

@@ -30,6 +30,9 @@
 #endif
 #include <stdint.h>
 
+#include <algorithm>
+#include <vector>
+
 #include "ddc_median.cuh"
 #include "ddc_neighbours.cuh"
 
@@ -2481,8 +2484,9 @@ __global__ void __launch_bounds__(256) k_init(unsigned* __restrict__ colcount, i
 // -- tile p is a row-major (ext_y + 2) x (ext_x + 2) array with a ghost frame of one cell, at tiles[off[p]] -- and one
 // warp per (edge list, part) walks the part's CSR entries: neighbour id, halo size and halo START (the index of
 // the first shared cell in the neighbour's flattened box, Partitioner.cpp:55-80) locate the source cells, the
-// overlap of the two boxes the ghost cells.  Corners are not exchanged (a corner-touching box is no neighbour,
-// DomainUtils.cpp:15-35).  lists: bit l set = use list l (l = periodic * 4 + edge).
+// overlap of the two boxes the ghost cells.  Corners are not exchanged here (a corner-touching box is no neighbour,
+// DomainUtils.cpp:15-35); the full-frame exchange adds them with k_halo_corners.  lists: bit l set = use list l
+// (l = periodic * 4 + edge).
 template <typename T>
 __global__ void __launch_bounds__(256) k_halo_exchange(BoxTable bx, int P, const int* __restrict__ counts,
     const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
@@ -2600,13 +2604,26 @@ __device__ __forceinline__ void halo_block_done(const HaloShards& hs)
     }
 }
 
+// The corner ghosts of the full-frame exchange as a list of 64-bit word copies: item i copies word src[i] of this
+// rank's tiles (one buffer: of the buffer) into word dst[i] of rank rank[i]'s tiles.  The host builds the list from
+// the boxes (halo_corner_items), so the kernels neither locate a corner's source nor divide.
+struct HaloCorners {
+    const long long* src; // [n]
+    const long long* dst; // [n]
+    const int* rank; // [n]; nullptr for one buffer
+    int n;
+};
+
 // One warp per (list l, owned part q): q's neighbours p in list l receive q's cells in their ghosts on the opposite
 // edge.  The lists are symmetric (p is in q's edge-e list iff q is in p's opposite-edge list, same periodic flag), so
 // q's entry in p's list -- found by binary search, the lists are id-ascending -- gives the halo size and start that
 // k_halo_exchange uses for that ghost run, and the cells and values written are exactly the ones it writes.
-__global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, const int* __restrict__ counts,
+// kCorners (the full-frame exchange): then one thread per corner item whose source part this rank owns, a local load
+// and a posted store into the receiver's tile.  Edges and corners write disjoint cells and read interiors only.
+template <bool kCorners>
+__device__ __forceinline__ void halo_push(const HaloShards& hs, BoxTable bx, const int* __restrict__ counts,
     const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
-    const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists)
+    const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists, const HaloCorners& corners)
 {
     const int P = hs.P, G = hs.ps.G;
     const bool go = *(volatile unsigned*)hs.opened == hs.ps.step;
@@ -2651,9 +2668,30 @@ __global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, c
             }
         }
     }
+    if constexpr (kCorners) {
+        const int n = go ? corners.n : 0;
+        const unsigned long long* local = reinterpret_cast<const unsigned long long*>(hs.tiles[hs.ps.rank]);
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+            reinterpret_cast<unsigned long long*>(hs.tiles[corners.rank[i]])[corners.dst[i]] = local[corners.src[i]];
+    }
     if (!go)
         return; // (block-uniform) k_halo_open timed out: no stores, no flag
     halo_block_done(hs);
+}
+
+__global__ void __launch_bounds__(256) k_halo_push(HaloShards hs, BoxTable bx, const int* __restrict__ counts,
+    const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
+    const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists)
+{
+    halo_push<false>(hs, bx, counts, offsets, cap, ids, halos, starts, off, lists, HaloCorners {});
+}
+
+// the middle kernel of the sharded full-frame exchange: k_halo_push's edges plus the corner items of this rank
+__global__ void __launch_bounds__(256) k_halo_push_full(HaloShards hs, BoxTable bx, const int* __restrict__ counts,
+    const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
+    const int* __restrict__ starts, const long long* __restrict__ off, unsigned lists, HaloCorners corners)
+{
+    halo_push<true>(hs, bx, counts, offsets, cap, ids, halos, starts, off, lists, corners);
 }
 
 __global__ void __launch_bounds__(32) k_halo_close(HaloShards hs)
@@ -2790,6 +2828,116 @@ __global__ void __launch_bounds__(256) k_halo_field_shards(HaloShards hs, HaloIt
         return; // (grid-uniform) k_halo_open timed out: nothing touched, no flag
     halo_copy_items<kScatter>(it, bx, [&](int k) { return hs.tiles[it.owner[k]] + it.base[k]; }, rows, nx, y_begin);
     halo_block_done(hs);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Corner ghosts: the four frame cells diagonally across a box's corners (the full-frame exchange)
+// ------------------------------------------------------------------------------------------------
+// Corner c of part p (ddc.h: BOTTOM_LEFT 0, BOTTOM_RIGHT 1, TOP_LEFT 2, TOP_RIGHT 3) is the cell
+// x = (c & 1 ? x0 + ex : x0 - 1), y = (c & 2 ? y0 + ey : y0 - 1), at tile row (c & 2 ? ey + 1 : 0), column
+// (c & 1 ? ex + 1 : 0).  Its source is the lowest-id box of positive area that contains the cell -- for an interior
+// corner (the cell lies in [0, nx) x [0, ny)) the cell itself, for a periodic one the cell wrapped in the directions in
+// which it lies outside, all of which must be periodic.  A box that touches p only at a corner has no domain overlap
+// with p, so no edge list names it, and zero-area parts have no lists at all: the owner is found by point location.
+// Host code, shared by ddc_api.cu and the emulation harness of the tests.
+//   ids / starts [2][4][P]: set (0 interior, 1 periodic), corner, part -> source part (-1: none) and the cell's index
+//   (y - y0[q]) * ex[q] + (x - x0[q]) in the source's flattened box (the halo_start convention).  For each (corner,
+//   part) at most one of the two sets has a source.
+inline void halo_corner_sources(int P, int nx, int ny, int px, int py, const int* x0, const int* y0, const int* ex,
+    const int* ey, int* ids, int* starts)
+{
+    // A bucket grid of about sqrt(P) x sqrt(P) over the domain; every positive-area box is registered, in id order, in
+    // each bucket it overlaps, so the first box of a bucket that contains a cell is its lowest-id source.  About one
+    // bucket per box for RCB output; still correct (only slower) for overlapping or degenerate caller boxes.
+    int side = 1;
+    while ((long long)side * side < P)
+        side++;
+    const int bw = std::min(side, nx), bh = std::min(side, ny);
+    const auto bucket_x = [&](int x) { return (int)((long long)x * bw / nx); };
+    const auto bucket_y = [&](int y) { return (int)((long long)y * bh / ny); };
+    std::vector<int> first((size_t)bw * bh + 1, 0), list;
+    for (int pass = 0; pass < 2; pass++) {
+        std::vector<int> fill(first.begin(), first.end() - 1);
+        for (int q = 0; q < P; q++) {
+            const int xa = std::max(x0[q], 0), xb = (int)std::min((long long)x0[q] + ex[q], (long long)nx) - 1;
+            const int ya = std::max(y0[q], 0), yb = (int)std::min((long long)y0[q] + ey[q], (long long)ny) - 1;
+            if (ex[q] <= 0 || ey[q] <= 0 || xa > xb || ya > yb)
+                continue;
+            for (int j = bucket_y(ya); j <= bucket_y(yb); j++)
+                for (int i = bucket_x(xa); i <= bucket_x(xb); i++) {
+                    if (pass == 0)
+                        first[(size_t)j * bw + i + 1]++;
+                    else
+                        list[fill[(size_t)j * bw + i]++] = q;
+                }
+        }
+        if (pass == 0) {
+            for (size_t b = 0; b < (size_t)bw * bh; b++)
+                first[b + 1] += first[b];
+            list.resize((size_t)first.back());
+        }
+    }
+    const auto locate = [&](int x, int y) {
+        const size_t b = (size_t)bucket_y(y) * bw + bucket_x(x);
+        for (int k = first[b]; k < first[b + 1]; k++) {
+            const int q = list[k];
+            if (x >= x0[q] && x - x0[q] < ex[q] && y >= y0[q] && y - y0[q] < ey[q])
+                return q;
+        }
+        return -1;
+    };
+    for (int c = 0; c < 4; c++)
+        for (int p = 0; p < P; p++) {
+            const long long x = c & 1 ? (long long)x0[p] + std::max(ex[p], 0) : x0[p] - 1LL;
+            const long long y = c & 2 ? (long long)y0[p] + std::max(ey[p], 0) : y0[p] - 1LL;
+            const bool out_x = x < 0 || x >= nx, out_y = y < 0 || y >= ny;
+            const int set = out_x || out_y;
+            int q = -1, xs = 0, ys = 0;
+            if ((!out_x || px) && (!out_y || py)) {
+                xs = (int)(((x % nx) + nx) % nx);
+                ys = (int)(((y % ny) + ny) % ny);
+                q = locate(xs, ys);
+            }
+            for (int s = 0; s < 2; s++) {
+                const size_t k = ((size_t)s * 4 + c) * P + p;
+                ids[k] = s == set ? q : -1;
+                starts[k] = s == set && q >= 0 ? (ys - y0[q]) * ex[q] + (xs - x0[q]) : 0;
+            }
+        }
+}
+
+// The corner items (HaloCorners) of the parts sharded over G ranks whose SOURCE part `rank` owns (G = 1: every item,
+// one buffer): the interior set first, n[0] items, then the periodic set, n[1] items in all.  ids / starts: from
+// halo_corner_sources; off: the ddc_halo_tile_offsets offsets.  src / dst / dst_rank: room for 4 P items each.
+inline void halo_corner_items(int P, int G, int rank, const int* ids, const int* starts, const int* ex, const int* ey,
+    const long long* off, long long* src, long long* dst, int* dst_rank, int* n)
+{
+    const auto owner = [&](int p) { return (int)(((long long)(p + 1) * G - 1) / P); };
+    const auto base = [&](int p) { return off[p] - off[(long long)owner(p) * P / G]; };
+    int k = 0;
+    for (int s = 0; s < 2; s++) {
+        for (int c = 0; c < 4; c++)
+            for (int p = 0; p < P; p++) {
+                const int q = ids[((size_t)s * 4 + c) * P + p];
+                if (q < 0 || owner(q) != rank)
+                    continue;
+                const int st = starts[((size_t)s * 4 + c) * P + p];
+                const long long pw = std::max(ex[p], 0) + 2, ph = std::max(ey[p], 0) + 2;
+                src[k] = base(q) + (long long)(st / ex[q] + 1) * (ex[q] + 2) + st % ex[q] + 1;
+                dst[k] = base(p) + (c & 2 ? ph - 1 : 0) * pw + (c & 1 ? pw - 1 : 0);
+                dst_rank[k] = owner(p);
+                k++;
+            }
+        n[s] = k;
+    }
+}
+
+// the corner ghosts of one buffer (ddc_halo_exchange_full_f64, after k_halo_exchange): one thread per item
+__global__ void __launch_bounds__(256) k_halo_corners(HaloCorners corners, double* tiles)
+{
+    unsigned long long* t = reinterpret_cast<unsigned long long*>(tiles);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < corners.n; i += gridDim.x * blockDim.x)
+        t[corners.dst[i]] = t[corners.src[i]];
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -53,6 +53,8 @@ typedef enum {
 } ddc_status;
 
 enum { DDC_LEFT = 0, DDC_RIGHT = 1, DDC_BOTTOM = 2, DDC_TOP = 3, DDC_N_EDGE = 4 };
+/* corners of a part's ghost frame (ddc_get_corner_neighbours, ddc_halo_exchange_full_f64) */
+enum { DDC_BOTTOM_LEFT = 0, DDC_BOTTOM_RIGHT = 1, DDC_TOP_LEFT = 2, DDC_TOP_RIGHT = 3, DDC_N_CORNER = 4 };
 
 /* flags of ddc_partition() */
 enum {
@@ -184,7 +186,8 @@ DDC_API int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny
    parts live in ONE device buffer: tile p is a row-major (ext_y[p] + 2) x (ext_x[p] + 2) array with a ghost frame of
    one cell around the part's box, starting at element offsets[p] (ddc_halo_tile_offsets: offsets[nparts] = total
    elements).  ddc_halo_exchange_f64 fills every ghost cell that faces a neighbour with that neighbour's adjacent
-   interior cell (interior lists; periodic != 0: the periodic lists too).  Corners are not exchanged. */
+   interior cell (interior lists; periodic != 0: the periodic lists too).  It leaves the four corner cells of every
+   frame as they are; ddc_halo_exchange_full_f64 below fills them too. */
 DDC_API int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets /* nparts + 1 */);
 DDC_API int ddc_halo_exchange_f64(ddc_handle_t h, double* tiles_dev, int periodic);
 
@@ -242,6 +245,36 @@ DDC_API int ddc_halo_scatter_f64(ddc_handle_t h, const double* field_dev, double
 DDC_API int ddc_halo_gather_f64(ddc_handle_t h, const double* tiles_dev, double* field_dev);
 DDC_API int ddc_halo_scatter_shards_f64(ddc_handle_t h, const double* rows_dev);
 DDC_API int ddc_halo_gather_shards_f64(ddc_handle_t h, double* rows_dev);
+
+/* Corner ghosts: the whole frame, for stencils that read the diagonal neighbour (9-point stencils, bilinear
+   interpolation at cell corners, B/C-grid averaging).  Corner c of part p with box {x0, y0, ex, ey} is the cell
+       DDC_BOTTOM_LEFT  (x0 - 1,  y0 - 1)   tile row 0,      column 0
+       DDC_BOTTOM_RIGHT (x0 + ex, y0 - 1)   tile row 0,      column ex + 1
+       DDC_TOP_LEFT     (x0 - 1,  y0 + ey)  tile row ey + 1, column 0
+       DDC_TOP_RIGHT    (x0 + ex, y0 + ey)  tile row ey + 1, column ex + 1
+   Its SOURCE is the box that contains that cell; when several do (caller-supplied boxes may overlap), the lowest-id box
+   of positive area.  The owner of a corner is often a box that touches p at that corner only, which is no neighbour in
+   the edge lists.  A corner is INTERIOR when its cell lies in [0, nx) x [0, ny); it is PERIODIC when the cell lies
+   outside in x and / or y, the decomposition is periodic in every direction in which it lies outside, and the wrapped
+   cell has a source.  Every other corner has no source.  The source may be p itself (a periodic corner of a part that
+   spans the domain), and zero-area parts have corners by the same rule.
+   ddc_get_corner_neighbours: for every part p, ids[p] = the source of corner `corner` in the interior (periodic = 0) or
+   periodic (periodic = 1) set, -1 when it has none there, and starts[p] = the cell's index in the source's flattened
+   box, (y - y0[q]) * ex[q] + (x - x0[q]) with x and y wrapped for a periodic corner (the halo_starts convention of
+   ddc_get_neighbours).  int32[nparts] host arrays, either may be NULL.  Valid after ddc_partition or
+   ddc_neighbours_from_boxes.
+   ddc_halo_exchange_full_f64 fills exactly what ddc_halo_exchange_f64 fills, bit for bit, plus every corner ghost
+   that has a source (interior set; periodic != 0: the periodic set too), copied as 64-bit words.  Preconditions and
+   status codes are those of ddc_halo_exchange_f64, and like it the call does nothing without neighbour tables (one
+   part, or no DDC_WANT_NEIGHBOURS).  ddc_halo_exchange_full_shards_f64 is the same on the sharded buffers, with the
+   checks and status codes of ddc_halo_exchange_shards_f64: it takes the next halo step number and mixes with sharded
+   exchanges, scatters and gathers in any order that is the same on every rank.  A corner ghost is stored by the rank
+   that owns its source part.  (A zero-area part has no interior: an edge list entry whose source is such a part is
+   filled from that part's frame, by both exchanges alike, and what it holds then is not defined.) */
+DDC_API int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, int32_t* ids /* nparts */,
+    int32_t* starts /* nparts */);
+DDC_API int ddc_halo_exchange_full_f64(ddc_handle_t h, double* tiles_dev, int periodic);
+DDC_API int ddc_halo_exchange_full_shards_f64(ddc_handle_t h, int periodic);
 
 /* ---- synthetic masks (SURVEY 8d): deterministic value-noise land-sea mask, generated directly
    into device memory so that no 4 GiB file is needed for the large configurations.

@@ -6,8 +6,10 @@
     torchrun --nproc-per-node G scripts/halo_bench.py --out r.json    # G GPUs, one process each
 
 One GPU: ddc_halo_exchange_f64 on one buffer against ddc_halo_exchange_shards_f64 with one rank (the same ghost
-cells, plus the open / close barriers of the sharded protocol), and ddc_halo_scatter_f64 / ddc_halo_gather_f64 against
-their sharded forms with one rank, all alternated in rounds.  G GPUs: the sharded calls over CUDA IPC, time per call =
+cells, plus the open / close barriers of the sharded protocol), the full-frame exchanges (ddc_halo_exchange_full_f64 /
+_full_shards_f64: the same plus the corner ghosts), and ddc_halo_scatter_f64 / ddc_halo_gather_f64 against their
+sharded forms with one rank, all alternated in rounds.  The host time of ddc_halo_tile_offsets (which also builds the
+corner items) and of one ddc_get_corner_neighbours (the corner table alone) is reported per configuration.  G GPUs: the sharded calls over CUDA IPC, time per call =
 the slowest rank's.  Times are CUDA events around `--iters` back-to-back calls after `--warmup` (enqueue included: it
 is what a caller pays).  Exchanges are periodic (the periodic lists are used where the decomposition has them).  Ghost
 cells moved come from the neighbour tables: a cell is read once (8 B) and written once (8 B); "cross-rank" cells are
@@ -61,6 +63,29 @@ def ghost_counts(h, P, G, periodic):
     return total, cross
 
 
+def corner_counts(h, P, G, periodic):
+    """corner ghosts one full-frame exchange writes: (all, written into another rank's buffer)"""
+    owner = lambda p: ((p + 1) * G - 1) // P
+    total = cross = 0
+    for per in range(2 if periodic else 1):
+        for c in range(4):
+            ids, _ = h.corner_neighbours(c, per)
+            has = ids >= 0
+            total += int(has.sum())
+            cross += int((owner(ids[has].astype(np.int64)) != owner(np.nonzero(has)[0])).sum())
+    return total, cross
+
+
+def host_ms(fn, reps=5):
+    """median host time of fn() in ms"""
+    t = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        fn()
+        t.append((time.perf_counter() - t0) * 1e3)
+    return round(float(np.median(t)), 4)
+
+
 def field_counts(boxes, ny, P, G):
     """cells a scatter / gather moves: (all, those whose row block and part belong to different ranks)"""
     b = np.asarray(boxes, dtype=np.int64)
@@ -104,10 +129,13 @@ def decompose(h, dev, cfg, world, rank):
     return d_mask
 
 
-def row(name, cfg, G, ms, cells, cross):
+def row(name, cfg, G, ms, cells, cross, corners=(0, 0)):
+    """an exchange; corners: (corner ghosts, of them cross-rank) -- (0, 0) for the edge exchange"""
+    cells, cross = cells + corners[0], cross + corners[1]
     bytes_moved = 16 * cells  # 8 B read + 8 B written per ghost cell
     return dict(config=name, nx=cfg["nx"], ny=cfg["ny"], parts=cfg["parts"], ranks=G, ms_per_exchange=round(ms, 5),
                 ghost_cells=cells, ghost_cells_local=cells - cross, ghost_cells_cross_rank=cross,
+                corner_cells=corners[0], corner_cells_cross_rank=corners[1],
                 bytes_read=8 * cells, bytes_written=8 * cells,
                 achieved_GBps=round(bytes_moved / (ms * 1e-3) / 1e9, 1))
 
@@ -124,15 +152,21 @@ def one_gpu(args):
         del d_mask
         P = cfg["parts"]
         off = h.halo_tile_offsets()
+        host = dict(config=name, parts=P, tile_offsets_host_ms=host_ms(h.halo_tile_offsets),
+                    corner_table_host_ms=host_ms(lambda: h.corner_neighbours(0, 1)))
+        print(json.dumps(host), flush=True)
         single = torch.zeros(int(off[-1]), dtype=torch.float64, device=dev)
         (ptr,) = capi.halo_connect([h], int(off[-1]))
         h.halo_shard_offsets()
         cells, cross = ghost_counts(h, P, 1, True)
+        corners = corner_counts(h, P, 1, True)
         fcells, fcross = field_counts(h.boxes(), cfg["ny"], P, 1)
         field = torch.zeros((cfg["ny"], cfg["nx"]), dtype=torch.float64, device=dev)
         back = torch.zeros_like(field)
         variants = {"single_buffer": lambda: h.halo_exchange_f64(single.data_ptr(), True),
                     "sharded_G1": lambda: h.halo_exchange_shards_f64(True),
+                    "full_single_buffer": lambda: h.halo_exchange_full_f64(single.data_ptr(), True),
+                    "full_sharded_G1": lambda: h.halo_exchange_full_shards_f64(True),
                     "scatter_single_buffer": lambda: h.halo_scatter_f64(field.data_ptr(), single.data_ptr()),
                     "gather_single_buffer": lambda: h.halo_gather_f64(single.data_ptr(), back.data_ptr()),
                     "scatter_sharded_G1": lambda: h.halo_scatter_shards_f64(field.data_ptr()),
@@ -147,10 +181,12 @@ def one_gpu(args):
         for k in variants:
             ms = float(np.median(samples[k]))
             r = row(name, cfg, 1, ms, cells, cross) if k in ("single_buffer", "sharded_G1") else \
+                row(name, cfg, 1, ms, cells, cross, corners) if k.startswith("full") else \
                 field_row(name, cfg, 1, k, ms, fcells, fcross)
             r.update(variant=k, samples_ms=[round(s, 5) for s in samples[k]], iters=args.iters)
             results.append(r)
             print(json.dumps(r), flush=True)
+        results.append(host)
         h.halo_close()
         h.close()
         del single, field, back
@@ -185,10 +221,12 @@ def multi_gpu(args):
         h.halo_import(handles)
         h.halo_shard_offsets()
         cells, cross = ghost_counts(h, P, world, True)
+        corners = corner_counts(h, P, world, True)
         fcells, fcross = field_counts(h.boxes(), cfg["ny"], P, world)
         yb, yc = capi.shard_rows(cfg["ny"], world, rank)
         rows = torch.zeros((max(yc, 1), cfg["nx"]), dtype=torch.float64, device=dev)
         variants = {"sharded": lambda: h.halo_exchange_shards_f64(True),
+                    "full_sharded": lambda: h.halo_exchange_full_shards_f64(True),
                     "scatter_sharded": lambda: h.halo_scatter_shards_f64(rows.data_ptr()),
                     "gather_sharded": lambda: h.halo_gather_shards_f64(rows.data_ptr())}
         for fn in variants.values():
@@ -202,7 +240,9 @@ def multi_gpu(args):
             t = torch.tensor(samples[k], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)  # per round: the slowest rank
             ms = float(np.median(t.cpu().numpy()))
-            r = row(name, cfg, world, ms, cells, cross) if k == "sharded" else field_row(name, cfg, world, k, ms, fcells, fcross)
+            r = row(name, cfg, world, ms, cells, cross) if k == "sharded" else \
+                row(name, cfg, world, ms, cells, cross, corners) if k == "full_sharded" else \
+                field_row(name, cfg, world, k, ms, fcells, fcross)
             r.update(variant=k, samples_ms=[round(float(s), 5) for s in t.cpu()], iters=args.iters)
             results.append(r)
             if rank == 0:

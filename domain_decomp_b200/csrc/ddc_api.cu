@@ -185,18 +185,11 @@ struct ddc_handle_s {
     DevBuf<uint8_t> bits;
     DevBuf<unsigned> colcount, colsum, colpfx, rowcount, rowcount_all, ypfx, done;
     DevBuf<DevScalars> sc;
-    DevBuf<long long> halo_off; // tile offsets of the halo exchange (ddc_halo_tile_offsets)
-    int halo_parts = 0;
-    // the (part, row) ranges of halo scatter / gather (HaloItems): [0] every field row, [1] this rank's ddc_shard_rows
-    DevBuf<int> halo_items; // [2][4 P + 1]
-    DevBuf<long long> halo_item_base; // [2][P]
-    int halo_items_n[2] = { 0, 0 }, halo_items_total[2] = { 0, 0 };
-    // the corner items of the full-frame exchange (HaloCorners), built with them: [0] one buffer, [1] the items whose
-    // source part this rank owns; each [src 4 P][dst 4 P] (+ [4 P] destination ranks), the interior set first
-    DevBuf<long long> halo_corner_ix; // [2][8 P]
-    DevBuf<int> halo_corner_rank; // [2][4 P]
-    int halo_corner_n[2][2] = {}; // [view][0: interior set, 1: both sets]
-    bool halo_corner_ok = false; // built for the current boxes and periodic flags
+    // the halo plan (ddc_halo_tile_offsets) and its tables on the device
+    HaloPlan halo;
+    DevBuf<unsigned char> halo_dev;
+    bool halo_ok = false; // the plan is of the current decomposition
+    bool halo_shard_ok = false; // ... and ddc_halo_shard_offsets was called for it
     DevBuf<unsigned> gate; // the word the gate kernel of the second stream waits for (see BoxGate)
     int use_gate = 1; // DDC_GATE: 0 never, 1 unless the shard is tiny, 2 always
     bool side_pdl = true; // DDC_SIDE_PDL: the scan of the neighbour counts launched programmatically behind the count kernel
@@ -253,8 +246,6 @@ struct ddc_handle_s {
     char* halo_peer[MAX_PEERS] = {}; // every rank's buffer as mapped here (halo_peer[rank] == halo_buf)
     int64_t halo_elems = 0; // capacity for tiles, in doubles
     bool halo_mapped = false, halo_local = false; // halo_local: the peers are handles of this process (ddc_halo_connect)
-    bool halo_shard_ok = false; // ddc_halo_shard_offsets ran for the current decomposition
-    long long halo_shard_max = 0; // the largest rank's tile total of that decomposition
     unsigned halo_step = 0; // exchanges enqueued since the buffers were joined
     int* halo_err = nullptr; // pinned, device-mapped: set by a halo kernel whose wait timed out
     int* halo_err_dev = nullptr;
@@ -274,6 +265,13 @@ struct ddc_handle_s {
 };
 
 namespace {
+// a new decomposition (ddc_partition, ddc_neighbours_from_boxes): the halo plan and the shard offsets are stale
+void halo_invalidate(ddc_handle_t h)
+{
+    h->halo_ok = false;
+    h->halo_shard_ok = false;
+}
+
 int fail(ddc_handle_t h, int code, const char* fmt, ...)
 {
     char buf[512];
@@ -709,11 +707,7 @@ int ddc_destroy(ddc_handle_t h)
     h->done.release();
     h->sc.release();
     h->gate.release();
-    h->halo_off.release();
-    h->halo_corner_ix.release();
-    h->halo_corner_rank.release();
-    h->halo_items.release();
-    h->halo_item_base.release();
+    h->halo_dev.release();
     h->plan.release();
     h->strips.release();
     h->boxes.release();
@@ -1028,9 +1022,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     h->have_nbr = false;
     h->totals_valid = false;
     h->small_cached = h->lists_cached = false;
-    h->halo_parts = 0;
-    h->halo_shard_ok = false;
-    h->halo_corner_ok = false;
+    halo_invalidate(h);
     memset(&h->stats, 0, sizeof h->stats);
     int launches = 0;
     // stage i begins: a CUDA event when profiling, and an NVTX range (the host-side enqueue of the stage; Nsight
@@ -1762,8 +1754,7 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
     h->px = px;
     h->py = py;
     h->mask_set = false; // the mask (if any) has to be set again before the next ddc_partition
-    h->halo_shard_ok = false;
-    h->halo_corner_ok = false;
+    halo_invalidate(h);
     h->d_mask = nullptr;
     h->pending = false;
     int rc = run_neighbours(h, P, nx, ny, px, py);
@@ -1782,81 +1773,37 @@ int ddc_neighbours_from_boxes(ddc_handle_t h, int nparts, int nx, int ny, const 
 // ------------------------------------------------------------------------------------------------
 // halo exchange (a consumer of the neighbour tables)
 // ------------------------------------------------------------------------------------------------
-// the corner source table of the current boxes (halo_corner_sources): ids / starts [2][4][P]
-static int corner_sources(ddc_handle_t h, std::vector<int32_t> box[4], std::vector<int>& ids, std::vector<int>& starts)
+// the halo plan of the current boxes (host only)
+static int build_halo_plan(ddc_handle_t h, HaloPlan& hp)
 {
     const int P = h->nparts;
+    std::vector<int32_t> box[4];
     for (int i = 0; i < 4; i++)
         box[i].resize(P);
     if (int rc = ddc_get_boxes(h, box[0].data(), box[1].data(), box[2].data(), box[3].data()))
         return rc;
-    ids.resize((size_t)8 * P);
-    starts.resize((size_t)8 * P);
-    halo_corner_sources(P, h->nx, h->ny, h->px, h->py, box[0].data(), box[1].data(), box[2].data(), box[3].data(),
-        ids.data(), starts.data());
-    return DDC_OK;
-}
-
-// the tile offsets of all parts in one buffer (offsets[P] = total), also left on the device for the exchange kernels,
-// and beside them the (part, row) ranges of scatter and gather (every field row, and this rank's ddc_shard_rows) and
-// the corner items of the full-frame exchange.  Everything is built here, where the host may wait for the stream: a
-// sharded call must not wait (one host thread may drive several ranks, whose open kernels wait for each other).
-static int tile_offsets(ddc_handle_t h, std::vector<long long>& off)
-{
-    const int P = h->nparts;
-    std::vector<int32_t> box[4];
-    std::vector<int> cids, cstarts;
-    if (int rc = corner_sources(h, box, cids, cstarts))
-        return rc;
-    const std::vector<int32_t>& y0 = box[1];
-    const std::vector<int32_t>& ex = box[2];
-    const std::vector<int32_t>& ey = box[3];
-    off.assign((size_t)P + 1, 0);
-    long long run = 0;
-    for (int p = 0; p < P; p++) {
-        off[p] = run;
-        run += (long long)(std::max(ex[p], 0) + 2) * (std::max(ey[p], 0) + 2);
-    }
-    off[P] = run;
-    const size_t per = (size_t)4 * P + 1;
-    std::vector<int> items(2 * per);
-    std::vector<long long> base((size_t)2 * P);
     int yb, yc;
     ddc_shard_rows(h->ny, h->nranks, h->rank, &yb, &yc);
-    for (int s = 0; s < 2; s++) {
-        int* t = items.data() + s * per;
-        h->halo_items_n[s] = halo_item_ranges(P, s ? h->nranks : 1, y0.data(), ex.data(), ey.data(), off.data(), s ? yb : 0,
-            s ? yb + yc : h->ny, t, base.data() + (size_t)s * P);
-        h->halo_items_total[s] = t[3 * P + h->halo_items_n[s]];
-    }
-    CUDA_TRY(h, h->halo_off.ensure((size_t)P + 1));
-    CUDA_TRY(h, h->halo_items.ensure(2 * per));
-    CUDA_TRY(h, h->halo_item_base.ensure((size_t)2 * P));
-    CUDA_TRY(h, cudaMemcpyAsync(h->halo_off.p, off.data(), sizeof(long long) * ((size_t)P + 1), cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(h->halo_items.p, items.data(), sizeof(int) * 2 * per, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(h->halo_item_base.p, base.data(), sizeof(long long) * 2 * P, cudaMemcpyHostToDevice, h->stream));
-    const size_t cp = (size_t)4 * P;
-    std::vector<long long> cix(4 * cp);
-    std::vector<int> crank(2 * cp);
-    for (int s = 0; s < 2; s++)
-        halo_corner_items(P, s ? h->nranks : 1, s ? h->rank : 0, cids.data(), cstarts.data(), ex.data(), ey.data(), off.data(),
-            cix.data() + 2 * s * cp, cix.data() + (2 * s + 1) * cp, crank.data() + s * cp, h->halo_corner_n[s]);
-    CUDA_TRY(h, h->halo_corner_ix.ensure(4 * cp));
-    CUDA_TRY(h, h->halo_corner_rank.ensure(2 * cp));
-    CUDA_TRY(h, cudaMemcpyAsync(h->halo_corner_ix.p, cix.data(), sizeof(long long) * 4 * cp, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(h->halo_corner_rank.p, crank.data(), sizeof(int) * 2 * cp, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    h->halo_parts = P;
-    h->halo_corner_ok = true;
+    hp = halo_plan(P, h->nranks, h->rank, h->nx, h->ny, h->px, h->py, box[0].data(), box[1].data(), box[2].data(),
+        box[3].data(), yb, yc);
     return DDC_OK;
 }
 
-// the corner items of view s (0 one buffer, 1 this rank's sources); periodic: both sets, else the interior set
-static HaloCorners halo_corners_of(ddc_handle_t h, int s, int periodic)
+// the halo plan of the current decomposition, also left on the device for the halo kernels: the tile offsets of all
+// parts in one buffer, the (part, row) ranges of scatter and gather and the corner items of the full-frame exchange.
+// Everything is built here, where the host may wait for the stream: a sharded call must not wait (one host thread may
+// drive several ranks, whose open kernels wait for each other).
+static int tile_offsets(ddc_handle_t h)
 {
-    const size_t cp = (size_t)4 * h->nparts;
-    return HaloCorners { h->halo_corner_ix.p + 2 * s * cp, h->halo_corner_ix.p + (2 * s + 1) * cp,
-        s ? h->halo_corner_rank.p + cp : nullptr, h->halo_corner_n[s][periodic ? 1 : 0] };
+    HaloPlan hp;
+    if (int rc = build_halo_plan(h, hp))
+        return rc;
+    CUDA_TRY(h, h->halo_dev.ensure(hp.block.size()));
+    CUDA_TRY(h, cudaMemcpyAsync(h->halo_dev.p, hp.block.data(), hp.block.size(), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->halo = std::move(hp);
+    h->halo_ok = true;
+    return DDC_OK;
 }
 
 int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
@@ -1864,11 +1811,10 @@ int ddc_halo_tile_offsets(ddc_handle_t h, int64_t* offsets)
     NEED_PARTITION(h);
     if (!offsets)
         return fail(h, DDC_ERR_ARG, "ddc_halo_tile_offsets: null output");
-    std::vector<long long> off;
-    if (int rc = tile_offsets(h, off))
+    if (int rc = tile_offsets(h))
         return rc;
-    for (size_t p = 0; p < off.size(); p++)
-        offsets[p] = off[p];
+    for (int p = 0; p <= h->nparts; p++)
+        offsets[p] = h->halo.off()[p];
     return DDC_OK;
 }
 
@@ -1878,25 +1824,25 @@ int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, int32_t*
     NEED_PARTITION(h);
     if (corner < 0 || corner >= DDC_N_CORNER || periodic < 0 || periodic > 1)
         return fail(h, DDC_ERR_ARG, "ddc_get_corner_neighbours: corner must be 0..3 and periodic 0/1");
-    std::vector<int32_t> box[4];
-    std::vector<int> cids, cstarts;
-    if (int rc = corner_sources(h, box, cids, cstarts))
-        return rc;
+    HaloPlan built;
+    if (!h->halo_ok)
+        if (int rc = build_halo_plan(h, built))
+            return rc;
+    const HaloPlan& hp = h->halo_ok ? h->halo : built;
     const size_t P = h->nparts, at = ((size_t)periodic * 4 + corner) * P;
     if (ids)
-        memcpy(ids, cids.data() + at, P * sizeof(int32_t));
+        memcpy(ids, hp.corner_ids.data() + at, P * sizeof(int32_t));
     if (starts)
-        memcpy(starts, cstarts.data() + at, P * sizeof(int32_t));
+        memcpy(starts, hp.corner_starts.data() + at, P * sizeof(int32_t));
     return DDC_OK;
 }
 
-constexpr int HALO_CORNER_BLOCKS = 4 * 148; // k_halo_corners' grid at most (grid-stride): 4 P items, 64 K at C5
 // one buffer: the edge ghosts (k_halo_exchange), and with `full` the corner ghosts after them (k_halo_corners)
 static int halo_exchange(ddc_handle_t h, double* tiles_dev, int periodic, bool full, const char* name)
 {
     if (!tiles_dev)
         return fail(h, DDC_ERR_ARG, "%s: null tiles", name);
-    if (h->halo_parts != h->nparts || (full && !h->halo_corner_ok))
+    if (!h->halo_ok)
         return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_tile_offsets() for this decomposition first", name);
     if (!h->have_nbr)
         return DDC_OK; // one part (or no tables asked for): nothing to exchange
@@ -1905,14 +1851,13 @@ static int halo_exchange(ddc_handle_t h, double* tiles_dev, int periodic, bool f
         return rc;
     const int P = h->nparts;
     Tables t = tables(h, P);
-    const long long warps = 8LL * P;
-    CUDA_TRY(h, launch_k(k_halo_exchange<double>, dim3((unsigned)((warps * 32 + 255) / 256)), dim3(256), 0, h->stream, false, t.bx, P,
-        h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, tiles_dev,
-        periodic ? 0xffu : 0x0fu));
-    const HaloCorners corners = halo_corners_of(h, 0, periodic);
+    CUDA_TRY(h, launch_k(k_halo_exchange<double>, dim3(halo_exchange_grid(P)), dim3(256), 0, h->stream, false, t.bx, P,
+        h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p,
+        h->halo.ptrs(h->halo_dev.p).off, tiles_dev, periodic ? 0xffu : 0x0fu));
+    const HaloCorners corners = h->halo.corners(h->halo_dev.p, 0, periodic);
     if (full && corners.n > 0) // (corners read interiors only: no order with the edges is needed)
-        CUDA_TRY(h, launch_k(k_halo_corners, dim3((unsigned)std::min((corners.n + 255) / 256, HALO_CORNER_BLOCKS)), dim3(256), 0,
-            h->stream, false, corners, tiles_dev));
+        CUDA_TRY(h, launch_k(k_halo_corners, dim3(halo_corner_grid(corners.n)), dim3(256), 0, h->stream, false, corners,
+            tiles_dev));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;
 }
@@ -1930,27 +1875,15 @@ int ddc_halo_exchange_full_f64(ddc_handle_t h, double* tiles_dev, int periodic)
 }
 
 // halo scatter / gather: the field rows <-> the tile interiors (k_halo_field, k_halo_field_shards)
-constexpr int HALO_FIELD_BLOCKS = 8 * 148; // at most: 8 blocks of 256 threads on each of B200's 148 SMs, grid-stride
-static HaloItems halo_items_of(ddc_handle_t h, int s) // s: 0 every field row, 1 this rank's shard rows
-{
-    const size_t P = h->nparts, per = 4 * P + 1;
-    const int* t = h->halo_items.p + s * per;
-    return HaloItems { t, t + P, t + 2 * P, t + 3 * P, h->halo_item_base.p + s * P, h->halo_items_n[s] };
-}
-static unsigned halo_field_grid(ddc_handle_t h, int s) // one warp per item, 8 per block
-{
-    return (unsigned)std::max(1, std::min((h->halo_items_total[s] + 7) / 8, HALO_FIELD_BLOCKS));
-}
-
 static int halo_field(ddc_handle_t h, bool scatter, double* field_dev, double* tiles_dev, const char* name)
 {
     if (!field_dev || !tiles_dev)
         return fail(h, DDC_ERR_ARG, "%s: null pointer", name);
-    if (h->halo_parts != h->nparts)
+    if (!h->halo_ok)
         return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_tile_offsets() for this decomposition first", name);
     Tables t = tables(h, h->nparts);
-    CUDA_TRY(h, launch_k(scatter ? k_halo_field<true> : k_halo_field<false>, dim3(halo_field_grid(h, 0)), dim3(256), 0, h->stream,
-        false, halo_items_of(h, 0), t.bx, tiles_dev, field_dev, h->nx));
+    CUDA_TRY(h, launch_k(scatter ? k_halo_field<true> : k_halo_field<false>, dim3(halo_field_grid(h->halo.items_total[0])),
+        dim3(256), 0, h->stream, false, h->halo.items(h->halo_dev.p, 0), t.bx, tiles_dev, field_dev, h->nx));
     CUDA_TRY(h, cudaGetLastError());
     return DDC_OK;
 }
@@ -1975,27 +1908,17 @@ int ddc_halo_shard_offsets(ddc_handle_t h, int64_t* offsets)
     NEED_PARTITION(h);
     if (!offsets)
         return fail(h, DDC_ERR_ARG, "ddc_halo_shard_offsets: null output");
-    std::vector<long long> off;
-    if (int rc = tile_offsets(h, off))
+    if (int rc = tile_offsets(h))
         return rc;
-    // every rank's total from the replicated boxes: the exchange refuses on every rank alike when one does not fit
-    const int P = h->nparts, G = h->nranks;
-    long long most = 0;
-    for (int r = 0; r < G; r++) {
-        int b, c;
-        ddc_shard_parts(P, G, r, &b, &c);
-        most = std::max(most, off[(size_t)b + c] - off[b]);
-    }
     int b, c;
-    ddc_shard_parts(P, G, h->rank, &b, &c);
+    ddc_shard_parts(h->nparts, h->nranks, h->rank, &b, &c);
+    const long long* off = h->halo.off();
     for (int i = 0; i <= c; i++)
         offsets[i] = off[(size_t)b + i] - off[b];
-    h->halo_shard_max = most;
     h->halo_shard_ok = true;
     return DDC_OK;
 }
 
-constexpr int HALO_PUSH_BLOCKS = 4 * 148; // k_halo_push's grid at most: a few waves of B200's 148 SMs
 // this rank's halo buffer: zeroed head (flags, block counter) + room for `elems` doubles; the error word beside it
 static int halo_alloc(ddc_handle_t h, int64_t elems)
 {
@@ -2082,74 +2005,61 @@ static int halo_shards_ready(ddc_handle_t h, const char* name)
 {
     if (!h->halo_buf || !h->halo_mapped)
         return fail(h, DDC_ERR_STATE, "%s: no halo buffers (ddc_halo_export + ddc_halo_import, or ddc_halo_connect)", name);
-    if (!h->halo_shard_ok || h->halo_parts != h->nparts)
+    if (!h->halo_shard_ok)
         return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_shard_offsets() for this decomposition first", name);
-    if (h->halo_shard_max > h->halo_elems)
-        return fail(h, DDC_ERR_ARG, "%s: a rank's tiles need %lld doubles, the buffers hold %lld", name, h->halo_shard_max,
+    if (h->halo.shard_max > h->halo_elems)
+        return fail(h, DDC_ERR_ARG, "%s: a rank's tiles need %lld doubles, the buffers hold %lld", name, h->halo.shard_max,
             (long long)h->halo_elems);
     return DDC_OK;
 }
 
-// the kernels' view of the buffers for the next sharded halo call: it takes the next step number
-static HaloShards halo_shards_next(ddc_handle_t h)
+// one sharded halo call with the next step number: k_halo_open, the middle kernel middle(hs) launches, k_halo_close
+extern "C++" { // (a template)
+template <typename Middle>
+static int halo_shards_call(ddc_handle_t h, Middle middle)
 {
-    HaloShards hs {};
-    hs.ps.rank = h->rank;
-    hs.ps.G = h->nranks;
-    hs.ps.enabled = 1;
-    hs.ps.step = ++h->halo_step;
-    for (int q = 0; q < h->nranks; q++) {
-        hs.ps.flags[q] = (unsigned*)h->halo_peer[q];
-        hs.tiles[q] = (double*)(h->halo_peer[q] + HALO_HEAD_BYTES);
-    }
-    hs.done = (unsigned*)h->halo_buf + 2 * MAX_PEERS;
-    hs.opened = hs.done + 1;
-    hs.err = h->halo_err_dev;
-    hs.P = h->nparts;
-    ddc_shard_parts(h->nparts, h->nranks, h->rank, &hs.p_begin, &hs.p_count);
-    return hs;
+    const HaloShards hs = halo_shards(h->nparts, h->nranks, h->rank, ++h->halo_step, h->halo_peer, h->halo_err_dev);
+    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
+    CUDA_TRY(h, middle(hs));
+    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
+    CUDA_TRY(h, cudaGetLastError());
+    return DDC_OK;
+}
+}
+
+// the edge ghosts (k_halo_push), and with `full` the corner ghosts beside them (k_halo_push_full)
+static int halo_exchange_shards(ddc_handle_t h, int periodic, bool full, const char* name)
+{
+    if (int rc = halo_shards_ready(h, name))
+        return rc;
+    if (!h->have_nbr)
+        return DDC_OK; // one part (or no tables asked for): nothing to exchange, no step taken
+    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
+        return rc;
+    Tables t = tables(h, h->nparts);
+    const long long* off = h->halo.ptrs(h->halo_dev.p).off;
+    const unsigned lists = periodic ? 0xffu : 0x0fu;
+    const HaloCorners corners = h->halo.corners(h->halo_dev.p, 1, periodic);
+    return halo_shards_call(h, [&](const HaloShards& hs) {
+        const dim3 grid(halo_push_grid(hs.p_count, full ? corners.n : 0));
+        if (full)
+            return launch_k(k_halo_push_full, grid, dim3(256), 0, h->stream, false, hs, t.bx, h->nbr_counts.p,
+                h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, off, lists, corners);
+        return launch_k(k_halo_push, grid, dim3(256), 0, h->stream, false, hs, t.bx, h->nbr_counts.p, h->nbr_offsets.p,
+            h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, off, lists);
+    });
 }
 
 int ddc_halo_exchange_shards_f64(ddc_handle_t h, int periodic)
 {
     NEED_PARTITION(h);
-    if (int rc = halo_shards_ready(h, "ddc_halo_exchange_shards_f64"))
-        return rc;
-    if (!h->have_nbr)
-        return DDC_OK; // one part (or no tables asked for): nothing to exchange
-    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
-        return rc;
-    Tables t = tables(h, h->nparts);
-    const HaloShards hs = halo_shards_next(h);
-    const unsigned lists = periodic ? 0xffu : 0x0fu;
-    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
-    CUDA_TRY(h, launch_k(k_halo_push, dim3((unsigned)std::max(1, std::min(hs.p_count, HALO_PUSH_BLOCKS))), dim3(256), 0, h->stream, false, hs, t.bx,
-        h->nbr_counts.p, h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, lists));
-    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
-    CUDA_TRY(h, cudaGetLastError());
-    return DDC_OK;
+    return halo_exchange_shards(h, periodic, false, "ddc_halo_exchange_shards_f64");
 }
 
 int ddc_halo_exchange_full_shards_f64(ddc_handle_t h, int periodic)
 {
     NEED_PARTITION(h);
-    if (int rc = halo_shards_ready(h, "ddc_halo_exchange_full_shards_f64")) // (halo_shard_ok: the corner items are current)
-        return rc;
-    if (!h->have_nbr)
-        return DDC_OK; // as ddc_halo_exchange_shards_f64: nothing to exchange, no step taken
-    if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
-        return rc;
-    Tables t = tables(h, h->nparts);
-    const HaloShards hs = halo_shards_next(h);
-    const HaloCorners corners = halo_corners_of(h, 1, periodic);
-    const int grid = std::max(1, std::min(std::max(hs.p_count, (corners.n + 255) / 256), HALO_PUSH_BLOCKS));
-    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
-    CUDA_TRY(h, launch_k(k_halo_push_full, dim3((unsigned)grid), dim3(256), 0, h->stream, false, hs, t.bx, h->nbr_counts.p,
-        h->nbr_offsets.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p, h->halo_off.p, periodic ? 0xffu : 0x0fu,
-        corners));
-    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
-    CUDA_TRY(h, cudaGetLastError());
-    return DDC_OK;
+    return halo_exchange_shards(h, periodic, true, "ddc_halo_exchange_full_shards_f64");
 }
 
 static int halo_field_shards(ddc_handle_t h, bool scatter, double* rows_dev, const char* name)
@@ -2161,13 +2071,11 @@ static int halo_field_shards(ddc_handle_t h, bool scatter, double* rows_dev, con
     if (!rows_dev && yc > 0) // (this rank only: its peers time out waiting for it and report DDC_ERR_PEER)
         return fail(h, DDC_ERR_ARG, "%s: null rows (this rank holds rows %d..%d)", name, yb, yb + yc - 1);
     Tables t = tables(h, h->nparts);
-    const HaloShards hs = halo_shards_next(h);
-    CUDA_TRY(h, launch_k(k_halo_open, dim3(1), dim3(32), 0, h->stream, false, hs, 3));
-    CUDA_TRY(h, launch_k(scatter ? k_halo_field_shards<true> : k_halo_field_shards<false>, dim3(halo_field_grid(h, 1)), dim3(256), 0,
-        h->stream, false, hs, halo_items_of(h, 1), t.bx, rows_dev, h->nx, yb));
-    CUDA_TRY(h, launch_k(k_halo_close, dim3(1), dim3(32), 0, h->stream, false, hs));
-    CUDA_TRY(h, cudaGetLastError());
-    return DDC_OK;
+    return halo_shards_call(h, [&](const HaloShards& hs) {
+        return launch_k(scatter ? k_halo_field_shards<true> : k_halo_field_shards<false>,
+            dim3(halo_field_grid(h->halo.items_total[1])), dim3(256), 0, h->stream, false, hs,
+            h->halo.items(h->halo_dev.p, 1), t.bx, rows_dev, h->nx, yb);
+    });
 }
 
 int ddc_halo_scatter_shards_f64(ddc_handle_t h, const double* rows_dev)

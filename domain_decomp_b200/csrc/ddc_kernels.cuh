@@ -2556,6 +2556,27 @@ struct HaloShards {
     int* err; // host-mapped error word (1: a rank did not reach the exchange in time)
     int P, p_begin, p_count; // all parts; this rank's range
 };
+// Host code, shared by ddc_api.cu and the emulation harness of the tests: the view of rank `rank` for halo step `step`.
+// bufs[q]: rank q's buffer as mapped here; err: the rank's error word as the device sees it.
+inline HaloShards halo_shards(int P, int G, int rank, unsigned step, char* const* bufs, int* err)
+{
+    HaloShards hs {};
+    hs.ps.rank = rank;
+    hs.ps.G = G;
+    hs.ps.enabled = 1;
+    hs.ps.step = step;
+    for (int q = 0; q < G; q++) {
+        hs.ps.flags[q] = reinterpret_cast<unsigned*>(bufs[q]);
+        hs.tiles[q] = reinterpret_cast<double*>(bufs[q] + HALO_HEAD_BYTES);
+    }
+    hs.done = reinterpret_cast<unsigned*>(bufs[rank]) + 2 * MAX_PEERS;
+    hs.opened = hs.done + 1;
+    hs.err = err;
+    hs.P = P;
+    hs.p_begin = (int)((long long)rank * P / G); // ddc_shard_parts
+    hs.p_count = (int)((long long)(rank + 1) * P / G) - hs.p_begin;
+    return hs;
+}
 __device__ __forceinline__ void halo_timed_out(const HaloShards& hs)
 {
 #ifndef DDC_HOST_EMU
@@ -2727,7 +2748,7 @@ struct HaloItems {
 };
 // the ranges of the field rows [lo, hi) with the parts sharded over G ranks (G = 1: one buffer) into
 // out[4 P + 1] = [part: P][j0: P][owner: P][first: P + 1] and base[P]; y0 / ex / ey: the boxes, off: the
-// ddc_halo_tile_offsets offsets.  Returns n.  Host code, shared by ddc_api.cu and the emulation harness of the tests.
+// ddc_halo_tile_offsets offsets.  Returns n.  Host code, part of halo_plan.
 inline int halo_item_ranges(int P, int G, const int* y0, const int* ex, const int* ey, const long long* off, int lo, int hi,
     int* out, long long* base)
 {
@@ -2839,7 +2860,7 @@ __global__ void __launch_bounds__(256) k_halo_field_shards(HaloShards hs, HaloIt
 // corner (the cell lies in [0, nx) x [0, ny)) the cell itself, for a periodic one the cell wrapped in the directions in
 // which it lies outside, all of which must be periodic.  A box that touches p only at a corner has no domain overlap
 // with p, so no edge list names it, and zero-area parts have no lists at all: the owner is found by point location.
-// Host code, shared by ddc_api.cu and the emulation harness of the tests.
+// Host code, part of halo_plan.
 //   ids / starts [2][4][P]: set (0 interior, 1 periodic), corner, part -> source part (-1: none) and the cell's index
 //   (y - y0[q]) * ex[q] + (x - x0[q]) in the source's flattened box (the halo_start convention).  For each (corner,
 //   part) at most one of the two sets has a source.
@@ -2939,6 +2960,93 @@ __global__ void __launch_bounds__(256) k_halo_corners(HaloCorners corners, doubl
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < corners.n; i += gridDim.x * blockDim.x)
         t[corners.dst[i]] = t[corners.src[i]];
 }
+
+// ------------------------------------------------------------------------------------------------
+// The halo plan: every table the host builds for the halo calls of one decomposition
+// ------------------------------------------------------------------------------------------------
+// Host code, shared by ddc_api.cu and the emulation harness of the tests; nothing else builds these tables.  View s of
+// the items and corners is 0: one buffer (every field row, every corner item), 1: this rank's shards (its
+// ddc_shard_rows block, the corner items whose source part it owns).  The tables the kernels read are one block of
+// memory, uploaded with one copy; off() / items() / corners() read them from a copy of the block at `at` (the device's,
+// or the block itself on the host).
+struct HaloPlan {
+    int P = 0;
+    std::vector<unsigned char> block;
+    std::vector<int> corner_ids, corner_starts; // [2][4][P] (halo_corner_sources): ddc_get_corner_neighbours
+    int items_n[2] = {}, items_total[2] = {};
+    int corner_n[2][2] = {}; // [view][0: interior set, 1: both sets]
+    long long shard_max = 0; // the largest rank's tile total: what every rank's halo buffer must hold
+
+    // the layout of the block: 64-bit [off: P + 1][item base: 2][P][corner src, dst: 2][2][4 P], then 32-bit
+    // [items: 2][4 P + 1][corner destination rank: 2][4 P]
+    struct Ptrs {
+        long long *off, *base[2], *corner[2];
+        int *items[2], *rank[2];
+    };
+    static size_t bytes(int P) { return sizeof(long long) * (19 * (size_t)P + 1) + sizeof(int) * (16 * (size_t)P + 2); }
+    Ptrs ptrs(void* at) const
+    {
+        const size_t Q = P;
+        long long* w = static_cast<long long*>(at);
+        int* i = reinterpret_cast<int*>(w + 19 * Q + 1);
+        return Ptrs { w, { w + Q + 1, w + 2 * Q + 1 }, { w + 3 * Q + 1, w + 11 * Q + 1 }, { i, i + 4 * Q + 1 },
+            { i + 8 * Q + 2, i + 12 * Q + 2 } };
+    }
+    const long long* off() const { return reinterpret_cast<const long long*>(block.data()); } // the host's [P + 1]
+    HaloItems items(void* at, int s) const
+    {
+        const Ptrs a = ptrs(at);
+        const int* t = a.items[s];
+        return HaloItems { t, t + P, t + 2 * P, t + 3 * P, a.base[s], items_n[s] };
+    }
+    HaloCorners corners(void* at, int s, int periodic) const // periodic: both sets, else the interior set
+    {
+        const Ptrs a = ptrs(at);
+        return HaloCorners { a.corner[s], a.corner[s] + 4 * (size_t)P, s ? a.rank[s] : nullptr, corner_n[s][periodic ? 1 : 0] };
+    }
+};
+
+// The plan of boxes x0 / y0 / ex / ey [P] on a domain nx x ny (periodic px / py), for rank `rank` of G, whose
+// ddc_shard_rows block is rows y_begin ... y_begin + y_count - 1.
+inline HaloPlan halo_plan(int P, int G, int rank, int nx, int ny, int px, int py, const int* x0, const int* y0,
+    const int* ex, const int* ey, int y_begin, int y_count)
+{
+    HaloPlan hp;
+    hp.P = P;
+    hp.block.assign(HaloPlan::bytes(P), 0);
+    const HaloPlan::Ptrs a = hp.ptrs(hp.block.data());
+    long long run = 0;
+    for (int p = 0; p < P; p++) {
+        a.off[p] = run;
+        run += (long long)(std::max(ex[p], 0) + 2) * (std::max(ey[p], 0) + 2);
+    }
+    a.off[P] = run;
+    for (int r = 0; r < G; r++) // every rank's total from the replicated boxes: the sharded calls refuse on every rank alike
+        hp.shard_max = std::max(hp.shard_max, a.off[(long long)(r + 1) * P / G] - a.off[(long long)r * P / G]);
+    hp.corner_ids.resize((size_t)8 * P);
+    hp.corner_starts.resize((size_t)8 * P);
+    halo_corner_sources(P, nx, ny, px, py, x0, y0, ex, ey, hp.corner_ids.data(), hp.corner_starts.data());
+    for (int s = 0; s < 2; s++) {
+        hp.items_n[s] = halo_item_ranges(P, s ? G : 1, y0, ex, ey, a.off, s ? y_begin : 0, s ? y_begin + y_count : ny,
+            a.items[s], a.base[s]);
+        hp.items_total[s] = a.items[s][3 * P + hp.items_n[s]];
+        halo_corner_items(P, s ? G : 1, s ? rank : 0, hp.corner_ids.data(), hp.corner_starts.data(), ex, ey, a.off,
+            a.corner[s], a.corner[s] + 4 * (size_t)P, a.rank[s], hp.corner_n[s]);
+    }
+    return hp;
+}
+
+// the grids of the halo kernels (B200: 148 SMs); all but k_halo_exchange's are grid-stride
+constexpr int HALO_PUSH_BLOCKS = 4 * 148; // k_halo_push's grid at most: a few waves of B200's 148 SMs
+constexpr int HALO_CORNER_BLOCKS = 4 * 148; // k_halo_corners' grid at most: 4 P items, 64 K at C5
+constexpr int HALO_FIELD_BLOCKS = 8 * 148; // at most: 8 blocks of 256 threads on each of B200's 148 SMs
+inline unsigned halo_exchange_grid(int P) { return (unsigned)((8LL * P * 32 + 255) / 256); } // a warp per (list, part)
+inline unsigned halo_push_grid(int p_count, int corners) // k_halo_push (corners = 0), k_halo_push_full
+{
+    return (unsigned)std::max(1, std::min(std::max(p_count, (corners + 255) / 256), HALO_PUSH_BLOCKS));
+}
+inline unsigned halo_corner_grid(int n) { return (unsigned)std::min((n + 255) / 256, HALO_CORNER_BLOCKS); }
+inline unsigned halo_field_grid(int items) { return (unsigned)std::max(1, std::min((items + 7) / 8, HALO_FIELD_BLOCKS)); } // a warp per item
 
 // ------------------------------------------------------------------------------------------------
 // synthetic land-sea mask: two octaves of integer value noise (bit-identical on host and device)

@@ -24,7 +24,7 @@ import halo_frame as hf  # noqa: E402
 import halo_global as hg  # noqa: E402
 from domain_decomp_b200 import capi  # noqa: E402
 from halo_shards_worker import CASES, _Dev, decompose  # noqa: E402
-from test_halo_fields_on_cpu_emulator import SENTINEL, exchanged, random_bits, scattered  # noqa: E402
+from halo_global import SENTINEL, exchanged, random_bits, scattered  # noqa: E402
 
 
 def main():

@@ -15,17 +15,10 @@ import pytest
 
 import halo_global as hg
 from conftest import ROOT
-from test_gpu_halo_shards import decompose, dev_view
-from test_halo_fields_on_cpu_emulator import SENTINEL, SPECIAL, exchanged, scattered
+from halo_global import (GPU_CASES as CASES, SENT, SENTINEL, connect, decompose, dev_view, exchanged, random_field,
+                         scattered, u64)
 
 pytestmark = pytest.mark.gpu
-
-CASES = [  # nx, ny, P, px, py
-    (528, 522, 64, True, True),
-    (2048, 1536, 1000, True, False),
-    (8192, 8192, 4096, False, False),
-]
-SENT = int(SENTINEL.view(np.int64))
 
 
 @pytest.fixture(scope="module")
@@ -35,19 +28,6 @@ def env():
         pytest.skip("no CUDA device")
     from domain_decomp_b200 import capi
     return capi, torch
-
-
-def random_field(torch, nx, ny, seed):
-    """int64 [ny, nx] of random bit patterns on the device, the special values planted; view it as float64 to pass it"""
-    g = torch.Generator(device="cuda").manual_seed(seed)
-    f = torch.randint(-2 ** 63, 2 ** 63 - 1, (ny, nx), dtype=torch.int64, device="cuda", generator=g)
-    pos = torch.randint(0, nx * ny, (len(SPECIAL),), device="cuda", generator=g)
-    f.view(-1)[pos] = torch.from_numpy(SPECIAL.view(np.int64)).cuda()
-    return f
-
-
-def u64(t):
-    return t.cpu().numpy().view(np.uint64)
 
 
 def frame_cells(boxes, off):
@@ -107,16 +87,6 @@ def test_c5_round_trip(env):
     h.close()
     del field, tiles, back, fr
     torch.cuda.empty_cache()
-
-
-def connect(capi, boxes, nx, ny, px, py, G):
-    handles = [capi.Handle(0, q, G, None) for q in range(G)]
-    for h in handles:
-        h.neighbours_from_boxes(boxes, nx, ny, px, py)
-    ptrs = capi.halo_connect(handles, hg.max_shard_total(boxes, G))
-    for h in handles:
-        h.halo_shard_offsets()
-    return handles, ptrs
 
 
 @pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])

@@ -17,9 +17,8 @@ import pytest
 import halo_frame as hf
 import halo_global as hg
 from conftest import ROOT
-from test_gpu_halo_fields import CASES, SENT, random_field, u64
-from test_gpu_halo_shards import decompose, dev_view
-from test_halo_fields_on_cpu_emulator import SENTINEL, exchanged, scattered
+from halo_global import (GPU_CASES as CASES, SENT, SENTINEL, connect, decompose, dev_view, exchanged, random_field,
+                         scattered, u64)
 
 pytestmark = pytest.mark.gpu
 
@@ -88,16 +87,6 @@ def test_c5_edges_and_corners(env):
     h.close()
     del edge, full, idx
     torch.cuda.empty_cache()
-
-
-def connect(capi, boxes, nx, ny, px, py, G):
-    handles = [capi.Handle(0, q, G, None) for q in range(G)]
-    for h in handles:
-        h.neighbours_from_boxes(boxes, nx, ny, px, py)
-    ptrs = capi.halo_connect(handles, hg.max_shard_total(boxes, G))
-    for h in handles:
-        h.halo_shard_offsets()
-    return handles, ptrs
 
 
 @pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])

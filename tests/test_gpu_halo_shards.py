@@ -13,14 +13,9 @@ import pytest
 
 import halo_global as hg
 from conftest import ROOT
+from halo_global import GPU_CASES as CASES, decompose, dev_view
 
 pytestmark = pytest.mark.gpu
-
-CASES = [  # nx, ny, P, px, py
-    (528, 522, 64, True, True),
-    (2048, 1536, 1000, True, False),
-    (8192, 8192, 4096, False, False),
-]
 
 
 @pytest.fixture(scope="module")
@@ -30,27 +25,6 @@ def env():
         pytest.skip("no CUDA device")
     from domain_decomp_b200 import capi
     return capi, torch
-
-
-class _Dev:
-    def __init__(self, ptr, n):
-        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (int(ptr), False), "version": 2,
-                                         "strides": None}
-
-
-def dev_view(torch, ptr, n):
-    """float64[n] over raw device memory (a halo buffer of the library)"""
-    return torch.as_tensor(_Dev(ptr, n), device="cuda") if n else torch.empty(0, dtype=torch.float64, device="cuda")
-
-
-def decompose(capi, torch, nx, ny, P, px, py, seed=3, land=0.45):
-    h = capi.Handle(0)
-    d_mask = torch.empty((ny, nx), dtype=torch.int32, device="cuda")
-    h.generate_mask_device(d_mask.data_ptr(), nx, ny, seed, land)
-    h.set_mask_device(d_mask.data_ptr(), nx, ny)
-    h.partition(P, px, py)
-    h._mask = d_mask
-    return h
 
 
 def check_exchanges(capi, torch, single_h, handles, ptrs, nx, ny, px, py, steps=2):

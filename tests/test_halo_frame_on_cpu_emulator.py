@@ -1,19 +1,14 @@
 """The full-frame halo exchange (corner ghosts: ddc_get_corner_neighbours, ddc_halo_exchange_full_f64 and
 ddc_halo_exchange_full_shards_f64) on a machine without a GPU.
 
-1. The kernels on emulated ranks: tests/emu_halo_frame.cpp, compiled here into a temporary directory, runs the
-   product's own corner table and item builders (halo_corner_sources, halo_corner_items) and kernels (k_halo_exchange +
-   k_halo_corners on one buffer, k_halo_push_full between k_halo_open and k_halo_close on G ranks, mixed with
-   k_halo_push, k_halo_field and k_halo_field_shards), under index-order and random schedules.
+1. The kernels on emulated ranks: tests/emu_halo.cpp (built by tests/halo_emu.py) runs the product's own halo plan
+   (halo_plan: the corner table and items) and kernels (k_halo_exchange + k_halo_corners on one buffer,
+   k_halo_push_full between k_halo_open and k_halo_close on G ranks, mixed with k_halo_push, k_halo_field and
+   k_halo_field_shards), under index-order and random schedules.
 2. The C ABI itself on oracle/libddc_cuda_emu.so (domain_decomp_b200/csrc/ddc_api.cu over a host stand-in of the CUDA
    runtime): the getter, the single-buffer call, the status codes, and the sharded call with one rank.
 The corner table is checked against halo_frame.corner_table, a brute-force owner map.  Says nothing about speed."""
-import atexit
 import ctypes as C
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -21,75 +16,10 @@ import pytest
 import halo_emu
 import halo_frame as hf
 import halo_global as hg
-from test_halo_fields_on_cpu_emulator import SENTINEL, cases, exchanged, random_bits, scattered, shard_rows
+from halo_global import SENTINEL, cases, exchanged, random_bits, scattered
 
 RANKS = (1, 2, 3, 5)
 SEEDS = ("0", "11", "4242")  # DDC_EMU_SCHED_SEED: "0" index order, otherwise random block / thread schedules
-
-_lib = None
-
-
-def lib() -> C.CDLL:
-    global _lib
-    if _lib is None:
-        out = tempfile.mkdtemp(prefix="ddc_emu_frame_")
-        atexit.register(shutil.rmtree, out, True)
-        so = os.path.join(out, "libddc_emu_frame.so")
-        root, emu = halo_emu.ROOT, os.path.join(halo_emu.ROOT, "oracle", "emu")
-        subprocess.check_call([halo_emu._compiler(), "-O2", "-std=c++17", "-fPIC", "-shared", "-fvisibility=hidden",
-                               "-ffp-contract=off", "-U_FORTIFY_SOURCE", "-DDDC_HOST_EMU",
-                               "-I" + os.path.join(root, "domain_decomp_b200", "csrc"), "-I" + os.path.join(root, "include"),
-                               "-I" + emu, "-o", so, os.path.join(root, "tests", "emu_halo_frame.cpp"),
-                               os.path.join(emu, "cuda_emu.cpp")])
-        L = C.CDLL(so)
-        i32p = np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")
-        f64p = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")
-        L.emu_halo_frame.argtypes = [C.c_int, i32p, i32p, i32p, i32p, i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                     i32p, i32p, C.c_int, C.c_char_p, C.c_int, f64p, f64p, f64p, f64p, f64p, f64p, f64p,
-                                     i32p, i32p, i32p]
-        L.emu_halo_frame.restype = C.c_int
-        L.emu_halo_frame_last_error.restype = C.c_char_p
-        _lib = L
-    return _lib
-
-
-class Run:
-    """what emu_frame returns: per op, the sharded tiles (concatenated in rank order), the single buffer, the gathered
-    rows and the single-buffer field, all as uint64; the error words; the corner table [2, 4, P]"""
-
-    def __init__(self, **kw):
-        self.__dict__.update(kw)
-
-
-def emu_frame(boxes, nbr, nx, ny, px, py, G, periodic, ops, tiles_in, field=None, rows_in=None, stall=-1):
-    L = lib()
-    boxes = np.ascontiguousarray(boxes, dtype=np.int32)
-    P = len(boxes)
-    lists = [(per, e) for per in range(2) for e in range(4)]
-    cat = lambda a: np.ascontiguousarray(np.concatenate([a[per][e] for per, e in lists] + [np.zeros(1, np.int32)]),
-                                         dtype=np.int32)
-    counts = np.ascontiguousarray(np.concatenate([nbr.counts[per][e] for per, e in lists]), dtype=np.int32)
-    rows = shard_rows(ny, G)
-    as_f64 = lambda a: np.ascontiguousarray(a).reshape(-1).view(np.float64)
-    tiles_in = np.ascontiguousarray(tiles_in, dtype=np.uint64)
-    field = np.zeros(nx * ny, np.uint64) if field is None else field
-    rows_in = np.zeros(nx * ny, np.uint64) if rows_in is None else rows_in
-    total, n = int(tiles_in.size), len(ops)
-    tiles, single = np.zeros(n * total), np.zeros(n * total)
-    out_rows, out_field = np.zeros(n * nx * ny), np.zeros(n * nx * ny)
-    err = np.zeros(G, dtype=np.int32)
-    ids, starts = np.zeros(8 * P, dtype=np.int32), np.zeros(8 * P, dtype=np.int32)
-    rc = L.emu_halo_frame(P, boxes.reshape(-1), counts, cat(nbr.ids), cat(nbr.halos), cat(nbr.starts), nx, ny, int(px),
-                          int(py), G, np.array([b for b, _ in rows], dtype=np.int32),
-                          np.array([c for _, c in rows], dtype=np.int32), int(periodic), ops.encode(), stall,
-                          as_f64(np.asarray(field, dtype=np.uint64)), as_f64(tiles_in),
-                          as_f64(np.asarray(rows_in, dtype=np.uint64)), tiles, single, out_rows, out_field, err, ids,
-                          starts)
-    if rc != 0:
-        raise RuntimeError("emu_halo_frame: " + L.emu_halo_frame_last_error().decode())
-    u = lambda a, m: a.view(np.uint64).reshape(n, m)
-    return Run(tiles=u(tiles, total), single=u(single, total), rows=u(out_rows, nx * ny), field=u(out_field, nx * ny),
-               err=err, ids=ids.reshape(2, 4, P), starts=starts.reshape(2, 4, P))
 
 
 def degenerate_cases(oracle, zero_width=True):
@@ -127,7 +57,7 @@ def test_corner_table_matches_brute_force(oracle):
     boxes_sets.append((one.boxes, one.nbr, 7, 5, True, True))
     for boxes, nbr, nx, ny, px, py in boxes_sets:
         off = hg.tile_offsets(np.maximum(boxes, 0))
-        run = emu_frame(boxes, nbr, nx, ny, px, py, 1, 0, "", np.zeros(int(off[-1]), np.uint64))
+        run = halo_emu.run(boxes, nbr, nx, ny, px, py, 1, 0, "", np.zeros(int(off[-1]), np.uint64))
         ids, starts = hf.corner_table(boxes, nx, ny, px, py)
         assert np.array_equal(run.ids, ids), (nx, ny, px, py, boxes.tolist())
         assert np.array_equal(run.starts, starts), (nx, ny, px, py, boxes.tolist())
@@ -148,8 +78,8 @@ def test_full_exchange_fills_the_whole_frame(oracle, monkeypatch, G, sched):
         tiles_in = as_bits(hg.initial_tiles(d.boxes, off, nx))
         for periodic in (0, 1):
             ctx = (G, sched, seed, nx, ny, d.P, periodic)
-            full = emu_frame(d.boxes, d.nbr, nx, ny, px, py, G, periodic, "f", tiles_in)
-            edge = emu_frame(d.boxes, d.nbr, nx, ny, px, py, G, periodic, "x", tiles_in)
+            full = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, "f", tiles_in)
+            edge = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, "x", tiles_in)
             assert full.err.tolist() == [0] * G, ctx
             want = as_bits(hf.expected_full_tiles(d.boxes, off, nx, ny, px, py, periodic))
             assert np.array_equal(full.single[0], want), ctx + ("single buffer",)
@@ -186,8 +116,8 @@ def test_degenerate_tilings(oracle, G):
         corners = hf.corner_cells(boxes, off).reshape(-1)
         for periodic in (0, 1):
             ctx = (G, seed, nx, ny, len(boxes), periodic)
-            full = emu_frame(boxes, nbr, nx, ny, px, py, G, periodic, "f", tiles_in)
-            edge = emu_frame(boxes, nbr, nx, ny, px, py, G, periodic, "x", tiles_in)
+            full = halo_emu.run(boxes, nbr, nx, ny, px, py, G, periodic, "f", tiles_in)
+            edge = halo_emu.run(boxes, nbr, nx, ny, px, py, G, periodic, "x", tiles_in)
             assert full.err.tolist() == [0] * G, ctx
             want = as_bits(hf.with_corners(boxes, off, nx, ny, px, py, periodic, field,
                                            edge.single[0].view(np.float64)))
@@ -213,7 +143,8 @@ def test_mixed_sequence_on_one_step_counter(oracle, monkeypatch, G, sched):
         field = random_bits(rng, nx * ny).reshape(ny, nx)
         tiles_in = np.full(int(off[-1]), SENTINEL, dtype=np.uint64)
         ops = "sfxfg"
-        run = emu_frame(d.boxes, d.nbr, nx, ny, px, py, G, periodic, ops, tiles_in, field, random_bits(rng, nx * ny))
+        run = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, ops, tiles_in, [field],
+                           random_bits(rng, nx * ny))
         ctx = (G, sched, seed, nx, ny, d.P, periodic)
         assert run.err.tolist() == [0] * G, ctx
         want = scattered(d.boxes, off, field, tiles_in)
@@ -237,7 +168,7 @@ def test_a_rank_that_never_arrives(oracle):
     off = hg.tile_offsets(d.boxes)
     tiles_in = random_bits(np.random.default_rng(7), int(off[-1]))
     for stall in range(G):
-        run = emu_frame(d.boxes, d.nbr, nx, ny, px, py, G, 1, "f", tiles_in, stall=stall)
+        run = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, 1, "f", tiles_in, stall=stall)
         assert run.err.tolist() == [0 if r == stall else 1 for r in range(G)], stall
         assert run.tiles[0].tobytes() == tiles_in.tobytes(), stall
 
@@ -249,7 +180,7 @@ def test_one_part_exchanges_nothing(oracle, G):
     d = oracle.partition(np.ones((ny, nx), dtype=np.int32), 1)
     off = hg.tile_offsets(d.boxes)
     tiles_in = np.full(int(off[-1]), SENTINEL, dtype=np.uint64)
-    run = emu_frame(d.boxes, d.nbr, nx, ny, True, True, G, 1, "ff", tiles_in)
+    run = halo_emu.run(d.boxes, d.nbr, nx, ny, True, True, G, 1, "ff", tiles_in)
     assert run.err.tolist() == [0] * G
     assert run.ids[1].tolist() == [[0]] * 4
     for i in range(2):
@@ -262,17 +193,7 @@ DDC_ERR_ARG, DDC_ERR_STATE = -1, -5
 
 @pytest.fixture(scope="module")
 def capi(oracle):
-    """domain_decomp_b200.capi bound to oracle/libddc_cuda_emu.so (as in test_c_abi_on_cpu_emulator)"""
-    import test_c_abi_on_cpu_emulator as A
-    from domain_decomp_b200 import capi as real
-    from conftest import ROOT
-    oracle.build()
-    lib = C.CDLL(os.path.join(ROOT, "oracle", "libddc_cuda_emu.so"))
-    ref = real.load()
-    for name in real.SYMBOLS:
-        getattr(lib, name).argtypes = getattr(ref, name).argtypes
-        getattr(lib, name).restype = getattr(ref, name).restype
-    return A.EmuCapi(real, lib)
+    return halo_emu.emu_capi(oracle)
 
 
 def host_view(ptr, n):

@@ -1,8 +1,8 @@
 """The sharded halo exchange (ddc_halo_exchange_shards_f64) on a machine without a GPU.
 
-tests/emu_halo_shards.cpp (built by tests/halo_emu.py) runs the product's own k_halo_open / k_halo_push / k_halo_close (ddc_kernels.cuh
-compiled as host C++) for G emulated ranks, phase by phase, each rank pushing into the others' buffers as it would
-over NVLink, and k_halo_exchange on one buffer beside them.  Interiors hold the global cell index, so every ghost
+tests/emu_halo.cpp (built by tests/halo_emu.py) runs the product's own k_halo_open / k_halo_push / k_halo_close
+(ddc_kernels.cuh compiled as host C++) for G emulated ranks, phase by phase, each rank pushing into the others' buffers
+as it would over NVLink, and k_halo_exchange on one buffer beside them.  Interiors hold the global cell index, so every ghost
 cell is checked for WHICH cell arrived (tests/halo_global.py); the sharded result must also equal the single-buffer
 kernel bit for bit, over three exchanges whose interiors change in between.  Says nothing about speed."""
 import itertools
@@ -26,10 +26,15 @@ def decomposition(oracle, seed, px, py):
 
 
 def run(oracle, d, nx, ny, px, py, G, periodic, steps=3, stall=-1):
+    """`steps` exchanges, each after a scatter of the global index + 1000 k into the interiors, with the library's
+    grids; returns the tiles before and the sharded and single-buffer tiles after each exchange (float64)"""
     off = hg.tile_offsets(d.boxes)
-    tiles_in = np.stack([hg.initial_tiles(d.boxes, off, nx, 1000.0 * k) for k in range(steps)])
-    out, single, err = halo_emu.emu_halo_shards(d, G, periodic, tiles_in, stall)
-    return off, tiles_in, out, single, err
+    tiles_in = hg.initial_tiles(d.boxes, off, nx)
+    fields = [np.arange(nx * ny, dtype=np.float64) + 1000.0 * k for k in range(steps)]
+    r = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, "sx" * steps, tiles_in, fields, stall=stall,
+                     grid_cap=0)
+    f64 = lambda a: a[1::2].view(np.float64)
+    return off, tiles_in[None], f64(r.tiles), f64(r.single), r.err
 
 
 @pytest.mark.parametrize("G", RANKS)
@@ -62,9 +67,7 @@ def test_more_ranks_than_parts(oracle):
 
 def test_one_part_is_a_no_op(oracle):
     d = oracle.partition(np.ones((9, 7), dtype=np.int32), 1)
-    off = hg.tile_offsets(d.boxes)
-    tiles_in = np.stack([hg.initial_tiles(d.boxes, off, 7)])
-    out, single, err = halo_emu.emu_halo_shards(d, 2, 1, tiles_in)
+    _, tiles_in, out, single, err = run(oracle, d, 7, 9, False, False, 2, 1, steps=1)
     assert np.array_equal(out[0], tiles_in[0]) and np.array_equal(single[0], tiles_in[0])
 
 

@@ -2487,6 +2487,9 @@ __global__ void __launch_bounds__(256) k_init(unsigned* __restrict__ colcount, i
 // overlap of the two boxes the ghost cells.  Corners are not exchanged here (a corner-touching box is no neighbour,
 // DomainUtils.cpp:15-35); the full-frame exchange adds them with k_halo_corners.  lists: bit l set = use list l
 // (l = periodic * 4 + edge).
+// A part of zero area is never a source: its list entries name no cell (its flattened box is empty, and a zero width
+// would be a divisor below).  When the boxes tile the domain that loses nothing: the box that holds the cell across a
+// ghost cannot overlap the receiver, so it touches the receiver's edge, is in the list and its halo covers the cell.
 template <typename T>
 __global__ void __launch_bounds__(256) k_halo_exchange(BoxTable bx, int P, const int* __restrict__ counts,
     const int* __restrict__ offsets, int cap, const int* __restrict__ ids, const int* __restrict__ halos,
@@ -2507,6 +2510,8 @@ __global__ void __launch_bounds__(256) k_halo_exchange(BoxTable bx, int P, const
         const size_t e = (size_t)l * cap + first + k;
         const int q = ids[e], h = halos[e], st = starts[e];
         const int qw = bx.ex[q];
+        if (qw <= 0 || bx.ey[q] <= 0)
+            continue; // a zero-area part is no source
         const T* theirs = tiles + off[q];
         const bool lr = edge < 2; // left / right: the shared cells run along y
         const int along = lr ? max(py0, bx.y0[q]) - py0 : max(px0, bx.x0[q]) - px0; // first shared cell along my edge
@@ -2658,7 +2663,8 @@ __device__ __forceinline__ void halo_push(const HaloShards& hs, BoxTable bx, con
             const int edge = lp & 3; // p's edge that faces q
             const int qw = bx.ex[q];
             const double* theirs = hs.tiles[hs.ps.rank] + (off[q] - off[hs.p_begin]);
-            const int n = counts[l * P + q], first = offsets[l * (P + 1) + q];
+            // a zero-area part is no source (k_halo_exchange): it pushes to none of its list entries
+            const int n = qw > 0 && bx.ey[q] > 0 ? counts[l * P + q] : 0, first = offsets[l * (P + 1) + q];
             for (int k = 0; k < n; k++) {
                 const int p = ids[(size_t)l * cap + first + k];
                 const int m = counts[lp * P + p];

@@ -269,8 +269,13 @@ DDC_API int ddc_halo_gather_shards_f64(ddc_handle_t h, double* rows_dev);
    part, or no DDC_WANT_NEIGHBOURS).  ddc_halo_exchange_full_shards_f64 is the same on the sharded buffers, with the
    checks and status codes of ddc_halo_exchange_shards_f64: it takes the next halo step number and mixes with sharded
    exchanges, scatters and gathers in any order that is the same on every rank.  A corner ghost is stored by the rank
-   that owns its source part.  (A zero-area part has no interior: an edge list entry whose source is such a part is
-   filled from that part's frame, by both exchanges alike, and what it holds then is not defined.) */
+   that owns its source part.
+   Parts of zero area, in every halo exchange above: a part of zero area is never a source; its entries in the edge
+   lists are skipped.  When the boxes tile the domain, which ddc_partition's always do, every ghost cell that faces a
+   neighbour therefore holds its (wrapped) cell, whatever the part sizes.  A zero-area receiver gets its ghosts by the
+   same rule: a zero-width part has a left and a right ghost column, a zero-height part a bottom and a top ghost row.
+   Boxes given to ddc_neighbours_from_boxes that overlap or leave cells uncovered are outside this rule: an edge ghost
+   may then have several sources, and which one it ends up holding is not defined. */
 DDC_API int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, int32_t* ids /* nparts */,
     int32_t* starts /* nparts */);
 DDC_API int ddc_halo_exchange_full_f64(ddc_handle_t h, double* tiles_dev, int periodic);

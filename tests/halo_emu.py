@@ -31,18 +31,22 @@ def _compiler():
     raise RuntimeError("no C++ compiler for the emulation harness")
 
 
-def lib() -> C.CDLL:
+def lib(sanitize=False) -> C.CDLL:
+    """the harness, compiled on the first call; later calls return it whatever they ask.  sanitize: built with
+    AddressSanitizer + UBSan, for a process that has libasan preloaded (tests/halo_asan_worker.py)."""
     global _lib
     if _lib is None:
         out = tempfile.mkdtemp(prefix="ddc_emu_halo_")
         atexit.register(shutil.rmtree, out, True)
         so = os.path.join(out, "libddc_emu_halo.so")
         emu = os.path.join(ROOT, "oracle", "emu")
-        subprocess.check_call([_compiler(), "-O2", "-std=c++17", "-fPIC", "-shared", "-fvisibility=hidden",
+        flags = ["-O1", "-g", "-fsanitize=address,undefined", "-fno-omit-frame-pointer"] if sanitize else ["-O2"]
+        env = {k: v for k, v in os.environ.items() if k != "LD_PRELOAD"}  # (the compiler runs without libasan)
+        subprocess.check_call([_compiler()] + flags + ["-std=c++17", "-fPIC", "-shared", "-fvisibility=hidden",
                                "-ffp-contract=off", "-U_FORTIFY_SOURCE", "-DDDC_HOST_EMU",
                                "-I" + os.path.join(ROOT, "domain_decomp_b200", "csrc"), "-I" + os.path.join(ROOT, "include"),
                                "-I" + emu, "-o", so, os.path.join(ROOT, "tests", "emu_halo.cpp"),
-                               os.path.join(emu, "cuda_emu.cpp")])
+                               os.path.join(emu, "cuda_emu.cpp")], env=env)
         L = C.CDLL(so)
         i32p = np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")
         f64p = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")

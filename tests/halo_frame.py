@@ -71,26 +71,35 @@ def with_corners(boxes, offsets, nx, ny, px, py, periodic, field, tiles, tables=
     return out
 
 
-def expected_full_tiles(boxes, offsets, nx, ny, px, py, periodic, add=0.0):
+def expected_full_tiles(boxes, offsets, nx, ny, px, py, periodic, add=0.0, tables=None):
     """halo_global.initial_tiles(add) after one full-frame exchange: the edge ghosts of halo_global.expected_tiles and
     every corner ghost with a source holding the global index of its wrapped cell (+ add); the rest UNTOUCHED"""
-    buf = hg.expected_tiles(boxes, offsets, nx, ny, px, py, periodic, add)
+    buf = hg.expected_tiles(boxes, offsets, nx, ny, px, py, periodic, add, tables)
     field = np.arange(nx * ny, dtype=np.float64).reshape(ny, nx) + add
-    return with_corners(boxes, offsets, nx, ny, px, py, periodic, field, buf)
+    return with_corners(boxes, offsets, nx, ny, px, py, periodic, field, buf, tables)
 
 
-def strip_tiling(rng, nx, ny, zero_width=True, zero_height=True):
+def strip_tiling(rng, nx, ny):
     """boxes [P, 4] that tile [0, nx) x [0, ny) as vertical strips cut into parts, some strips of width 0 and some parts
     of height 0 (the degenerate tilings RCB can leave on tiny grids)"""
-    def cuts(n, k, zeros):
-        c = np.sort(rng.integers(0 if zeros else 1, n + (1 if zeros else 0), size=k - 1))
-        if not zeros:
-            c = np.unique(c)
-        return np.concatenate([[0], c, [n]])
-    xs = cuts(nx, int(rng.integers(1, 5)), zero_width)
+    def cuts(n, k):
+        return np.concatenate([[0], np.sort(rng.integers(0, n + 1, size=k - 1)), [n]])
+    xs = cuts(nx, int(rng.integers(1, 5)))
     boxes = []
     for i in range(len(xs) - 1):
-        ys = cuts(ny, int(rng.integers(1, 5)), zero_height)
+        ys = cuts(ny, int(rng.integers(1, 5)))
         for j in range(len(ys) - 1):
             boxes.append((xs[i], ys[j], xs[i + 1] - xs[i], ys[j + 1] - ys[j]))
     return np.array(boxes, dtype=np.int32)
+
+
+def degenerate_cases(oracle):
+    """strip tilings with zero-height parts and zero-width strips, every periodic combination; their neighbour lists
+    are what ddc_neighbours_from_boxes computes for them (the oracle's restatement of discover_neighbours).  The lists
+    name the zero-area parts too; the exchanges never read one (a part of zero area is never a source)."""
+    for seed in range(12):
+        rng = np.random.default_rng(500 + seed)
+        nx, ny = int(rng.integers(3, 30)), int(rng.integers(3, 30))
+        boxes = strip_tiling(rng, nx, ny)
+        px, py = bool(seed & 1), bool(seed & 2)
+        yield boxes, oracle.neighbours(boxes, nx, ny, px, py), nx, ny, px, py, seed

@@ -54,11 +54,13 @@ def ghost_cells(boxes, offsets):
     return np.concatenate(idx), np.concatenate(xs), np.concatenate(ys)
 
 
-def expected_tiles(boxes, offsets, nx, ny, px, py, periodic, add=0.0):
-    """initial_tiles(add) after one exchange (interior lists; periodic: the periodic ones too)"""
+def expected_tiles(boxes, offsets, nx, ny, px, py, periodic, add=0.0, tables=None):
+    """initial_tiles(add) after one exchange (interior lists; periodic: the periodic ones too).  tables: whether the
+    handle has neighbour tables -- by default as after ddc_partition, which builds none for one part (and then the
+    exchange does nothing); ddc_neighbours_from_boxes builds them for one part too."""
     buf = initial_tiles(boxes, offsets, nx, add)
-    if len(boxes) < 2:
-        return buf  # one part: no neighbour tables, nothing is exchanged
+    if not (len(boxes) > 1 if tables is None else tables):
+        return buf
     idx, x, y = ghost_cells(boxes, offsets)
     ok = np.ones(len(idx), dtype=bool)
     if not (periodic and px):
@@ -138,11 +140,27 @@ def decomposition(oracle, seed, px, py):
     return oracle.partition(mask, P, px, py, use_hist=True), nx, ny
 
 
+def empty_part_cases(oracle):
+    """RCB output with empty parts: tiny grids cut into more parts than they have ocean columns or rows, which leaves
+    zero-height parts and zero-width strips, every periodic combination.  The boxes still tile the domain."""
+    out = []
+    for case, (px, py) in enumerate(itertools.product((False, True), repeat=2)):
+        for k, (nx, ny, P) in enumerate([(11, 11, 36), (6, 5, 19)]):
+            seed = 16 + 2 * case + k
+            rng = np.random.default_rng(900 + seed)
+            mask = (rng.random((ny, nx)) >= 0.6 + 0.3 * rng.random()).astype(np.int32)
+            out.append((oracle.partition(mask, P, px, py, use_hist=True), nx, ny, px, py, seed))
+    zero_width, zero_height = (any((d.boxes[:, i] == 0).any() for d, *_ in out) for i in (2, 3))
+    assert zero_width and zero_height, "the empty-part cases lost their zero-width strips or zero-height parts"
+    return out
+
+
 def cases(oracle):
     for case, (px, py) in enumerate(itertools.product((False, True), repeat=2)):
         for seed in (case, case + 4, case + 8, case + 12):
             d, nx, ny = decomposition(oracle, seed, px, py)
             yield d, nx, ny, px, py, seed
+    yield from empty_part_cases(oracle)
 
 
 # ---- the GPU tests (torch is passed in: this module imports without it) ----------------------------------------------
@@ -151,7 +169,20 @@ GPU_CASES = [  # nx, ny, P, px, py
     (2048, 1536, 1000, True, False),
     (8192, 8192, 4096, False, False),
 ]
+GPU_EMPTY_CASES = [  # nx, ny, P, px, py on empty_part_mask: more parts than ocean columns
+    (11, 11, 36, True, True),
+    (1024, 1024, 1024, True, False),
+]
 SENT = int(SENTINEL.view(np.int64))
+
+
+def empty_part_mask(nx, ny):
+    """ocean in a band of three rows across the middle and in one column: RCB cuts it into zero-width strips and
+    zero-height parts when there are more parts than ocean columns"""
+    mask = np.zeros((ny, nx), dtype=np.int32)
+    mask[ny // 2 - 1:ny // 2 + 2, :] = 1
+    mask[:, nx // 3] = 1
+    return mask
 
 
 class _Dev:
@@ -166,12 +197,21 @@ def dev_view(torch, ptr, n):
 
 
 def decompose(capi, torch, nx, ny, P, px, py, seed=3, land=0.45):
+    """a handle on device 0 with the decomposition of a generated mask; for a GPU_EMPTY_CASES case of empty_part_mask,
+    checked to have zero-width strips and zero-height parts"""
     h = capi.Handle(0)
     d_mask = torch.empty((ny, nx), dtype=torch.int32, device="cuda")
-    h.generate_mask_device(d_mask.data_ptr(), nx, ny, seed, land)
+    if (nx, ny, P, px, py) in GPU_EMPTY_CASES:
+        d_mask.copy_(torch.from_numpy(empty_part_mask(nx, ny)))
+        torch.cuda.synchronize()  # (the library works on its own stream)
+    else:
+        h.generate_mask_device(d_mask.data_ptr(), nx, ny, seed, land)
     h.set_mask_device(d_mask.data_ptr(), nx, ny)
     h.partition(P, px, py)
     h._mask = d_mask
+    if (nx, ny, P, px, py) in GPU_EMPTY_CASES:
+        b = h.boxes()
+        assert (b[:, 2] == 0).any() and (b[:, 3] == 0).any(), "no zero-width strip or no zero-height part"
     return h
 
 

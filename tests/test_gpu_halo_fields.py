@@ -15,8 +15,8 @@ import pytest
 
 import halo_global as hg
 from conftest import ROOT
-from halo_global import (GPU_CASES as CASES, SENT, SENTINEL, connect, decompose, dev_view, exchanged, random_field,
-                         scattered, u64)
+from halo_global import (GPU_CASES as CASES, GPU_EMPTY_CASES as EMPTY_CASES, SENT, SENTINEL, connect, decompose,
+                         dev_view, exchanged, random_field, scattered, u64)
 
 pytestmark = pytest.mark.gpu
 
@@ -42,7 +42,7 @@ def frame_cells(boxes, off):
     return np.concatenate(rows)
 
 
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_single_buffer(env, case):
     capi, torch = env
     nx, ny, P, px, py = case
@@ -89,7 +89,7 @@ def test_c5_round_trip(env):
     torch.cuda.empty_cache()
 
 
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_one_gpu_shards(env, case):
     capi, torch = env
     nx, ny, P, px, py = case

@@ -17,8 +17,8 @@ import pytest
 import halo_frame as hf
 import halo_global as hg
 from conftest import ROOT
-from halo_global import (GPU_CASES as CASES, SENT, SENTINEL, connect, decompose, dev_view, exchanged, random_field,
-                         scattered, u64)
+from halo_global import (GPU_CASES as CASES, GPU_EMPTY_CASES as EMPTY_CASES, SENT, SENTINEL, connect, decompose,
+                         dev_view, exchanged, random_field, scattered, u64)
 
 pytestmark = pytest.mark.gpu
 
@@ -32,7 +32,7 @@ def env():
     return capi, torch
 
 
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_single_buffer(env, case):
     capi, torch = env
     nx, ny, P, px, py = case
@@ -52,9 +52,26 @@ def test_single_buffer(env, case):
     h.close()
 
 
+def check_scattered_index(torch, boxes, off, tiles, nx, chunk=1 << 27):
+    """every interior cell of the tiles holds its global index y * nx + x, every frame cell UNTOUCHED: on the tiles'
+    device, `chunk` buffer cells at a time"""
+    b = torch.from_numpy(np.asarray(boxes, dtype=np.int64)).to(tiles.device)
+    o = torch.from_numpy(np.asarray(off, dtype=np.int64)).to(tiles.device)
+    for k0 in range(0, int(off[-1]), chunk):
+        k = torch.arange(k0, min(k0 + chunk, int(off[-1])), device=tiles.device)
+        p = torch.searchsorted(o, k, right=True) - 1
+        x0, y0, ex, ey = b[p].unbind(1)
+        r, c = (k - o[p]) // (ex + 2), (k - o[p]) % (ex + 2)
+        inside = (r >= 1) & (r <= ey) & (c >= 1) & (c <= ex)
+        want = torch.where(inside, ((y0 + r - 1) * nx + x0 + c - 1).double(), hg.UNTOUCHED)
+        assert torch.equal(tiles[k0:k0 + len(k)], want), k0
+        del k, p, x0, y0, ex, ey, r, c, inside, want
+
+
 def test_c5_edges_and_corners(env):
-    """C5 (32768^2, 16384 parts, periodic in x): the full exchange leaves every non-corner cell as
-    ddc_halo_exchange_f64 does, and every one of the 4 P corners as the corner table says (about 35 GB)"""
+    """C5 (32768^2, 16384 parts, periodic in x), interiors the global index: the scatter puts every cell where it
+    belongs, the edge exchange gives every edge ghost its wrapped cell (16.7 M), the full exchange leaves every non-corner
+    cell as the edge exchange does, and every one of the 4 P corners as the corner table says (about 35 GB)"""
     capi, torch = env
     nx = ny = 32768
     px, py = True, False
@@ -68,11 +85,16 @@ def test_c5_edges_and_corners(env):
     h.halo_scatter_f64(field.data_ptr(), edge.data_ptr())
     h.synchronize()
     del field
+    check_scattered_index(torch, boxes, off, edge, nx)
     full = edge.clone()
     torch.cuda.synchronize()
     h.halo_exchange_f64(edge.data_ptr(), True)
     h.halo_exchange_full_f64(full.data_ptr(), True)
     h.synchronize()
+    gi, gx, gy = (torch.from_numpy(a).cuda() for a in hg.ghost_cells(boxes, off))
+    want = torch.where((gy >= 0) & (gy < ny), ((gy % ny) * nx + gx % nx).double(), hg.UNTOUCHED)  # px, not py
+    assert len(gi) > 16_000_000 and torch.equal(edge[gi], want)
+    del gi, gx, gy, want
     idx = torch.from_numpy(hf.corner_cells(boxes, off).reshape(-1)).cuda()
     got = full[idx].cpu().numpy()
     assert bool((edge[idx] == hg.UNTOUCHED).all())
@@ -89,7 +111,7 @@ def test_c5_edges_and_corners(env):
     torch.cuda.empty_cache()
 
 
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_one_gpu_shards(env, case):
     """scatter, full exchange, edge exchange, full exchange, gather on G handles sharing the B200, against the single
     buffer after every call"""
@@ -156,7 +178,7 @@ def box_sum_tiles(boxes, off, tiles):
     return out
 
 
-@pytest.mark.parametrize("case", CASES[:2], ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES[:2] + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_nine_point_stencil(env, case):
     """scatter -> full exchange -> 3 x 3 box sum per tile -> gather == the box sum of the global field, zero-padded in
     non-periodic directions and wrapped in periodic ones (integer-valued doubles: the sums are exact)"""

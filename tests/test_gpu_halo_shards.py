@@ -13,7 +13,7 @@ import pytest
 
 import halo_global as hg
 from conftest import ROOT
-from halo_global import GPU_CASES as CASES, decompose, dev_view
+from halo_global import GPU_CASES as CASES, GPU_EMPTY_CASES as EMPTY_CASES, decompose, dev_view
 
 pytestmark = pytest.mark.gpu
 
@@ -67,7 +67,7 @@ def check_exchanges(capi, torch, single_h, handles, ptrs, nx, ny, px, py, steps=
             assert np.array_equal(cat.cpu().numpy(), want), ctx
 
 
-@pytest.mark.parametrize("case", CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
+@pytest.mark.parametrize("case", CASES + EMPTY_CASES, ids=lambda c: "%dx%d_p%d" % c[:3])
 def test_one_gpu_shards(env, case):
     capi, torch = env
     nx, ny, P, px, py = case

@@ -16,23 +16,11 @@ import pytest
 import halo_emu
 import halo_frame as hf
 import halo_global as hg
+from halo_frame import degenerate_cases
 from halo_global import SENTINEL, cases, exchanged, random_bits, scattered
 
 RANKS = (1, 2, 3, 5)
 SEEDS = ("0", "11", "4242")  # DDC_EMU_SCHED_SEED: "0" index order, otherwise random block / thread schedules
-
-
-def degenerate_cases(oracle, zero_width=True):
-    """strip tilings with zero-height parts and (zero_width) zero-width strips, every periodic combination; their
-    neighbour lists are what ddc_neighbours_from_boxes computes for them (the oracle's restatement of
-    discover_neighbours).  The exchanges run without zero-width strips: the edge exchange divides by the source's width
-    (k_halo_exchange, k_halo_push), which the emulation traps on."""
-    for seed in range(12):
-        rng = np.random.default_rng(500 + seed)
-        nx, ny = int(rng.integers(3, 30)), int(rng.integers(3, 30))
-        boxes = hf.strip_tiling(rng, nx, ny, zero_width=zero_width)
-        px, py = bool(seed & 1), bool(seed & 2)
-        yield boxes, oracle.neighbours(boxes, nx, ny, px, py), nx, ny, px, py, seed
 
 
 def as_bits(a):
@@ -72,8 +60,6 @@ def test_full_exchange_fills_the_whole_frame(oracle, monkeypatch, G, sched):
     or stays UNTOUCHED; edges equal ddc_halo_exchange_f64's; sharded equals the single buffer"""
     monkeypatch.setenv("DDC_EMU_SCHED_SEED", sched)
     for d, nx, ny, px, py, seed in cases(oracle):
-        if (d.boxes[:, 2:] <= 0).any():
-            continue  # halo_global's edge expectation assumes no empty part (the degenerate test covers them)
         off = hg.tile_offsets(d.boxes)
         tiles_in = as_bits(hg.initial_tiles(d.boxes, off, nx))
         for periodic in (0, 1):
@@ -90,42 +76,24 @@ def test_full_exchange_fills_the_whole_frame(oracle, monkeypatch, G, sched):
             assert (edge.single[0][corners] == as_bits(hg.UNTOUCHED)).all(), ctx
 
 
-def fed_by_empty_parts(boxes, nbr, offsets, periodic):
-    """buffer indices of the tiles with an empty part in one of their edge lists.  An empty part has no interior: the
-    edge exchange reads the ghosts it feeds from its frame, which the same exchange is writing, so those tiles' edge
-    ghosts depend on the schedule (in the edge exchange as much as in the full one) and are left out of comparisons."""
-    empty = (np.asarray(boxes)[:, 2:] <= 0).any(axis=1)
-    P = len(boxes)
-    hit = np.zeros(P, dtype=bool)
-    for per in range(2 if periodic else 1):
-        for e in range(4):
-            owner = np.repeat(np.arange(P), nbr.counts[per][e])
-            hit[owner[empty[nbr.ids[per][e]]]] = True
-    off = np.asarray(offsets, dtype=np.int64)
-    return np.concatenate([np.arange(off[p], off[p + 1]) for p in np.nonzero(hit)[0]] + [np.zeros(0, np.int64)])
-
-
 @pytest.mark.parametrize("G", RANKS)
 def test_degenerate_tilings(oracle, G):
-    """zero-width strips and zero-height parts (ddc_neighbours_from_boxes input): every corner ghost from the brute-force
-    table, on one buffer and sharded; every other frame cell as the edge exchange leaves it"""
-    for boxes, nbr, nx, ny, px, py, seed in degenerate_cases(oracle, zero_width=False):
+    """zero-width strips and zero-height parts (ddc_neighbours_from_boxes input): every ghost of the edge and the
+    full exchange holds the cell across it, zero-area receivers included, on one buffer and sharded"""
+    for boxes, nbr, nx, ny, px, py, seed in degenerate_cases(oracle):
         off = hg.tile_offsets(boxes)
         tiles_in = as_bits(hg.initial_tiles(boxes, off, nx))
-        field = np.arange(nx * ny, dtype=np.float64).reshape(ny, nx)
-        corners = hf.corner_cells(boxes, off).reshape(-1)
         for periodic in (0, 1):
             ctx = (G, seed, nx, ny, len(boxes), periodic)
             full = halo_emu.run(boxes, nbr, nx, ny, px, py, G, periodic, "f", tiles_in)
             edge = halo_emu.run(boxes, nbr, nx, ny, px, py, G, periodic, "x", tiles_in)
-            assert full.err.tolist() == [0] * G, ctx
-            want = as_bits(hf.with_corners(boxes, off, nx, ny, px, py, periodic, field,
-                                           edge.single[0].view(np.float64)))
-            keep = np.ones(int(off[-1]), dtype=bool)
-            keep[fed_by_empty_parts(boxes, nbr, off, periodic)] = False
-            keep[corners] = True
-            assert np.array_equal(full.single[0][keep], want[keep]), ctx
-            assert np.array_equal(full.tiles[0][keep], want[keep]), ctx
+            assert full.err.tolist() == [0] * G and edge.err.tolist() == [0] * G, ctx
+            want = as_bits(hg.expected_tiles(boxes, off, nx, ny, px, py, periodic))
+            assert np.array_equal(edge.single[0], want), ctx + ("edge, single buffer",)
+            assert np.array_equal(edge.tiles[0], want), ctx + ("edge, sharded",)
+            want = as_bits(hf.expected_full_tiles(boxes, off, nx, ny, px, py, periodic))
+            assert np.array_equal(full.single[0], want), ctx + ("full, single buffer",)
+            assert np.array_equal(full.tiles[0], want), ctx + ("full, sharded",)
 
 
 @pytest.mark.parametrize("G", RANKS)
@@ -135,8 +103,6 @@ def test_mixed_sequence_on_one_step_counter(oracle, monkeypatch, G, sched):
     harness checks after every op that each block counter is back at zero and no rank stored outside its rows"""
     monkeypatch.setenv("DDC_EMU_SCHED_SEED", sched)
     for d, nx, ny, px, py, seed in cases(oracle):
-        if (d.boxes[:, 2:] <= 0).any():
-            continue
         rng = np.random.default_rng(seed + 300)
         off = hg.tile_offsets(d.boxes)
         periodic = seed & 1
@@ -206,8 +172,9 @@ def table_of(h):
 
 
 @pytest.mark.parametrize("nx,ny,P,px,py", [(37, 29, 7, True, False), (50, 41, 12, True, True), (23, 70, 9, False, True),
-                                           (40, 30, 1, True, True)])
+                                           (40, 30, 1, True, True), (6, 5, 25, True, True), (6, 5, 18, False, False)])
 def test_c_abi_single_buffer(capi, nx, ny, P, px, py):
+    """the last two: more parts than columns, so that ddc_partition leaves zero-width strips and zero-height parts"""
     rng = np.random.default_rng(P)
     mask = (rng.random((ny, nx)) > 0.35).astype(np.int32)
     h = capi.Handle(0)
@@ -215,6 +182,8 @@ def test_c_abi_single_buffer(capi, nx, ny, P, px, py):
         h.set_mask_host(mask)
         h.partition(P, px, py)
         boxes = h.boxes()
+        if P > nx:
+            assert (boxes[:, 2] == 0).any() and (boxes[:, 3] == 0).any(), boxes.tolist()
         ids, starts = table_of(h)
         want_ids, want_starts = hf.corner_table(boxes, nx, ny, px, py)
         assert np.array_equal(ids, want_ids) and np.array_equal(starts, want_starts)
@@ -230,7 +199,8 @@ def test_c_abi_single_buffer(capi, nx, ny, P, px, py):
 
 
 def test_c_abi_degenerate_boxes(capi, oracle):
-    """ddc_neighbours_from_boxes input: the getter and the full exchange on zero-width strips and zero-height parts"""
+    """ddc_neighbours_from_boxes input: the getter, the edge and the full exchange on zero-width strips and zero-height
+    parts"""
     h = capi.Handle(0)
     try:
         for boxes, nbr, nx, ny, px, py, seed in degenerate_cases(oracle):
@@ -238,19 +208,15 @@ def test_c_abi_degenerate_boxes(capi, oracle):
             ids, starts = table_of(h)
             want_ids, want_starts = hf.corner_table(boxes, nx, ny, px, py)
             assert np.array_equal(ids, want_ids) and np.array_equal(starts, want_starts), seed
-        for boxes, nbr, nx, ny, px, py, seed in degenerate_cases(oracle, zero_width=False):
-            h.neighbours_from_boxes(boxes, nx, ny, px, py)
             off = h.halo_tile_offsets()
             edge, full = hg.initial_tiles(boxes, off, nx), hg.initial_tiles(boxes, off, nx)
             h.halo_exchange_f64(edge.ctypes.data, 1)
             h.halo_exchange_full_f64(full.ctypes.data, 1)
             h.synchronize()
-            field = np.arange(nx * ny, dtype=np.float64).reshape(ny, nx)
-            want = hf.with_corners(boxes, off, nx, ny, px, py, 1, field, edge, tables=True)
-            keep = np.ones(int(off[-1]), dtype=bool)
-            keep[fed_by_empty_parts(boxes, nbr, off, 1)] = False
-            keep[hf.corner_cells(boxes, off).reshape(-1)] = True
-            assert full[keep].tobytes() == want[keep].tobytes(), seed
+            want = hg.expected_tiles(boxes, off, nx, ny, px, py, 1, tables=True)
+            assert edge.tobytes() == want.tobytes(), seed
+            want = hf.expected_full_tiles(boxes, off, nx, ny, px, py, 1, tables=True)
+            assert full.tobytes() == want.tobytes(), seed
     finally:
         h.close()
 

@@ -41,17 +41,18 @@ def run(oracle, d, nx, ny, px, py, G, periodic, steps=3, stall=-1):
 @pytest.mark.parametrize("sched", SEEDS)
 def test_sharded_exchange_matches_single_buffer_and_expected(oracle, monkeypatch, G, sched):
     monkeypatch.setenv("DDC_EMU_SCHED_SEED", sched)
-    for case, (px, py) in enumerate(itertools.product((False, True), repeat=2)):
-        for seed in (case, case + 4, case + 8):
-            d, nx, ny = decomposition(oracle, seed, px, py)
-            for periodic in (0, 1):
-                ctx = (G, sched, seed, px, py, periodic, d.P)
-                off, _, out, single, err = run(oracle, d, nx, ny, px, py, G, periodic)
-                assert err.tolist() == [0] * G, ctx
-                for k in range(out.shape[0]):
-                    want = hg.expected_tiles(d.boxes, off, nx, ny, px, py, periodic, 1000.0 * k)
-                    assert np.array_equal(single[k], want), ctx + (k, "single-buffer kernel")
-                    assert out[k].tobytes() == single[k].tobytes(), ctx + (k, "sharded != single buffer")
+    todo = [(decomposition(oracle, seed, px, py), px, py, seed)
+            for case, (px, py) in enumerate(itertools.product((False, True), repeat=2)) for seed in (case, case + 4, case + 8)]
+    todo += [((d, nx, ny), px, py, seed) for d, nx, ny, px, py, seed in hg.empty_part_cases(oracle)]
+    for (d, nx, ny), px, py, seed in todo:
+        for periodic in (0, 1):
+            ctx = (G, sched, seed, px, py, periodic, d.P)
+            off, _, out, single, err = run(oracle, d, nx, ny, px, py, G, periodic)
+            assert err.tolist() == [0] * G, ctx
+            for k in range(out.shape[0]):
+                want = hg.expected_tiles(d.boxes, off, nx, ny, px, py, periodic, 1000.0 * k)
+                assert np.array_equal(single[k], want), ctx + (k, "single-buffer kernel")
+                assert out[k].tobytes() == single[k].tobytes(), ctx + (k, "sharded != single buffer")
 
 
 def test_more_ranks_than_parts(oracle):

@@ -36,6 +36,7 @@ SYMBOLS = (
     "ddc_halo_exchange_shards_f64", "ddc_halo_close",
     "ddc_halo_scatter_f64", "ddc_halo_gather_f64", "ddc_halo_scatter_shards_f64", "ddc_halo_gather_shards_f64",
     "ddc_get_corner_neighbours", "ddc_halo_exchange_full_f64", "ddc_halo_exchange_full_shards_f64",
+    "ddc_halo_set_width",
 )
 
 
@@ -117,6 +118,7 @@ def load() -> C.CDLL:
     L.ddc_get_corner_neighbours.argtypes = [vp, i32, i32, vp, vp]
     L.ddc_halo_exchange_full_f64.argtypes = [vp, vp, i32]
     L.ddc_halo_exchange_full_shards_f64.argtypes = [vp, i32]
+    L.ddc_halo_set_width.argtypes = [vp, i32]
     L.ddc_generate_mask_device.argtypes = [vp, vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     L.ddc_generate_mask_host.argtypes = [vp, i32, i32, i32, i32, C.c_uint64, C.c_double]
     _lib = L
@@ -337,6 +339,10 @@ class Handle:
     def halo_exchange_full_shards_f64(self, periodic: bool = False):
         """halo_exchange_shards_f64 plus the corner ghosts"""
         self._ck(self.L.ddc_halo_exchange_full_shards_f64(self.h, int(periodic)), "ddc_halo_exchange_full_shards_f64")
+
+    def halo_set_width(self, w: int):
+        """frames of width w for every halo call (ddc_halo_set_width); take the tile / shard offsets again after it"""
+        self._ck(self.L.ddc_halo_set_width(self.h, int(w)), "ddc_halo_set_width")
 
     def neighbour_counts(self, edge: int, periodic: int) -> np.ndarray:
         out = np.empty(self.nparts, dtype=np.int32)

@@ -190,6 +190,7 @@ struct ddc_handle_s {
     DevBuf<unsigned char> halo_dev;
     bool halo_ok = false; // the plan is of the current decomposition
     bool halo_shard_ok = false; // ... and ddc_halo_shard_offsets was called for it
+    int halo_w = 1; // the frame width of the halo calls (ddc_halo_set_width)
     DevBuf<unsigned> gate; // the word the gate kernel of the second stream waits for (see BoxGate)
     int use_gate = 1; // DDC_GATE: 0 never, 1 unless the shard is tiny, 2 always
     bool side_pdl = true; // DDC_SIDE_PDL: the scan of the neighbour counts launched programmatically behind the count kernel
@@ -1785,12 +1786,13 @@ static int build_halo_plan(ddc_handle_t h, HaloPlan& hp)
     int yb, yc;
     ddc_shard_rows(h->ny, h->nranks, h->rank, &yb, &yc);
     hp = halo_plan(P, h->nranks, h->rank, h->nx, h->ny, h->px, h->py, box[0].data(), box[1].data(), box[2].data(),
-        box[3].data(), yb, yc);
+        box[3].data(), yb, yc, h->halo_w);
     return DDC_OK;
 }
 
 // the halo plan of the current decomposition, also left on the device for the halo kernels: the tile offsets of all
-// parts in one buffer, the (part, row) ranges of scatter and gather and the corner items of the full-frame exchange.
+// parts in one buffer, the (part, row) ranges of scatter and gather and the corner items of the full-frame exchange
+// (w = 1) or the rectangle items of both exchanges (w >= 2).
 // Everything is built here, where the host may wait for the stream: a sharded call must not wait (one host thread may
 // drive several ranks, whose open kernels wait for each other).
 static int tile_offsets(ddc_handle_t h)
@@ -1803,6 +1805,19 @@ static int tile_offsets(ddc_handle_t h)
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->halo = std::move(hp);
     h->halo_ok = true;
+    return DDC_OK;
+}
+
+int ddc_halo_set_width(ddc_handle_t h, int width)
+{
+    if (!h)
+        return DDC_ERR_ARG;
+    if (width < 1 || width > DDC_MAX_HALO_WIDTH)
+        return fail(h, DDC_ERR_ARG, "ddc_halo_set_width: width %d is not in 1..%d", width, DDC_MAX_HALO_WIDTH);
+    if (width != h->halo_w) {
+        h->halo_w = width;
+        halo_invalidate(h); // another layout: the tile and shard offsets are to be taken again
+    }
     return DDC_OK;
 }
 
@@ -1837,7 +1852,8 @@ int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, int32_t*
     return DDC_OK;
 }
 
-// one buffer: the edge ghosts (k_halo_exchange), and with `full` the corner ghosts after them (k_halo_corners)
+// one buffer: the edge ghosts (k_halo_exchange), and with `full` the corner ghosts after them (k_halo_corners); wide
+// frames: the rectangle items of both (k_halo_rects)
 static int halo_exchange(ddc_handle_t h, double* tiles_dev, int periodic, bool full, const char* name)
 {
     if (!tiles_dev)
@@ -1846,6 +1862,14 @@ static int halo_exchange(ddc_handle_t h, double* tiles_dev, int periodic, bool f
         return fail(h, DDC_ERR_STATE, "%s: call ddc_halo_tile_offsets() for this decomposition first", name);
     if (!h->have_nbr)
         return DDC_OK; // one part (or no tables asked for): nothing to exchange
+    if (h->halo.w > 1) {
+        const HaloRects rects = h->halo.rects(h->halo_dev.p, 0, periodic, full);
+        if (rects.n > 0)
+            CUDA_TRY(h, launch_k(k_halo_rects, dim3(halo_field_grid(rects.n)), dim3(256), 0, h->stream, false, rects,
+                tiles_dev));
+        CUDA_TRY(h, cudaGetLastError());
+        return DDC_OK;
+    }
     int rc = fetch_totals(h); // (re-runs the fill pass with the exact capacity if the bounded one overflowed)
     if (rc)
         return rc;
@@ -1942,6 +1966,7 @@ static int halo_alloc(ddc_handle_t h, int64_t elems)
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_close));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<true>));
     CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_field_shards<false>));
+    CUDA_TRY(h, cudaFuncGetAttributes(&fa, k_halo_push_rects));
     h->halo_elems = elems;
     h->halo_step = 0;
     return DDC_OK;
@@ -2027,13 +2052,20 @@ static int halo_shards_call(ddc_handle_t h, Middle middle)
 }
 }
 
-// the edge ghosts (k_halo_push), and with `full` the corner ghosts beside them (k_halo_push_full)
+// the edge ghosts (k_halo_push), and with `full` the corner ghosts beside them (k_halo_push_full); wide frames: the
+// rectangle items of both whose source part this rank owns (k_halo_push_rects)
 static int halo_exchange_shards(ddc_handle_t h, int periodic, bool full, const char* name)
 {
     if (int rc = halo_shards_ready(h, name))
         return rc;
     if (!h->have_nbr)
         return DDC_OK; // one part (or no tables asked for): nothing to exchange, no step taken
+    if (h->halo.w > 1) {
+        const HaloRects rects = h->halo.rects(h->halo_dev.p, 1, periodic, full);
+        return halo_shards_call(h, [&](const HaloShards& hs) {
+            return launch_k(k_halo_push_rects, dim3(halo_field_grid(rects.n)), dim3(256), 0, h->stream, false, hs, rects);
+        });
+    }
     if (int rc = fetch_totals(h)) // (may wait for the stream: before anything of the exchange is enqueued)
         return rc;
     Tables t = tables(h, h->nparts);

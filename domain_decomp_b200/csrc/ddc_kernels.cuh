@@ -31,6 +31,7 @@
 #include <stdint.h>
 
 #include <algorithm>
+#include <climits>
 #include <vector>
 
 #include "ddc_median.cuh"
@@ -2743,7 +2744,8 @@ __global__ void __launch_bounds__(32) k_halo_close(HaloShards hs)
 // tile is at element base[k] of the buffer of rank owner[k] (one buffer: owner 0, base = the ddc_halo_tile_offsets
 // offset; sharded: rebased to the owner's first part).  The host computes both: in a kernel, the 64-bit divisions that
 // find the owner are a subroutine call, and the registers saved around it spill.
-// Only non-empty ranges are listed, so first[] is strictly increasing.
+// Only non-empty ranges are listed, so first[] is strictly increasing.  With a frame of width w (ddc_halo_set_width)
+// the interior cell (i, j) is at row j + w, column i + w of a tile that is ex + 2 w wide.
 struct HaloItems {
     const int* part; // [n]
     const int* j0; // [n]
@@ -2751,6 +2753,7 @@ struct HaloItems {
     const int* first; // [n + 1], first[0] = 0, first[n] = all items
     const long long* base; // [n]
     int n;
+    int w; // the frame width
 };
 // the ranges of the field rows [lo, hi) with the parts sharded over G ranks (G = 1: one buffer) into
 // out[4 P + 1] = [part: P][j0: P][owner: P][first: P + 1] and base[P]; y0 / ex / ey: the boxes, off: the
@@ -2825,10 +2828,10 @@ __device__ __forceinline__ void halo_copy_items(const HaloItems& it, BoxTable bx
     }
     while (w < end) {
         const int p = it.part[k], ex = bx.ex[p], stop = min(end, it.first[k + 1]);
-        int j = it.j0[k] + (w - it.first[k]);
-        unsigned long long* tile = reinterpret_cast<unsigned long long*>(tile_of(k)) + (size_t)(j + 1) * (ex + 2) + 1;
+        const int j = it.j0[k] + (w - it.first[k]), tw = ex + 2 * it.w;
+        unsigned long long* tile = reinterpret_cast<unsigned long long*>(tile_of(k)) + (size_t)(j + it.w) * tw + it.w;
         unsigned long long* row = reinterpret_cast<unsigned long long*>(field) + (size_t)(bx.y0[p] + j - y_base) * nx + bx.x0[p];
-        for (; w < stop; w++, tile += ex + 2, row += nx)
+        for (; w < stop; w++, tile += tw, row += nx)
             halo_copy_row<kScatter>(tile, row, ex, lane);
         k++;
     }
@@ -2867,44 +2870,50 @@ __global__ void __launch_bounds__(256) k_halo_field_shards(HaloShards hs, HaloIt
 // which it lies outside, all of which must be periodic.  A box that touches p only at a corner has no domain overlap
 // with p, so no edge list names it, and zero-area parts have no lists at all: the owner is found by point location.
 // Host code, part of halo_plan.
-//   ids / starts [2][4][P]: set (0 interior, 1 periodic), corner, part -> source part (-1: none) and the cell's index
-//   (y - y0[q]) * ex[q] + (x - x0[q]) in the source's flattened box (the halo_start convention).  For each (corner,
-//   part) at most one of the two sets has a source.
-inline void halo_corner_sources(int P, int nx, int ny, int px, int py, const int* x0, const int* y0, const int* ex,
-    const int* ey, int* ids, int* starts)
-{
-    // A bucket grid of about sqrt(P) x sqrt(P) over the domain; every positive-area box is registered, in id order, in
-    // each bucket it overlaps, so the first box of a bucket that contains a cell is its lowest-id source.  About one
-    // bucket per box for RCB output; still correct (only slower) for overlapping or degenerate caller boxes.
-    int side = 1;
-    while ((long long)side * side < P)
-        side++;
-    const int bw = std::min(side, nx), bh = std::min(side, ny);
-    const auto bucket_x = [&](int x) { return (int)((long long)x * bw / nx); };
-    const auto bucket_y = [&](int y) { return (int)((long long)y * bh / ny); };
-    std::vector<int> first((size_t)bw * bh + 1, 0), list;
-    for (int pass = 0; pass < 2; pass++) {
-        std::vector<int> fill(first.begin(), first.end() - 1);
-        for (int q = 0; q < P; q++) {
-            const int xa = std::max(x0[q], 0), xb = (int)std::min((long long)x0[q] + ex[q], (long long)nx) - 1;
-            const int ya = std::max(y0[q], 0), yb = (int)std::min((long long)y0[q] + ey[q], (long long)ny) - 1;
-            if (ex[q] <= 0 || ey[q] <= 0 || xa > xb || ya > yb)
-                continue;
-            for (int j = bucket_y(ya); j <= bucket_y(yb); j++)
-                for (int i = bucket_x(xa); i <= bucket_x(xb); i++) {
-                    if (pass == 0)
-                        first[(size_t)j * bw + i + 1]++;
-                    else
-                        list[fill[(size_t)j * bw + i]++] = q;
-                }
-        }
-        if (pass == 0) {
-            for (size_t b = 0; b < (size_t)bw * bh; b++)
-                first[b + 1] += first[b];
-            list.resize((size_t)first.back());
+// The point location of the halo plan: a bucket grid of about sqrt(P) x sqrt(P) over the domain; every positive-area
+// box is registered, in id order, in each bucket it overlaps, so the first box of a bucket that contains a cell is its
+// lowest-id source.  About one bucket per box for RCB output; still correct (only slower) for overlapping or degenerate
+// caller boxes.
+struct HaloBuckets {
+    int nx, ny, bw, bh;
+    const int *x0, *y0, *ex, *ey;
+    std::vector<int> first, list;
+    int bucket_x(int x) const { return (int)((long long)x * bw / nx); }
+    int bucket_y(int y) const { return (int)((long long)y * bh / ny); }
+    HaloBuckets(int P, int nx_, int ny_, const int* x0_, const int* y0_, const int* ex_, const int* ey_)
+        : nx(nx_), ny(ny_), x0(x0_), y0(y0_), ex(ex_), ey(ey_)
+    {
+        int side = 1;
+        while ((long long)side * side < P)
+            side++;
+        bw = std::min(side, nx);
+        bh = std::min(side, ny);
+        first.assign((size_t)bw * bh + 1, 0);
+        for (int pass = 0; pass < 2; pass++) {
+            std::vector<int> fill(first.begin(), first.end() - 1);
+            for (int q = 0; q < P; q++) {
+                const int xa = std::max(x0[q], 0), xb = (int)std::min((long long)x0[q] + ex[q], (long long)nx) - 1;
+                const int ya = std::max(y0[q], 0), yb = (int)std::min((long long)y0[q] + ey[q], (long long)ny) - 1;
+                if (ex[q] <= 0 || ey[q] <= 0 || xa > xb || ya > yb)
+                    continue;
+                for (int j = bucket_y(ya); j <= bucket_y(yb); j++)
+                    for (int i = bucket_x(xa); i <= bucket_x(xb); i++) {
+                        if (pass == 0)
+                            first[(size_t)j * bw + i + 1]++;
+                        else
+                            list[fill[(size_t)j * bw + i]++] = q;
+                    }
+            }
+            if (pass == 0) {
+                for (size_t b = 0; b < (size_t)bw * bh; b++)
+                    first[b + 1] += first[b];
+                list.resize((size_t)first.back());
+            }
         }
     }
-    const auto locate = [&](int x, int y) {
+    // the lowest-id positive-area box that contains cell (x, y) of the domain, -1 if none does
+    int locate(int x, int y) const
+    {
         const size_t b = (size_t)bucket_y(y) * bw + bucket_x(x);
         for (int k = first[b]; k < first[b + 1]; k++) {
             const int q = list[k];
@@ -2912,7 +2921,31 @@ inline void halo_corner_sources(int P, int nx, int ny, int px, int py, const int
                 return q;
         }
         return -1;
-    };
+    }
+    // f(q, xa, xb, ya, yb) once for every positive-area box q that overlaps [xa, xb) x [ya, yb) (inside the domain),
+    // with the overlap: a box that spans several buckets is taken in the bucket of the overlap's first cell only
+    template <typename F>
+    void overlapping(int xa, int xb, int ya, int yb, F f) const
+    {
+        for (int j = bucket_y(ya); j <= bucket_y(yb - 1); j++)
+            for (int i = bucket_x(xa); i <= bucket_x(xb - 1); i++)
+                for (int k = first[(size_t)j * bw + i]; k < first[(size_t)j * bw + i + 1]; k++) {
+                    const int q = list[k];
+                    const int ia = std::max(xa, x0[q]), ib = (int)std::min((long long)xb, (long long)x0[q] + ex[q]);
+                    const int ja = std::max(ya, y0[q]), jb = (int)std::min((long long)yb, (long long)y0[q] + ey[q]);
+                    if (ia < ib && ja < jb && bucket_x(ia) == i && bucket_y(ja) == j)
+                        f(q, ia, ib, ja, jb);
+                }
+    }
+};
+
+//   ids / starts [2][4][P]: set (0 interior, 1 periodic), corner, part -> source part (-1: none) and the cell's index
+//   (y - y0[q]) * ex[q] + (x - x0[q]) in the source's flattened box (the halo_start convention).  For each (corner,
+//   part) at most one of the two sets has a source.
+inline void halo_corner_sources(int P, int nx, int ny, int px, int py, const HaloBuckets& bk, int* ids, int* starts)
+{
+    const int *x0 = bk.x0, *y0 = bk.y0, *ex = bk.ex, *ey = bk.ey;
+    const auto locate = [&](int x, int y) { return bk.locate(x, y); };
     for (int c = 0; c < 4; c++)
         for (int p = 0; p < P; p++) {
             const long long x = c & 1 ? (long long)x0[p] + std::max(ex[p], 0) : x0[p] - 1LL;
@@ -2968,23 +3001,184 @@ __global__ void __launch_bounds__(256) k_halo_corners(HaloCorners corners, doubl
 }
 
 // ------------------------------------------------------------------------------------------------
+// Wide frames (ddc_halo_set_width, w >= 2): the ghosts as rectangle copies
+// ------------------------------------------------------------------------------------------------
+// Tile p is (ey + 2 w) x (ex + 2 w); its frame cell (x, y) -- x0 - w <= x < x0 + ex + w, the same in y, outside the box
+// -- is at row y - y0 + w, column x - x0 + w.  Its source is the positive-area box that contains the cell: the cell
+// itself when it lies in [0, nx) x [0, ny) (interior set), else the cell wrapped (x mod nx, y mod ny) if the
+// decomposition is periodic in every direction in which it lies outside (periodic set).  This is the corner rule of
+// halo_corner_sources applied to every frame cell; at w = 1 on a tiling it selects exactly the ghosts the edge lists
+// fill.  The neighbour lists cannot serve w >= 2: the box two cells away need not touch p.
+// The host cuts each of the 8 frame regions of every part (4 edge strips, 4 w x w corner blocks) into its wrapped
+// pieces -- a strip wider than the domain wraps as often as it needs -- drops the pieces across a non-periodic
+// boundary and intersects each remaining piece with the boxes that overlap it (HaloBuckets): about 20 rectangles per
+// part for RCB output, O(neighbours) rather than O(ghost cells).  A rectangle is a copy of w x h 64-bit words from the
+// source's interior into the receiver's frame, which never overlap, so the items need no order among themselves.
+struct HaloRect {
+    long long src, dst; // first word: in the source part's tiles (this rank's buffer), in the receiver's (rank's buffer)
+    int src_stride, dst_stride; // row strides: the source's and the receiver's tile widths
+    int w, h; // columns, rows; w * h < 2^31
+    int rank; // the receiver's rank (one buffer: 0)
+    int pad;
+};
+// The items, in four groups: [interior corners][interior edges][periodic edges][periodic corners], so that every
+// exchange is one contiguous range (HaloPlan::rects): edge = [1], full = [0, 1], periodic edge = [1, 2], periodic full
+// = [0, 3].
+struct HaloRects {
+    const HaloRect* r;
+    int n;
+};
+
+// Every rectangle of the frames of width w (every part a receiver), tile-relative: src / dst are the words in the
+// source's and the receiver's tile; `part` / `source` the two parts, group as in HaloRects.  Host code, part of
+// halo_plan.
+struct HaloPiece {
+    HaloRect r;
+    int part, source, group;
+};
+inline void halo_pieces(int P, int nx, int ny, int px, int py, int w, const HaloBuckets& bk, std::vector<HaloPiece>& out)
+{
+    const int *x0 = bk.x0, *y0 = bk.y0, *ex = bk.ex, *ey = bk.ey;
+    const auto fdiv = [](long long a, long long n) { return a >= 0 ? a / n : -((-a + n - 1) / n); };
+    out.reserve((size_t)12 * P); // about 20 per part for RCB output, 8 on a regular grid: few regrowths
+    for (int p = 0; p < P; p++) {
+        const long long ax = x0[p], ay = y0[p], bx = ax + std::max(ex[p], 0), by = ay + std::max(ey[p], 0);
+        const long long xs[4] = { ax - w, ax, bx, bx + w }, ys[4] = { ay - w, ay, by, by + w };
+        const long long tw = bx - ax + 2LL * w;
+        for (int r = 0; r < 9; r++) {
+            const int cx = r % 3, cy = r / 3; // 0: before the box, 1: along it, 2: after it
+            if (cx == 1 && cy == 1)
+                continue; // the interior
+            const bool corner = cx != 1 && cy != 1;
+            for (long long ya = ys[cy]; ya < ys[cy + 1];) { // the wrapped pieces in y ...
+                const long long ky = fdiv(ya, ny), yb = std::min(ys[cy + 1], (ky + 1) * ny);
+                for (long long xa = xs[cx]; xa < xs[cx + 1];) { // ... and in x
+                    const long long kx = fdiv(xa, nx), xb = std::min(xs[cx + 1], (kx + 1) * nx);
+                    if ((kx == 0 || px) && (ky == 0 || py)) {
+                        const bool wrapped = kx != 0 || ky != 0;
+                        const int group = wrapped ? (corner ? 3 : 2) : (corner ? 0 : 1);
+                        bk.overlapping((int)(xa - kx * nx), (int)(xb - kx * nx), (int)(ya - ky * ny), (int)(yb - ky * ny),
+                            [&](int q, int ia, int ib, int ja, int jb) {
+                                const long long sw = ex[q] + 2LL * w;
+                                const int rows = std::max(1, INT_MAX / (ib - ia)); // w * h < 2^31 per item
+                                for (long long j = ja; j < jb; j += rows) {
+                                    HaloPiece pc {};
+                                    pc.r.src = (j - y0[q] + (long long)w) * sw + (ia - x0[q] + w);
+                                    pc.r.dst = (j + ky * ny - ay + w) * tw + (ia + kx * nx - ax + w);
+                                    pc.r.src_stride = (int)sw;
+                                    pc.r.dst_stride = (int)tw;
+                                    pc.r.w = ib - ia;
+                                    pc.r.h = (int)std::min((long long)rows, (long long)jb - j);
+                                    pc.part = p;
+                                    pc.source = q;
+                                    pc.group = group;
+                                    out.push_back(pc);
+                                }
+                            });
+                    }
+                    xa = xb;
+                }
+                ya = yb;
+            }
+        }
+    }
+}
+
+// The items of view G / rank (G = 1: one buffer, every item) from the pieces: those whose SOURCE part `rank` owns,
+// rebased to the buffers; at[5]: the group boundaries.  off: the ddc_halo_tile_offsets offsets.
+inline int halo_rect_items(int P, int G, int rank, const std::vector<HaloPiece>& pieces, const long long* off,
+    HaloRect* out, int* at)
+{
+    const auto owner = [&](int p) { return (int)(((long long)(p + 1) * G - 1) / P); };
+    const auto base = [&](int p) { return off[p] - off[(long long)owner(p) * P / G]; };
+    int n = 0;
+    for (int g = 0; g < 4; g++) {
+        at[g] = n;
+        for (const HaloPiece& pc : pieces)
+            if (pc.group == g && owner(pc.source) == rank) {
+                out[n] = pc.r;
+                out[n].src += base(pc.source);
+                out[n].dst += base(pc.part);
+                out[n].rank = owner(pc.part);
+                n++;
+            }
+    }
+    at[4] = n;
+    return n;
+}
+
+// one rectangle, by one warp: the lanes spread over its w x h cells (a left or right strip row is only w cells),
+// every load of a round issued before its stores, as halo_copy_row does; 32-bit index arithmetic (DESIGN.md 7)
+constexpr int HALO_RECT_LOADS = 4;
+__device__ __forceinline__ void halo_copy_rect(const HaloRect& it, const unsigned long long* __restrict__ src,
+    unsigned long long* __restrict__ dst, int lane)
+{
+    const unsigned w = (unsigned)it.w, n = w * (unsigned)it.h;
+    src += it.src;
+    dst += it.dst;
+    for (unsigned c0 = lane; c0 < n; c0 += 32 * HALO_RECT_LOADS) {
+        unsigned long long v[HALO_RECT_LOADS];
+        unsigned row[HALO_RECT_LOADS], col[HALO_RECT_LOADS];
+#pragma unroll
+        for (int u = 0; u < HALO_RECT_LOADS; u++) {
+            const unsigned c = c0 + 32u * u;
+            row[u] = c / w;
+            col[u] = c - row[u] * w;
+            if (c < n)
+                v[u] = src[(size_t)row[u] * it.src_stride + col[u]];
+        }
+#pragma unroll
+        for (int u = 0; u < HALO_RECT_LOADS; u++)
+            if (c0 + 32u * u < n)
+                dst[(size_t)row[u] * it.dst_stride + col[u]] = v[u];
+    }
+}
+
+// the wide-frame exchanges of one buffer (ddc_halo_exchange_f64 / _full_f64 at w >= 2): a warp per item, grid-stride
+__global__ void __launch_bounds__(256) k_halo_rects(HaloRects rects, double* tiles)
+{
+    unsigned long long* t = reinterpret_cast<unsigned long long*>(tiles);
+    const int lane = lane_id(), warps = gridDim.x * (blockDim.x >> 5);
+    for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < rects.n; i += warps)
+        halo_copy_rect(rects.r[i], t, t, lane);
+}
+
+// the middle kernel of the sharded wide-frame exchanges, between k_halo_open and k_halo_close: the items whose source
+// part this rank owns, local loads and posted stores into the receiver's tile wherever it lives (as k_halo_push)
+__global__ void __launch_bounds__(256) k_halo_push_rects(HaloShards hs, HaloRects rects)
+{
+    if (*(volatile unsigned*)hs.opened != hs.ps.step)
+        return; // (grid-uniform) k_halo_open timed out: nothing touched, no flag
+    const unsigned long long* local = reinterpret_cast<const unsigned long long*>(hs.tiles[hs.ps.rank]);
+    const int lane = lane_id(), warps = gridDim.x * (blockDim.x >> 5);
+    for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < rects.n; i += warps) {
+        const HaloRect& it = rects.r[i];
+        halo_copy_rect(it, local, reinterpret_cast<unsigned long long*>(hs.tiles[it.rank]), lane);
+    }
+    halo_block_done(hs);
+}
+
+// ------------------------------------------------------------------------------------------------
 // The halo plan: every table the host builds for the halo calls of one decomposition
 // ------------------------------------------------------------------------------------------------
 // Host code, shared by ddc_api.cu and the emulation harness of the tests; nothing else builds these tables.  View s of
 // the items and corners is 0: one buffer (every field row, every corner item), 1: this rank's shards (its
 // ddc_shard_rows block, the corner items whose source part it owns).  The tables the kernels read are one block of
-// memory, uploaded with one copy; off() / items() / corners() read them from a copy of the block at `at` (the device's,
-// or the block itself on the host).
+// memory, uploaded with one copy; off() / items() / corners() / rects() read them from a copy of the block at `at` (the
+// device's, or the block itself on the host).  w: the frame width; the corner items serve w = 1 only, the rectangle
+// items w >= 2 only (none are built at w = 1).
 struct HaloPlan {
-    int P = 0;
+    int P = 0, w = 1;
     std::vector<unsigned char> block;
     std::vector<int> corner_ids, corner_starts; // [2][4][P] (halo_corner_sources): ddc_get_corner_neighbours
     int items_n[2] = {}, items_total[2] = {};
     int corner_n[2][2] = {}; // [view][0: interior set, 1: both sets]
+    int rect_at[2][5] = {}; // [view]: the group boundaries of the rectangle items (HaloRects)
     long long shard_max = 0; // the largest rank's tile total: what every rank's halo buffer must hold
 
     // the layout of the block: 64-bit [off: P + 1][item base: 2][P][corner src, dst: 2][2][4 P], then 32-bit
-    // [items: 2][4 P + 1][corner destination rank: 2][4 P]
+    // [items: 2][4 P + 1][corner destination rank: 2][4 P] (bytes(P), a multiple of 8), then the rectangle items of
+    // view 0 and of view 1
     struct Ptrs {
         long long *off, *base[2], *corner[2];
         int *items[2], *rank[2];
@@ -3003,41 +3197,56 @@ struct HaloPlan {
     {
         const Ptrs a = ptrs(at);
         const int* t = a.items[s];
-        return HaloItems { t, t + P, t + 2 * P, t + 3 * P, a.base[s], items_n[s] };
+        return HaloItems { t, t + P, t + 2 * P, t + 3 * P, a.base[s], items_n[s], w };
     }
     HaloCorners corners(void* at, int s, int periodic) const // periodic: both sets, else the interior set
     {
         const Ptrs a = ptrs(at);
         return HaloCorners { a.corner[s], a.corner[s] + 4 * (size_t)P, s ? a.rank[s] : nullptr, corner_n[s][periodic ? 1 : 0] };
     }
+    HaloRects rects(void* at, int s, int periodic, bool full) const // the groups of one exchange (HaloRects)
+    {
+        const HaloRect* r = reinterpret_cast<const HaloRect*>(static_cast<unsigned char*>(at) + bytes(P)) + (s ? rect_at[0][4] : 0);
+        const int b = full ? 0 : 1, e = periodic ? (full ? 4 : 3) : 2;
+        return HaloRects { r + rect_at[s][b], rect_at[s][e] - rect_at[s][b] };
+    }
 };
 
 // The plan of boxes x0 / y0 / ex / ey [P] on a domain nx x ny (periodic px / py), for rank `rank` of G, whose
-// ddc_shard_rows block is rows y_begin ... y_begin + y_count - 1.
+// ddc_shard_rows block is rows y_begin ... y_begin + y_count - 1, with frames of width w (the default: one cell).
 inline HaloPlan halo_plan(int P, int G, int rank, int nx, int ny, int px, int py, const int* x0, const int* y0,
-    const int* ex, const int* ey, int y_begin, int y_count)
+    const int* ex, const int* ey, int y_begin, int y_count, int w = 1)
 {
     HaloPlan hp;
     hp.P = P;
-    hp.block.assign(HaloPlan::bytes(P), 0);
+    hp.w = w;
+    const HaloBuckets bk(P, nx, ny, x0, y0, ex, ey);
+    std::vector<HaloPiece> pieces;
+    if (w > 1)
+        halo_pieces(P, nx, ny, px, py, w, bk, pieces);
+    hp.block.assign(HaloPlan::bytes(P) + 2 * pieces.size() * sizeof(HaloRect), 0);
     const HaloPlan::Ptrs a = hp.ptrs(hp.block.data());
     long long run = 0;
     for (int p = 0; p < P; p++) {
         a.off[p] = run;
-        run += (long long)(std::max(ex[p], 0) + 2) * (std::max(ey[p], 0) + 2);
+        run += (std::max(ex[p], 0) + 2LL * w) * (std::max(ey[p], 0) + 2LL * w);
     }
     a.off[P] = run;
     for (int r = 0; r < G; r++) // every rank's total from the replicated boxes: the sharded calls refuse on every rank alike
         hp.shard_max = std::max(hp.shard_max, a.off[(long long)(r + 1) * P / G] - a.off[(long long)r * P / G]);
     hp.corner_ids.resize((size_t)8 * P);
     hp.corner_starts.resize((size_t)8 * P);
-    halo_corner_sources(P, nx, ny, px, py, x0, y0, ex, ey, hp.corner_ids.data(), hp.corner_starts.data());
+    halo_corner_sources(P, nx, ny, px, py, bk, hp.corner_ids.data(), hp.corner_starts.data());
+    HaloRect* rects = reinterpret_cast<HaloRect*>(hp.block.data() + HaloPlan::bytes(P));
     for (int s = 0; s < 2; s++) {
         hp.items_n[s] = halo_item_ranges(P, s ? G : 1, y0, ex, ey, a.off, s ? y_begin : 0, s ? y_begin + y_count : ny,
             a.items[s], a.base[s]);
         hp.items_total[s] = a.items[s][3 * P + hp.items_n[s]];
-        halo_corner_items(P, s ? G : 1, s ? rank : 0, hp.corner_ids.data(), hp.corner_starts.data(), ex, ey, a.off,
-            a.corner[s], a.corner[s] + 4 * (size_t)P, a.rank[s], hp.corner_n[s]);
+        if (w == 1)
+            halo_corner_items(P, s ? G : 1, s ? rank : 0, hp.corner_ids.data(), hp.corner_starts.data(), ex, ey, a.off,
+                a.corner[s], a.corner[s] + 4 * (size_t)P, a.rank[s], hp.corner_n[s]);
+        else
+            rects += halo_rect_items(P, s ? G : 1, s ? rank : 0, pieces, a.off, rects, hp.rect_at[s]);
     }
     return hp;
 }

@@ -281,6 +281,38 @@ DDC_API int ddc_get_corner_neighbours(ddc_handle_t h, int corner, int periodic, 
 DDC_API int ddc_halo_exchange_full_f64(ddc_handle_t h, double* tiles_dev, int periodic);
 DDC_API int ddc_halo_exchange_full_shards_f64(ddc_handle_t h, int periodic);
 
+/* Wide halos: ghost frames of width w for stencils that reach further than one cell (biharmonic operators, high-order
+   advection, or k sweeps of a 5- or 9-point stencil per exchange with w = k).  ddc_halo_set_width sets the w that every
+   halo call of the handle uses; the default is 1, which is exactly the layout and behaviour described above.  It may be
+   called before ddc_partition.  A w that differs from the current one drops the tile and shard offsets, as a new
+   decomposition does: every halo call returns DDC_ERR_STATE until ddc_halo_tile_offsets / ddc_halo_shard_offsets are
+   called again.  w < 1 or w > DDC_MAX_HALO_WIDTH is DDC_ERR_ARG.  The bound keeps a corner block (w * w cells) and
+   x0 - w, x0 + ext + w of every box whose extents stay below INT_MAX - 2 DDC_MAX_HALO_WIDTH within the 32-bit ints of
+   the kernels' index arithmetic.
+   With width w:
+     - Layout: tile p is a row-major (ext_y + 2 w) x (ext_x + 2 w) array; interior cell (i, j) is at row j + w, column
+       i + w.  ddc_halo_tile_offsets and ddc_halo_shard_offsets return these sizes; the sharded buffers remain the
+       single-buffer layout restricted to the rank's parts.  Scatter and gather read and write the interiors only, at
+       that position, bit for bit.
+     - Source rule: a frame cell of p lies outside p's box at (x, y), x0 - w <= x < x0 + ext_x + w and the same in y.
+       Its source is the positive-area box that contains the cell -- the cell itself when it lies in [0, nx) x [0, ny)
+       (interior), else the wrapped cell (x mod nx, y mod ny) when the decomposition is periodic in every direction in
+       which the cell lies outside (periodic).  A frame wider than the domain wraps as often as it needs.  This is the
+       corner rule above applied to every frame cell; on a tiling at w = 1 it selects exactly the ghosts the edge lists
+       fill.
+     - ddc_halo_exchange_f64 / ddc_halo_exchange_shards_f64 fill every cell of the four w-deep edge strips that has a
+       source (interior; periodic != 0: periodic too); the _full_ calls also fill the four w x w corner blocks.  Cells
+       with no source keep what they held.  When the boxes tile the domain, which ddc_partition's always do, every
+       filled cell holds its wrapped cell, zero-width and zero-height parts included; overlapping caller boxes stay
+       outside the rule as above.  Without neighbour tables the exchanges still do nothing; the status codes and the
+       shared step counter of the sharded calls are unchanged; ddc_get_corner_neighbours still describes the diagonal
+       cell, whatever w.
+     - Sharded: every rank must set the same w.  A mismatch cannot make a kernel write past a buffer -- each rank
+       checks every rank's tile total at its own w against the common elems, and its items address only tiles of
+       that size -- but its ghosts are wrong. */
+#define DDC_MAX_HALO_WIDTH 1024
+DDC_API int ddc_halo_set_width(ddc_handle_t h, int width);
+
 /* ---- synthetic masks (SURVEY 8d): deterministic value-noise land-sea mask, generated directly
    into device memory so that no 4 GiB file is needed for the large configurations.
    land_frac in [0,1] is the target land fraction; rows as in ddc_set_mask_device. */

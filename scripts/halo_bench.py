@@ -4,6 +4,7 @@
 
     python scripts/halo_bench.py --out result.json                   # one GPU
     torchrun --nproc-per-node G scripts/halo_bench.py --out r.json    # G GPUs, one process each
+    python scripts/halo_bench.py --widths 1 2 4 --out result.json    # frames of width 1, 2 and 4 (ddc_halo_set_width)
 
 One GPU: ddc_halo_exchange_f64 on one buffer against ddc_halo_exchange_shards_f64 with one rank (the same ghost
 cells, plus the open / close barriers of the sharded protocol), the full-frame exchanges (ddc_halo_exchange_full_f64 /
@@ -16,7 +17,11 @@ cells moved come from the neighbour tables: a cell is read once (8 B) and writte
 written into another rank's buffer.  Scatter and gather move every cell of the field (nx ny cells, 8 B read + 8 B
 written each); their "cross-rank" cells are those whose row (ddc_shard_rows) and part (ddc_shard_parts) belong to
 different ranks.  Rates are compared with the 6546.9 GB/s of a read+write copy measured on a B200 (DESIGN.md 4).  The
-GPU name and power limit are read in the same run.  Writes JSON to --out (and prints it); nothing in the tree."""
+GPU name and power limit are read in the same run.  --widths: every call and the host time of ddc_halo_tile_offsets
+are measured at each frame width (default 1), every row says its width; one halo buffer, sized for the widest frame,
+serves all widths.  Ghost cells at w >= 2 are counted from the boxes by the source rule of ddc.h (the decompositions
+tile the domain, so a frame cell has a source unless it lies across a non-periodic edge), cross-rank ones only with one
+rank (0).  Writes JSON to --out (and prints it); nothing in the tree."""
 import argparse
 import json
 import os
@@ -74,6 +79,16 @@ def corner_counts(h, P, G, periodic):
             total += int(has.sum())
             cross += int((owner(ids[has].astype(np.int64)) != owner(np.nonzero(has)[0])).sum())
     return total, cross
+
+
+def wide_counts(boxes, nx, ny, px, py, w):
+    """(edge-strip ghosts, corner-block ghosts) one periodic exchange of width w fills: a frame cell of a tiling has a
+    source unless it lies across a non-periodic domain edge"""
+    b = np.asarray(boxes, dtype=np.int64)
+    x0, y0, ex, ey = b[:, 0], b[:, 1], np.maximum(b[:, 2], 0), np.maximum(b[:, 3], 0)
+    cx = np.where(px, w, np.minimum(w, x0)) + np.where(px, w, np.minimum(w, nx - x0 - ex))  # columns left + right
+    cy = np.where(py, w, np.minimum(w, y0)) + np.where(py, w, np.minimum(w, ny - y0 - ey))  # rows below + above
+    return int((cx * ey + cy * ex).sum()), int((cx * cy).sum())
 
 
 def host_ms(fn, reps=5):
@@ -140,6 +155,15 @@ def row(name, cfg, G, ms, cells, cross, corners=(0, 0)):
                 achieved_GBps=round(bytes_moved / (ms * 1e-3) / 1e9, 1))
 
 
+def exchange_counts(h, cfg, w):
+    """(ghost cells, cross-rank, (corner cells, cross-rank)) of one periodic exchange at width w, one rank"""
+    P = cfg["parts"]
+    if w == 1:
+        return ghost_counts(h, P, 1, True) + (corner_counts(h, P, 1, True),)
+    edge, corner = wide_counts(h.boxes(), cfg["nx"], cfg["ny"], cfg["px"], cfg["py"], w)
+    return edge, 0, (corner, 0)
+
+
 def one_gpu(args):
     dev = torch.device("cuda", 0)
     stream = torch.cuda.Stream(dev)  # (a stream of its own: 0 would hand the handle back its internal stream)
@@ -151,42 +175,47 @@ def one_gpu(args):
         d_mask = decompose(h, dev, cfg, 1, 0)
         del d_mask
         P = cfg["parts"]
-        off = h.halo_tile_offsets()
-        host = dict(config=name, parts=P, tile_offsets_host_ms=host_ms(h.halo_tile_offsets),
-                    corner_table_host_ms=host_ms(lambda: h.corner_neighbours(0, 1)))
-        print(json.dumps(host), flush=True)
-        single = torch.zeros(int(off[-1]), dtype=torch.float64, device=dev)
-        (ptr,) = capi.halo_connect([h], int(off[-1]))
-        h.halo_shard_offsets()
-        cells, cross = ghost_counts(h, P, 1, True)
-        corners = corner_counts(h, P, 1, True)
+        h.halo_set_width(max(args.widths))
+        elems = int(h.halo_tile_offsets()[-1])
+        single = torch.zeros(elems, dtype=torch.float64, device=dev)
+        (ptr,) = capi.halo_connect([h], elems)
         fcells, fcross = field_counts(h.boxes(), cfg["ny"], P, 1)
         field = torch.zeros((cfg["ny"], cfg["nx"]), dtype=torch.float64, device=dev)
         back = torch.zeros_like(field)
-        variants = {"single_buffer": lambda: h.halo_exchange_f64(single.data_ptr(), True),
-                    "sharded_G1": lambda: h.halo_exchange_shards_f64(True),
-                    "full_single_buffer": lambda: h.halo_exchange_full_f64(single.data_ptr(), True),
-                    "full_sharded_G1": lambda: h.halo_exchange_full_shards_f64(True),
-                    "scatter_single_buffer": lambda: h.halo_scatter_f64(field.data_ptr(), single.data_ptr()),
-                    "gather_single_buffer": lambda: h.halo_gather_f64(single.data_ptr(), back.data_ptr()),
-                    "scatter_sharded_G1": lambda: h.halo_scatter_shards_f64(field.data_ptr()),
-                    "gather_sharded_G1": lambda: h.halo_gather_shards_f64(back.data_ptr())}
-        for fn in variants.values():
-            timed(fn, stream, args.warmup)
-        samples = {k: [] for k in variants}
-        for _ in range(args.rounds):  # alternated: the variants share whatever else the machine does
-            for k, fn in variants.items():
-                samples[k].append(timed(fn, stream, args.iters))
-        h.synchronize()
-        for k in variants:
-            ms = float(np.median(samples[k]))
-            r = row(name, cfg, 1, ms, cells, cross) if k in ("single_buffer", "sharded_G1") else \
-                row(name, cfg, 1, ms, cells, cross, corners) if k.startswith("full") else \
-                field_row(name, cfg, 1, k, ms, fcells, fcross)
-            r.update(variant=k, samples_ms=[round(s, 5) for s in samples[k]], iters=args.iters)
-            results.append(r)
-            print(json.dumps(r), flush=True)
-        results.append(host)
+        for w in args.widths:
+            h.halo_set_width(w)
+            h.halo_tile_offsets()
+            host = dict(config=name, parts=P, width=w, tile_offsets_host_ms=host_ms(h.halo_tile_offsets),
+                        corner_table_host_ms=host_ms(lambda: h.corner_neighbours(0, 1)))
+            print(json.dumps(host), flush=True)
+            h.halo_shard_offsets()
+            cells, cross, corners = exchange_counts(h, cfg, w)
+            variants = {"single_buffer": lambda: h.halo_exchange_f64(single.data_ptr(), True),
+                        "sharded_G1": lambda: h.halo_exchange_shards_f64(True),
+                        "full_single_buffer": lambda: h.halo_exchange_full_f64(single.data_ptr(), True),
+                        "full_sharded_G1": lambda: h.halo_exchange_full_shards_f64(True),
+                        "scatter_single_buffer": lambda: h.halo_scatter_f64(field.data_ptr(), single.data_ptr()),
+                        "gather_single_buffer": lambda: h.halo_gather_f64(single.data_ptr(), back.data_ptr()),
+                        "scatter_sharded_G1": lambda: h.halo_scatter_shards_f64(field.data_ptr()),
+                        "gather_sharded_G1": lambda: h.halo_gather_shards_f64(back.data_ptr())}
+            for fn in variants.values():
+                timed(fn, stream, args.warmup)
+            samples = {k: [] for k in variants}
+            for _ in range(args.rounds):  # alternated: the variants share whatever else the machine does
+                for k, fn in variants.items():
+                    samples[k].append(timed(fn, stream, args.iters))
+            h.synchronize()
+            for k in variants:
+                ms = float(np.median(samples[k]))
+                r = row(name, cfg, 1, ms, cells, cross) if k in ("single_buffer", "sharded_G1") else \
+                    row(name, cfg, 1, ms, cells, cross, corners) if k.startswith("full") else \
+                    field_row(name, cfg, 1, k, ms, fcells, fcross)
+                if k.startswith(("single", "sharded", "full")):
+                    r["share_of_copy_rate"] = round(r["achieved_GBps"] / COPY_GBPS, 4)
+                r.update(variant=k, width=w, samples_ms=[round(s, 5) for s in samples[k]], iters=args.iters)
+                results.append(r)
+                print(json.dumps(r), flush=True)
+            results.append(host)
         h.halo_close()
         h.close()
         del single, field, back
@@ -263,8 +292,11 @@ def main():
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--rounds", type=int, default=5)
+    ap.add_argument("--widths", nargs="+", type=int, default=[1], help="frame widths (ddc_halo_set_width); one GPU only")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
+    if "WORLD_SIZE" in os.environ and args.widths != [1]:
+        sys.exit("halo_bench: --widths is measured on one GPU only (the cross-rank ghosts of wide frames are not counted)")
     if not torch.cuda.is_available():
         sys.exit("halo_bench: no CUDA device (there is nothing to measure without one)")
     t0 = time.time()

@@ -90,9 +90,12 @@ _emu = None
 
 
 def emu_partition(mask: np.ndarray, P: int, px: bool = False, py: bool = False, *, ranks: int = 1, strip_k: int = 0,
-                  scan_rpc: int = 0, smem_limit: int = 0):
+                  scan_rpc: int = 0, smem_limit: int = 0, nbr_cap: int | None = None):
     """One decomposition through the product's REAL kernels on the host emulation of the CUDA execution model
-    (oracle/emu/), on `ranks` emulated row-sharded ranks.  Returns (Decomposition, info dict)."""
+    (oracle/emu/), on `ranks` emulated row-sharded ranks.  Returns (Decomposition, info dict).
+    nbr_cap: entries reserved for the eight neighbour lists together (ids, halos and starts each); by default enough
+    for every part to list every other one, 16 P^2, which is gigabytes beyond a few thousand parts.  A capacity below
+    the lists' total is an error."""
     global _emu
     if _emu is None:
         build()
@@ -108,7 +111,7 @@ def emu_partition(mask: np.ndarray, P: int, px: bool = False, py: bool = False, 
     boxes = np.zeros((P, 4), dtype=np.int32)
     pid = np.zeros((ny, nx), dtype=np.int32)
     counts = np.zeros(8 * P, dtype=np.int32)
-    cap = 8 * (3 * P + 64) + 16 * P * P  # every part can list every other one
+    cap = 8 * (3 * P + 64) + 16 * P * P if nbr_cap is None else int(nbr_cap)
     flat = np.zeros(3 * cap, dtype=np.int32)
     out = np.zeros(8, dtype=np.int64)
     rc = _emu.emu_partition(mask, nx, ny, P, int(px), int(py), ranks, strip_k, scan_rpc, smem_limit, boxes, pid, counts, flat,

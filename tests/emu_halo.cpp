@@ -1,14 +1,16 @@
 // emu_halo.cpp -- TEST INFRASTRUCTURE.  The halo calls (scatter, edge exchange, full-frame exchange and gather, on
-// one buffer and sharded) through the product's REAL kernels and host code (halo_plan and halo_shards;
-// k_halo_exchange + k_halo_corners and k_halo_field on one buffer, k_halo_push / k_halo_push_full / k_halo_field_shards
-// between k_halo_open and k_halo_close on the shards; ddc_kernels.cuh compiled with -DDDC_HOST_EMU) on the host
-// emulation of the CUDA execution model, for G emulated ranks on one halo step counter.  The buffers and launches
-// follow ddc_api.cu: each rank's buffer is [HALO_HEAD_BYTES head][tiles of its parts], the kernels receive every
-// rank's buffer as "mapped" and push into them.  The ranks run phase by phase (all signal R, all wait for R, all run
-// the middle kernel, all wait for D), as oracle/emu/emu_pipeline.cpp runs the decomposition's kernels.  Beside them the
-// single-buffer kernels run on one buffer holding all parts and one whole field.  Every rank's rows live in an
-// allocation of their own with a guard band on either side, so a store outside the rank's block is seen.  It says
-// nothing about speed.  Compiled by tests/halo_emu.py (into a temporary directory) against oracle/emu/cuda_emu.cpp.
+// one buffer and sharded) with frames of width w (ddc_halo_set_width), through the product's REAL kernels and host code
+// (halo_plan with the width and halo_shards; at w = 1 k_halo_exchange + k_halo_corners on one buffer and k_halo_push /
+// k_halo_push_full between k_halo_open and k_halo_close on the shards, at w >= 2 k_halo_rects and k_halo_push_rects;
+// k_halo_field / k_halo_field_shards at the width; ddc_kernels.cuh compiled with -DDDC_HOST_EMU) on the host emulation
+// of the CUDA execution model, for G emulated ranks on one halo step counter.  The buffers and launches follow
+// ddc_api.cu: each rank's buffer is [HALO_HEAD_BYTES head][tiles of its parts], every tile sized for the width, and the
+// kernels receive every rank's buffer as "mapped" and push into them.  The ranks run phase by phase (all signal R, all
+// wait for R, all run the middle kernel, all wait for D), as oracle/emu/emu_pipeline.cpp runs the decomposition's
+// kernels.  Beside them the single-buffer kernels run on one buffer holding all parts and one whole field.  Every rank's
+// rows live in an allocation of their own with a guard band on either side, so a store outside the rank's block is
+// seen.  It says nothing about speed.  Compiled by tests/halo_emu.py (into a temporary directory) against
+// oracle/emu/cuda_emu.cpp.
 #include "cuda_emu.h"
 #include "ddc_kernels.cuh"
 
@@ -43,7 +45,8 @@ __attribute__((visibility("default"))) const char* emu_halo_last_error(void) { r
 // run in order on the sharded buffers AND on the single buffer, with one halo step counter.
 // grid_cap: 0 the library's grids, else at most that many blocks for the grid-stride kernels (few blocks: the loops
 // and the block counter see several rounds and blocks).
-// corner_ids / corner_starts [2][4][P]: the plan's corner table (ddc_get_corner_neighbours).
+// corner_ids / corner_starts [2][4][P]: the plan's corner table (ddc_get_corner_neighbours).  w: the frame width
+// (ddc_halo_set_width); at w >= 2 the exchanges run k_halo_rects / k_halo_push_rects, as ddc_api.cu does.
 // fields[k][ny * nx]: what each rank's rows hold for the k-th scatter (rank r: rows rows_b[r] ...), and what the
 // single-buffer scatter reads.  tiles_in[total]: the tiles before the first op (every buffer); rows_in[ny * nx]: the
 // rows (and the single-buffer field) a gather writes into before the first op.  After op i: tiles_out[i] = the ranks'
@@ -54,14 +57,14 @@ __attribute__((visibility("default"))) int emu_halo(int P, const int32_t* boxes,
     const int32_t* ids, const int32_t* halos, const int32_t* starts, int nx, int ny, int px, int py, int G,
     const int32_t* rows_b, const int32_t* rows_c, int periodic, const char* ops, int stall, int grid_cap,
     const double* fields, const double* tiles_in, const double* rows_in, double* tiles_out, double* single_out,
-    double* rows_out, double* field_out, int32_t* err_out, int32_t* corner_ids, int32_t* corner_starts)
+    double* rows_out, double* field_out, int32_t* err_out, int32_t* corner_ids, int32_t* corner_starts, int w)
 {
     g_err.clear();
     if (const char* e = std::getenv("DDC_EMU_SCHED_SEED"))
         cuda_emu::set_schedule_seed(std::strtoull(e, nullptr, 10));
     else
         cuda_emu::set_schedule_seed(0);
-    if (P < 1 || G < 1 || G > MAX_PEERS || nx < 1 || ny < 1) {
+    if (P < 1 || G < 1 || G > MAX_PEERS || nx < 1 || ny < 1 || w < 1) {
         g_err = "bad arguments";
         return -1;
     }
@@ -93,7 +96,7 @@ __attribute__((visibility("default"))) int emu_halo(int P, const int32_t* boxes,
     // every rank's halo plan, as ddc_api.cu's tile_offsets() builds it; the single buffer uses view 0 of rank 0's
     std::vector<HaloPlan> plan(G);
     for (int r = 0; r < G; r++)
-        plan[r] = halo_plan(P, G, r, nx, ny, px, py, bx.x0, bx.y0, bx.ex, bx.ey, rows_b[r], rows_c[r]);
+        plan[r] = halo_plan(P, G, r, nx, ny, px, py, bx.x0, bx.y0, bx.ex, bx.ey, rows_b[r], rows_c[r], w);
     std::memcpy(corner_ids, plan[0].corner_ids.data(), sizeof(int32_t) * 8 * P);
     std::memcpy(corner_starts, plan[0].corner_starts.data(), sizeof(int32_t) * 8 * P);
     const long long* off = plan[0].off();
@@ -156,7 +159,10 @@ __attribute__((visibility("default"))) int emu_halo(int P, const int32_t* boxes,
                 void* at = plan[r].block.data();
                 const HaloItems items = plan[r].items(at, 1);
                 const HaloCorners corners = plan[r].corners(at, 1, periodic);
-                if (op == 'x')
+                const HaloRects rects = plan[r].rects(at, 1, periodic, op == 'f');
+                if (exchange && w > 1)
+                    LAUNCH(grid(halo_field_grid(rects.n)), Dim3(256), k_halo_push_rects(hs[r], rects));
+                else if (op == 'x')
                     LAUNCH(grid(halo_push_grid(pc[r], 0)), Dim3(256),
                         k_halo_push(hs[r], bx, cnt.data(), offs.data(), cap, vid.data(), vh.data(), vs.data(), off, lists));
                 else if (op == 'f')
@@ -174,7 +180,11 @@ __attribute__((visibility("default"))) int emu_halo(int P, const int32_t* boxes,
                 if (r != stall)
                     LAUNCH(Dim3(1), Dim3(32), k_halo_close(hs[r]));
         }
-        if (exchange && have_nbr) {
+        if (exchange && have_nbr && w > 1) {
+            const HaloRects rects = plan[0].rects(single_plan, 0, periodic, op == 'f');
+            if (rects.n > 0)
+                LAUNCH(grid(halo_field_grid(rects.n)), Dim3(256), k_halo_rects(rects, single.data()));
+        } else if (exchange && have_nbr) {
             LAUNCH(Dim3(halo_exchange_grid(P)), Dim3(256), // (not grid-stride: never capped)
                 k_halo_exchange<double>(bx, P, cnt.data(), offs.data(), cap, vid.data(), vh.data(), vs.data(), off,
                     single.data(), lists));

@@ -52,19 +52,20 @@ def lib(sanitize=False) -> C.CDLL:
         f64p = np.ctypeslib.ndpointer(np.float64, flags="C_CONTIGUOUS")
         L.emu_halo.argtypes = [C.c_int, i32p, i32p, i32p, i32p, i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                i32p, i32p, C.c_int, C.c_char_p, C.c_int, C.c_int, f64p, f64p, f64p, f64p, f64p, f64p, f64p,
-                               i32p, i32p, i32p]
+                               i32p, i32p, i32p, C.c_int]
         L.emu_halo.restype = C.c_int
         L.emu_halo_last_error.restype = C.c_char_p
         _lib = L
     return _lib
 
 
-def run(boxes, nbr, nx, ny, px, py, G, periodic, ops, tiles_in, fields=(), rows_in=None, stall=-1, grid_cap=4):
-    """run `ops` ('s' scatter, 'x' edge exchange, 'f' full-frame exchange, 'g' gather) on G emulated ranks and on one
-    buffer.  boxes / nbr: a decomposition (oracle.partition's boxes and nbr); tiles_in: the tiles before the first op;
-    fields: one field [ny, nx] per 's', in order (more are ignored); rows_in: what the rows hold before the first op
-    (zeros by default).  Arrays are passed as their 64-bit patterns.  stall: a rank that runs none of the kernels.
-    grid_cap: at most that many blocks for the grid-stride kernels, 0 the library's grids."""
+def run(boxes, nbr, nx, ny, px, py, G, periodic, ops, tiles_in, fields=(), rows_in=None, stall=-1, grid_cap=4, w=1):
+    """run `ops` ('s' scatter, 'x' edge exchange, 'f' full-frame exchange, 'g' gather) with frames of width w on G
+    emulated ranks and on one buffer.  boxes / nbr: a decomposition (oracle.partition's boxes and nbr); tiles_in: the
+    tiles before the first op, in the layout of width w; fields: one field [ny, nx] per 's', in order (more are ignored);
+    rows_in: what the rows hold before the first op (zeros by default).  Arrays are passed as their 64-bit patterns.
+    stall: a rank that runs none of the kernels.  grid_cap: at most that many blocks for the grid-stride kernels, 0 the
+    library's grids."""
     L = lib()
     boxes = np.ascontiguousarray(boxes, dtype=np.int32)
     P = len(boxes)
@@ -88,7 +89,7 @@ def run(boxes, nbr, nx, ny, px, py, G, periodic, ops, tiles_in, fields=(), rows_
     rc = L.emu_halo(P, boxes.reshape(-1), counts, cat(nbr.ids), cat(nbr.halos), cat(nbr.starts), nx, ny, int(px), int(py),
                     G, np.array([b for b, _ in rows], dtype=np.int32), np.array([c for _, c in rows], dtype=np.int32),
                     int(periodic), ops.encode(), stall, grid_cap, as_f64(fields), as_f64(tiles_in), as_f64(rows_in),
-                    tiles, single, out_rows, out_field, err, ids, starts)
+                    tiles, single, out_rows, out_field, err, ids, starts, int(w))
     if rc != 0:
         raise RuntimeError("emu_halo: " + L.emu_halo_last_error().decode())
     u = lambda a, m: a.view(np.uint64).reshape(n, m)

@@ -1,13 +1,13 @@
 """Wide halos (ddc_halo_set_width: ghost frames of width w for scatter, gather and both exchanges) on a machine without a
 GPU.
 
-1. The kernels on emulated ranks: tests/emu_halo_width.cpp (built by tests/halo_width_emu.py) runs the product's halo
-   plan with the width (the rectangle items) and kernels (k_halo_rects on one buffer, k_halo_push_rects between k_halo_open and
+1. The kernels on emulated ranks: tests/emu_halo.cpp (built by tests/halo_emu.py) runs the product's halo plan with the
+   width (the rectangle items) and kernels (k_halo_rects on one buffer, k_halo_push_rects between k_halo_open and
    k_halo_close on G ranks, mixed with k_halo_field and k_halo_field_shards at that width), under index-order and random
    schedules, against halo_width's expectation over the whole buffer, untouched cells included.
 2. The C ABI on oracle/libddc_cuda_emu.so: w = 1 is the default bit for bit, the width's status codes, and the sharded
    calls with one rank.
-3. The same kernels at w = 2 and 3 under AddressSanitizer + UBSan (tests/halo_width_asan_worker.py).
+3. The same kernels at w = 2 and 3 under AddressSanitizer + UBSan (tests/halo_asan_worker.py).
 Says nothing about speed."""
 import ctypes as C
 import os
@@ -18,9 +18,9 @@ import numpy as np
 import pytest
 
 import halo_emu
+import halo_frame as hf
 import halo_global as hg
 import halo_width as hw
-import halo_width_emu
 from conftest import ROOT
 from halo_frame import degenerate_cases
 from halo_global import SENTINEL, cases, random_bits
@@ -54,7 +54,7 @@ def test_exchanges_follow_the_rule(oracle, w):
         tiny += w > nx or w > ny
         for periodic in (0, 1):
             ctx = (w, seed, nx, ny, len(boxes), px, py, periodic)
-            run = halo_width_emu.run(boxes, nbr, nx, ny, px, py, 2, periodic, "xf", tiles_in, w=w)
+            run = halo_emu.run(boxes, nbr, nx, ny, px, py, 2, periodic, "xf", tiles_in, w=w)
             assert run.err.tolist() == [0, 0], ctx
             for i, full in enumerate((False, True)):
                 want = as_bits(hw.expected(boxes, off, nx, ny, px, py, periodic, full, w))
@@ -69,8 +69,8 @@ def test_wide_frames_wrap_several_times(oracle):
     nx, ny, w = 2, 3, 5
     d = oracle.partition(np.ones((ny, nx), dtype=np.int32), 2, True, True, use_hist=True)
     off = hw.tile_offsets(d.boxes, w)
-    run = halo_width_emu.run(d.boxes, d.nbr, nx, ny, True, True, 1, 1, "f",
-                             as_bits(hw.initial_tiles(d.boxes, off, nx, ny, w)), w=w)
+    run = halo_emu.run(d.boxes, d.nbr, nx, ny, True, True, 1, 1, "f", as_bits(hw.initial_tiles(d.boxes, off, nx, ny, w)),
+                       w=w)
     got = run.single[0].view(np.float64)
     assert not (got == hg.UNTOUCHED).any()
     idx, x, y, _ = hw.frame_cells(d.boxes, off, w)
@@ -92,8 +92,8 @@ def test_mixed_sequence_on_one_step_counter(oracle, monkeypatch, G, sched):
         field = random_bits(rng, nx * ny).reshape(ny, nx)
         tiles_in = np.full(int(off[-1]), SENTINEL, dtype=np.uint64)
         ops = "sxfxg"
-        run = halo_width_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, ops, tiles_in, [field],
-                                 random_bits(rng, nx * ny), w=w)
+        run = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, G, periodic, ops, tiles_in, [field], random_bits(rng, nx * ny),
+                           w=w)
         ctx = (G, sched, seed, w, nx, ny, d.P, periodic)
         assert run.err.tolist() == [0] * G, ctx
         want = hw.scattered(d.boxes, off, field, tiles_in, w)
@@ -107,16 +107,26 @@ def test_mixed_sequence_on_one_step_counter(oracle, monkeypatch, G, sched):
 
 
 def test_width_one_is_the_one_cell_frame(oracle):
-    """w = 1 through the width harness gives every buffer of the one-cell harness (tests/emu_halo.cpp, which builds
-    the plan without a width)"""
+    """w = 1 is the one-cell frame: scatter, edge exchange, full exchange and gather on one buffer and on two ranks give
+    the one-cell expectations of halo_global and halo_frame, built from the global field"""
     for d, nx, ny, px, py, seed in cases(oracle):
         rng = np.random.default_rng(seed)
         field = random_bits(rng, nx * ny).reshape(ny, nx)
-        tiles_in = np.full(int(hg.tile_offsets(d.boxes)[-1]), SENTINEL, dtype=np.uint64)
-        assert np.array_equal(hw.tile_offsets(d.boxes, 1), hg.tile_offsets(d.boxes))
-        a = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, 2, 1, "sxfg", tiles_in, [field])
-        b = halo_width_emu.run(d.boxes, d.nbr, nx, ny, px, py, 2, 1, "sxfg", tiles_in, [field], w=1)
-        assert all(np.array_equal(x, y) for x, y in zip(a, b)), seed
+        off = hg.tile_offsets(d.boxes)
+        tiles_in = np.full(int(off[-1]), SENTINEL, dtype=np.uint64)
+        assert np.array_equal(hw.tile_offsets(d.boxes, 1), off)
+        ops = "sxfg"
+        run = halo_emu.run(d.boxes, d.nbr, nx, ny, px, py, 2, 1, ops, tiles_in, [field], w=1)
+        assert run.err.tolist() == [0, 0], seed
+        want = hg.scattered(d.boxes, off, field, tiles_in)
+        for i, op in enumerate(ops):
+            if op in "xf":
+                want = hg.exchanged(d.boxes, off, nx, ny, px, py, 1, field, want)
+            if op == "f":
+                want = hf.with_corners(d.boxes, off, nx, ny, px, py, 1, field, want)
+            assert np.array_equal(run.single[i], want), (seed, i, "single buffer")
+            assert run.tiles[i].tobytes() == want.tobytes(), (seed, i, "sharded")
+        assert run.rows[-1].tobytes() == field.tobytes() and run.field[-1].tobytes() == field.tobytes(), seed
 
 
 # ---- 2. the C ABI on the emulated runtime ----------------------------------------------------------------------------
@@ -299,8 +309,8 @@ def test_wide_halo_kernels_are_clean_under_address_sanitizer(oracle):
         pytest.skip("libasan not available")
     env = dict(os.environ, LD_PRELOAD=asan, ASAN_OPTIONS="detect_leaks=0:detect_stack_use_after_return=0:halt_on_error=1",
                UBSAN_OPTIONS="halt_on_error=1:print_stacktrace=1")
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "halo_width_asan_worker.py")], capture_output=True,
-                         text=True, timeout=900, env=env)
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "halo_asan_worker.py"), "2", "3"],
+                         capture_output=True, text=True, timeout=900, env=env)
     assert "ERROR: AddressSanitizer" not in out.stderr and "runtime error:" not in out.stderr, out.stderr[-4000:]
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-4000:]
-    assert "HALO WIDTH ASAN RUN OK" in out.stdout
+    assert "HALO ASAN RUN OK" in out.stdout and "widths [2, 3]" in out.stdout

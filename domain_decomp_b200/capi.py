@@ -36,7 +36,7 @@ SYMBOLS = (
     "ddc_halo_exchange_shards_f64", "ddc_halo_close",
     "ddc_halo_scatter_f64", "ddc_halo_gather_f64", "ddc_halo_scatter_shards_f64", "ddc_halo_gather_shards_f64",
     "ddc_get_corner_neighbours", "ddc_halo_exchange_full_f64", "ddc_halo_exchange_full_shards_f64",
-    "ddc_halo_set_width",
+    "ddc_halo_set_width", "ddc_set_mask_u8_host", "ddc_set_mask_u8_device",
 )
 
 
@@ -88,6 +88,8 @@ def load() -> C.CDLL:
     L.ddc_peer_close.argtypes = [vp]
     L.ddc_set_mask_host.argtypes = [vp, vp, i32, i32, i32, i32]
     L.ddc_set_mask_device.argtypes = [vp, vp, i32, i32, i32, i32]
+    L.ddc_set_mask_u8_host.argtypes = [vp, vp, i32, i32, i32, i32]
+    L.ddc_set_mask_u8_device.argtypes = [vp, vp, i32, i32, i32, i32]
     L.ddc_shard_rows.argtypes = [i32, i32, i32, C.POINTER(i32), C.POINTER(i32)]
     L.ddc_shard_rows.restype = None
     L.ddc_partition.argtypes = [vp, i32, i32, i32, i32]
@@ -240,6 +242,21 @@ class Handle:
         y_count = ny if y_count is None else y_count
         self.shape = (ny, nx, y_begin, y_count)
         self._ck(self.L.ddc_set_mask_device(self.h, dev_ptr, nx, ny, y_begin, y_count), "ddc_set_mask_device")
+
+    def set_mask_u8_host(self, rows: np.ndarray, ny: int | None = None, y_begin: int = 0):
+        """rows: uint8 or bool [y_count, nx] host array (this rank's rows); a cell is ocean <=> its byte is non-zero."""
+        assert rows.dtype in (np.uint8, np.bool_) and rows.flags.c_contiguous and rows.ndim == 2
+        y_count, nx = rows.shape
+        ny = y_count if ny is None else ny
+        self._keep = rows
+        self.shape = (ny, nx, y_begin, y_count)
+        self._ck(self.L.ddc_set_mask_u8_host(self.h, rows.ctypes.data, nx, ny, y_begin, y_count), "ddc_set_mask_u8_host")
+
+    def set_mask_u8_device(self, dev_ptr: int, nx: int, ny: int, y_begin: int = 0, y_count: int | None = None):
+        """dev_ptr: one byte per cell (a torch.bool / torch.uint8 tensor's data_ptr()), rows of nx bytes."""
+        y_count = ny if y_count is None else y_count
+        self.shape = (ny, nx, y_begin, y_count)
+        self._ck(self.L.ddc_set_mask_u8_device(self.h, dev_ptr, nx, ny, y_begin, y_count), "ddc_set_mask_u8_device")
 
     def generate_mask_device(self, dev_ptr: int, nx: int, ny: int, seed: int, land_frac: float,
                              y_begin: int = 0, y_count: int | None = None):

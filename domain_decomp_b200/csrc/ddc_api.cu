@@ -172,9 +172,10 @@ struct ddc_handle_s {
 
     // input
     int nx = 0, ny = 0, y_begin = 0, y_count = 0;
-    const int32_t* d_mask = nullptr; // borrowed or == mask_own.p
+    const void* d_mask = nullptr; // borrowed or == mask_own.p
+    int mask_esize = 4; // bytes per mask cell: 4 int32 (ddc_set_mask_*), 1 uint8 (ddc_set_mask_u8_*)
     bool mask_set = false;
-    DevBuf<int32_t> mask_own;
+    DevBuf<uint8_t> mask_own;
 
     // state of the last partition
     bool partitioned = false, have_pid = false, have_nbr = false;
@@ -902,7 +903,9 @@ static int check_shard(ddc_handle_t h, int nx, int ny, int y_begin, int y_count)
     return DDC_OK;
 }
 
-int ddc_set_mask_device(ddc_handle_t h, const int32_t* rows, int nx, int ny, int y_begin, int y_count)
+// the four set_mask calls: esize bytes per cell; host: copied into the handle's buffer, else borrowed
+static int set_mask(ddc_handle_t h, const void* rows, int esize, bool host, int nx, int ny, int y_begin, int y_count,
+    const char* name)
 {
     if (!h)
         return DDC_ERR_ARG;
@@ -910,8 +913,17 @@ int ddc_set_mask_device(ddc_handle_t h, const int32_t* rows, int nx, int ny, int
     if (rc)
         return rc;
     if (!rows && y_count > 0)
-        return fail(h, DDC_ERR_ARG, "ddc_set_mask_device: null mask");
+        return fail(h, DDC_ERR_ARG, "%s: null mask", name);
+    if (host) {
+        CUDA_TRY(h, cudaSetDevice(h->device));
+        const size_t n = (size_t)nx * y_count * esize;
+        CUDA_TRY(h, h->mask_own.ensure(n));
+        if (n)
+            CUDA_TRY(h, cudaMemcpyAsync(h->mask_own.p, rows, n, cudaMemcpyHostToDevice, h->stream));
+        rows = h->mask_own.p;
+    }
     h->d_mask = rows;
+    h->mask_esize = esize;
     h->nx = nx;
     h->ny = ny;
     h->y_begin = y_begin;
@@ -921,28 +933,24 @@ int ddc_set_mask_device(ddc_handle_t h, const int32_t* rows, int nx, int ny, int
     return DDC_OK;
 }
 
+int ddc_set_mask_device(ddc_handle_t h, const int32_t* rows, int nx, int ny, int y_begin, int y_count)
+{
+    return set_mask(h, rows, 4, false, nx, ny, y_begin, y_count, "ddc_set_mask_device");
+}
+
 int ddc_set_mask_host(ddc_handle_t h, const int32_t* rows, int nx, int ny, int y_begin, int y_count)
 {
-    if (!h)
-        return DDC_ERR_ARG;
-    int rc = check_shard(h, nx, ny, y_begin, y_count);
-    if (rc)
-        return rc;
-    if (!rows && y_count > 0)
-        return fail(h, DDC_ERR_ARG, "ddc_set_mask_host: null mask");
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    const size_t n = (size_t)nx * y_count;
-    CUDA_TRY(h, h->mask_own.ensure(n));
-    if (n)
-        CUDA_TRY(h, cudaMemcpyAsync(h->mask_own.p, rows, n * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
-    h->d_mask = h->mask_own.p;
-    h->nx = nx;
-    h->ny = ny;
-    h->y_begin = y_begin;
-    h->y_count = y_count;
-    h->mask_set = true;
-    h->partitioned = false;
-    return DDC_OK;
+    return set_mask(h, rows, 4, true, nx, ny, y_begin, y_count, "ddc_set_mask_host");
+}
+
+int ddc_set_mask_u8_device(ddc_handle_t h, const uint8_t* rows, int nx, int ny, int y_begin, int y_count)
+{
+    return set_mask(h, rows, 1, false, nx, ny, y_begin, y_count, "ddc_set_mask_u8_device");
+}
+
+int ddc_set_mask_u8_host(ddc_handle_t h, const uint8_t* rows, int nx, int ny, int y_begin, int y_count)
+{
+    return set_mask(h, rows, 1, true, nx, ny, y_begin, y_count, "ddc_set_mask_u8_host");
 }
 
 namespace {
@@ -1200,11 +1208,15 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
         h->clean_p2p = p2p;
     }
     h->clean[ci] = sig; // K2 of this step puts the buffer back into k_init's state
-    const bool vec = (NX % 4 == 0) && (((uintptr_t)h->d_mask) % 16 == 0);
+    // int32 mask: 16-byte loads of 4 columns; byte mask: 4-byte loads of 4 columns
+    const bool u8 = h->mask_esize == 1;
+    const bool vec = (NX % 4 == 0) && (((uintptr_t)h->d_mask) % (u8 ? 4 : 16) == 0);
     int* yr = reinterpret_cast<int*>(colcount + yr_off + 2 * h->rank);
     if (rows > 0 || p2p) { // an empty shard still has to push its (empty) counts and raise its flag
-        int rpc = vec ? pick_rows_per_cta(k_scan_mask<true>, std::max(rows, 1), gridx)
-                      : pick_rows_per_cta(k_scan_mask<false>, std::max(rows, 1), gridx);
+        int rpc = u8 ? (vec ? pick_rows_per_cta(k_scan_mask_u8<true>, std::max(rows, 1), gridx)
+                            : pick_rows_per_cta(k_scan_mask_u8<false>, std::max(rows, 1), gridx))
+                     : (vec ? pick_rows_per_cta(k_scan_mask<true>, std::max(rows, 1), gridx)
+                            : pick_rows_per_cta(k_scan_mask<false>, std::max(rows, 1), gridx));
         if (h->scan_rpc >= 8)
             rpc = h->scan_rpc & ~7;
         // the last `scan_tail` percent of the rows go in chunks of a quarter of the size (see the kernel)
@@ -1215,8 +1227,14 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
             nsmall = (rows - nbig * rpc + small - 1) / small;
         }
         dim3 grid(gridx, std::max(1, nbig + nsmall));
-        CUDA_TRY(h, launch_k(vec ? k_scan_mask<true> : k_scan_mask<false>, grid, dim3(256), 0, s, pdl, h->d_mask, NX, rows,
-            h->y_begin, NB, rpc, h->bits.p, colcount, yr, push_col, ps, h->done.p, yr_off, dbg, nbig, small));
+        if (u8)
+            CUDA_TRY(h, launch_k(vec ? k_scan_mask_u8<true> : k_scan_mask_u8<false>, grid, dim3(256), 0, s, pdl,
+                static_cast<const uint8_t*>(h->d_mask), NX, rows, h->y_begin, NB, rpc, h->bits.p, colcount, yr, push_col, ps,
+                h->done.p, yr_off, dbg, nbig, small));
+        else
+            CUDA_TRY(h, launch_k(vec ? k_scan_mask<true> : k_scan_mask<false>, grid, dim3(256), 0, s, pdl,
+                static_cast<const int32_t*>(h->d_mask), NX, rows, h->y_begin, NB, rpc, h->bits.p, colcount, yr, push_col, ps,
+                h->done.p, yr_off, dbg, nbig, small));
         launches++;
     }
     if (G > 1 && !p2p) // the first exchange step: column histogram and every rank's dot y-range in one sum

@@ -6,7 +6,8 @@
 //
 //   K1 k_scan_mask     int32 mask -> 1-bit ocean map + per-column ocean counts + dot y-range
 //                      (replaces Grid.cpp:176-188 and the Zoltan geometry callbacks
-//                       ZoltanPartitioner.cpp:19-67; HBM-bound, 4 B/cell read)
+//                       ZoltanPartitioner.cpp:19-67; HBM-bound, 4 B/cell read); k_scan_mask_u8: the same
+//                      from a byte mask (1 B/cell read), the same outputs bit for bit
 //   K2 k_xcuts         prefix sums of the column counts, preset cut directions, all x levels of
 //                      the RCB: every strip's path root -> strip walked at once, no level barriers
 //   K3 k_strip_rows    per-strip per-row ocean counts from the bit map (1/32 of the mask bytes)
@@ -812,6 +813,224 @@ __global__ void __launch_bounds__(256, 4) k_scan_mask(const int32_t* __restrict_
     }
     // every CTA has been counted: the counters are ready for the next step (k_init is then only needed when
     // the geometry changes)
+    for (unsigned i = threadIdx.x; i <= gridDim.x; i += blockDim.x)
+        done[i] = 0u;
+}
+
+// ------------------------------------------------------------------------------------------------
+// K1 on a byte mask (ddc_set_mask_u8_*): ocean <=> byte != 0
+// ------------------------------------------------------------------------------------------------
+// The int32 scan's geometry, grid and outputs, bit for bit: one warp per 128-column group, a lane owns 4 columns,
+// 8 rows make one packed register (nibble k = row k) and everything after that is the int32 kernel's epilogue.  A
+// lane's 4 columns are now one 4-byte word per row, so a warp load is one whole 128-byte line; to keep the bytes in
+// flight of the int32 kernel (4 to 8 16-byte loads per lane) a lane keeps 16 to 32 rows in flight, as two halves of
+// 16 rows, the next half requested before the current one is consumed.  VEC: NX % 4 == 0 and a 4-byte aligned
+// base pointer; otherwise every byte is loaded on its own, and no load ever reaches past a row's NX bytes.
+__device__ __forceinline__ unsigned ocean_nibble_u8(unsigned v)
+{
+    // the top bit of every byte: byte != 0; then bits 7, 15, 23, 31 gathered into bits 28..31 by one multiply
+    const unsigned t = (((v & 0x7f7f7f7fu) + 0x7f7f7f7fu) | v) & 0x80808080u;
+    return (t * 0x00204081u) >> 28;
+}
+
+template <bool VEC>
+__device__ __forceinline__ unsigned load_cols_u8(const uint8_t* __restrict__ row, int x, int xl, int NX)
+{
+    if (VEC)
+        return __ldcs(reinterpret_cast<const unsigned*>(row + xl));
+    unsigned v = 0;
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+        if (x + i < NX)
+            v |= (unsigned)__ldcs(row + x + i) << (8 * i);
+    return v;
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(256, 4) k_scan_mask_u8(const uint8_t* __restrict__ mask, int NX, int rows,
+    int y_begin, int NB, int rows_per_cta, uint8_t* __restrict__ bits, unsigned* __restrict__ colcount,
+    int* __restrict__ yr /* this rank's {-(first ocean row), last ocean row}, max-reduced */,
+    PeerPush push, PeerSync ps, unsigned* __restrict__ done /* [gridDim.x + 1], zeroed by k_init */, int yr_off,
+    unsigned long long* dbg, int nbig /* row chunks of rows_per_cta rows; the chunks after them hold rows_small */,
+    int rows_small)
+{
+    __shared__ __align__(16) uint8_t sbits[SCAN_STAGE_ROWS][128];
+    __shared__ int s_last;
+    pdl_trigger(); // the x-cut kernel may become resident (and warm up) while the scan is still running
+    const int lane = lane_id(), warp = threadIdx.x >> 5;
+    const int g = min(blockIdx.x * 8 + warp, NB / 16 - 1);
+    const bool warp_valid = blockIdx.x * 8 + warp < NB / 16;
+    const int big = (int)blockIdx.y < nbig;
+    const int r0 = big ? blockIdx.y * rows_per_cta : nbig * rows_per_cta + ((int)blockIdx.y - nbig) * rows_small;
+    const int r1 = min(rows, r0 + (big ? rows_per_cta : rows_small));
+    const int x = g * 128 + lane * 4;
+    unsigned c0 = 0, c1 = 0, c2 = 0, c3 = 0;
+    int ylo = 0x7fffffff, yhi = -1;
+
+    // VEC: out-of-range lanes (x >= NX, only in the last group) re-read the last 4 bytes of the row and are masked
+    // off below
+    const int xl = VEC ? min(x, NX - 4) : x;
+    const unsigned lane_valid = ((VEC && x >= NX) || !warp_valid) ? 0u : 0xffffffffu;
+    unsigned h0[16], h1[16];
+    // the previous step's labelling kernel still reads the bit map, and the mask may come from the caller's
+    // kernel just before this one in the stream
+    pdl_wait();
+    if (threadIdx.x == 0)
+        stamp_first(dbg, TS_SCAN);
+    if (VEC && r0 + 32 <= r1) {
+#pragma unroll
+        for (int k = 0; k < 16; k++)
+            h0[k] = load_cols_u8<true>(mask + (size_t)(r0 + k) * NX, x, xl, NX);
+    }
+    // rows [rb, rb + 8) of this CTA, packed: column counts, bit-map bytes (staged, flushed as whole lines) and the
+    // rows that hold an ocean cell, as in k_scan_mask
+    auto consume = [&](int rb, unsigned packed) {
+        packed &= lane_valid;
+        c0 += __popc(packed & 0x11111111u);
+        c1 += __popc(packed & 0x22222222u);
+        c2 += __popc(packed & 0x44444444u);
+        c3 += __popc(packed & 0x88888888u);
+        const unsigned other = __shfl_down_sync(0xffffffffu, packed, 1);
+        const unsigned even = (packed & 0x0f0f0f0fu) | ((other & 0x0f0f0f0fu) << 4); // rows 0,2,4,6
+        const unsigned odd = ((packed >> 4) & 0x0f0f0f0fu) | (other & 0xf0f0f0f0u); // rows 1,3,5,7
+        if (!(lane & 1)) {
+            uint8_t* sp = &sbits[(rb - r0) & (SCAN_STAGE_ROWS - 1)][warp * 16 + (lane >> 1)];
+#pragma unroll
+            for (int k = 0; k < 8; k++)
+                sp[k * 128] = (uint8_t)(((k & 1) ? odd : even) >> (8 * (k >> 1)));
+        }
+        if ((((rb - r0) + 8) & (SCAN_STAGE_ROWS - 1)) == 0 || rb + 8 >= r1) {
+            const int rs = r0 + ((rb - r0) & ~(SCAN_STAGE_ROWS - 1));
+            const int nr = min(rb + 8, r1) - rs;
+            __syncthreads();
+            for (int i = threadIdx.x; i < nr * 8; i += blockDim.x) {
+                const int row = i >> 3, c = i & 7;
+                if (blockIdx.x * 8 + c < NB / 16)
+                    *reinterpret_cast<uint4*>(bits + (size_t)(rs + row) * NB + (size_t)blockIdx.x * 128 + c * 16)
+                        = *reinterpret_cast<const uint4*>(&sbits[row][c * 16]);
+            }
+            __syncthreads();
+        }
+        const unsigned any = __reduce_or_sync(0xffffffffu, packed);
+        if (any) {
+            ylo = min(ylo, rb + ((__ffs(any) - 1) >> 2));
+            yhi = rb + ((31 - __clz(any)) >> 2);
+        }
+    };
+    for (int r = r0; r < r1; r += 32) {
+        if (VEC && r + 32 <= r1) {
+            // h0 holds rows [r, r + 16): request [r + 16, r + 32), consume h0, request the next iteration's first half
+#pragma unroll
+            for (int k = 0; k < 16; k++)
+                h1[k] = load_cols_u8<true>(mask + (size_t)(r + 16 + k) * NX, x, xl, NX);
+#pragma unroll
+            for (int b = 0; b < 2; b++) {
+                unsigned packed = 0;
+#pragma unroll
+                for (int k = 0; k < 8; k++)
+                    packed |= ocean_nibble_u8(h0[8 * b + k]) << (4 * k);
+                consume(r + 8 * b, packed);
+            }
+            if (r + 64 <= r1) {
+#pragma unroll
+                for (int k = 0; k < 16; k++)
+                    h0[k] = load_cols_u8<true>(mask + (size_t)(r + 32 + k) * NX, x, xl, NX);
+            }
+#pragma unroll
+            for (int b = 0; b < 2; b++) {
+                unsigned packed = 0;
+#pragma unroll
+                for (int k = 0; k < 8; k++)
+                    packed |= ocean_nibble_u8(h1[8 * b + k]) << (4 * k);
+                consume(r + 16 + 8 * b, packed);
+            }
+        } else {
+            // the last rows of the chunk (or every row without VEC): batches of 8 rows, loads guarded by row
+            for (int rb = r; rb < min(r + 32, r1); rb += 8) {
+                unsigned v[8];
+#pragma unroll
+                for (int k = 0; k < 8; k++) {
+                    v[k] = 0u;
+                    if (rb + k < r1 && warp_valid)
+                        v[k] = load_cols_u8<VEC>(mask + (size_t)(rb + k) * NX, x, xl, NX);
+                }
+                unsigned packed = 0;
+#pragma unroll
+                for (int k = 0; k < 8; k++)
+                    packed |= ocean_nibble_u8(v[k]) << (4 * k);
+                consume(rb, packed);
+            }
+        }
+    }
+    if (c0)
+        atomicAdd(colcount + x, c0);
+    if (c1)
+        atomicAdd(colcount + x + 1, c1);
+    if (c2)
+        atomicAdd(colcount + x + 2, c2);
+    if (c3)
+        atomicAdd(colcount + x + 3, c3);
+    if (lane == 0 && yhi >= 0) {
+        const int ny0 = -(y_begin + ylo), y1 = y_begin + yhi;
+        if (ny0 > yr[0])
+            atomicMax(&yr[0], ny0);
+        if (y1 > yr[1])
+            atomicMax(&yr[1], y1);
+    }
+    if (threadIdx.x == 0)
+        stamp_last(dbg, TS_SCAN + 1);
+    if (push.n <= 1)
+        return;
+    // exchange step 1 (several GPUs), as in k_scan_mask
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        s_last = atomicAdd(&done[blockIdx.x], 1u) == gridDim.y - 1;
+        if (s_last)
+            __threadfence();
+    }
+    __syncthreads();
+    if (!s_last)
+        return;
+    const int c = blockIdx.x * 1024 + threadIdx.x * 4;
+    if (c < yr_off) {
+        const uint4 v = __ldcg(reinterpret_cast<const uint4*>(colcount + c));
+        if (push.packed) {
+            const unsigned long long w0 = ll_word(v.x | (v.y << 16), ps.step), w1 = ll_word(v.z | (v.w << 16), ps.step);
+            for (int q = 0; q < push.n; q++)
+                if (q != push.rank)
+                    ll_store2(reinterpret_cast<unsigned long long*>(push.dst[q]) + (c >> 1), w0, w1);
+        } else {
+            const unsigned long long w0 = ll_word(v.x, ps.step), w1 = ll_word(v.y, ps.step), w2 = ll_word(v.z, ps.step),
+                                     w3 = ll_word(v.w, ps.step);
+            for (int q = 0; q < push.n; q++)
+                if (q != push.rank) {
+                    unsigned long long* d = reinterpret_cast<unsigned long long*>(push.dst[q]) + c;
+                    ll_store2(d, w0, w1);
+                    ll_store2(d + 2, w2, w3);
+                }
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        stamp_last(dbg, TS_SCAN + 2);
+        s_last = atomicAdd(&done[gridDim.x], 1u) == gridDim.x - 1;
+        if (s_last)
+            __threadfence();
+    }
+    __syncthreads();
+    if (!s_last)
+        return;
+    if ((int)threadIdx.x < push.n) {
+        const int q = threadIdx.x;
+        if (q != push.rank) {
+            unsigned long long* d = reinterpret_cast<unsigned long long*>(push.dst[q]) + ll_column_words(yr_off, push.packed);
+            ll_store2(d, ll_word((unsigned)__ldcg(yr), ps.step), ll_word((unsigned)__ldcg(yr + 1), ps.step));
+        } else
+            peer_signal_local(ps, 0);
+        if (threadIdx.x == 0)
+            stamp_last(dbg, TS_SCAN + 3);
+    }
     for (unsigned i = threadIdx.x; i <= gridDim.x; i += blockDim.x)
         done[i] = 0u;
 }

@@ -144,6 +144,18 @@ DDC_API int ddc_set_mask_host(ddc_handle_t h, const int32_t* rows, int nx, int n
 DDC_API int ddc_set_mask_device(ddc_handle_t h, const int32_t* rows, int nx, int ny, int y_begin,
     int y_count);
 
+/* The same with one byte per cell (a bool / uint8 tensor, a netCDF byte or ubyte variable): the same arguments,
+   shard rule, ownership and status codes.  A cell is ocean <=> its byte is non-zero, read as unsigned, so 0xFF is
+   ocean (the int32 rule makes -1 land): a signed byte mask that stores land as a negative value must be converted
+   first.  The scan reads a quarter of the int32 bytes and computes the same decomposition bit for bit.  The handle
+   keeps the type of the mask it was last given; switching between decompositions is allowed, and with nranks > 1
+   every rank may use either type.  Fastest with nx % 4 == 0 and a 4-byte aligned pointer; other masks are read
+   byte by byte, never past a row's nx bytes. */
+DDC_API int ddc_set_mask_u8_host(ddc_handle_t h, const uint8_t* rows, int nx, int ny, int y_begin,
+    int y_count);
+DDC_API int ddc_set_mask_u8_device(ddc_handle_t h, const uint8_t* rows, int nx, int ny, int y_begin,
+    int y_count);
+
 /* the row block of `rank`: rows_per_rank = ceil(ny / nranks), last ranks may be short / empty */
 DDC_API void ddc_shard_rows(int ny, int nranks, int rank, int* y_begin, int* y_count);
 

@@ -156,12 +156,6 @@ cudaError_t opt_in_smem(K kernel, int device, int which, size_t need)
         have = need;
     return e;
 }
-
-int env_int(const char* name, int dflt)
-{
-    const char* e = getenv(name);
-    return e && *e ? atoi(e) : dflt;
-}
 } // namespace
 
 struct ddc_handle_s {
@@ -192,16 +186,7 @@ struct ddc_handle_s {
     bool halo_ok = false; // the plan is of the current decomposition
     bool halo_shard_ok = false; // ... and ddc_halo_shard_offsets was called for it
     int halo_w = 1; // the frame width of the halo calls (ddc_halo_set_width)
-    DevBuf<unsigned> gate; // the word the gate kernel of the second stream waits for (see BoxGate)
-    int use_gate = 1; // DDC_GATE: 0 never, 1 unless the shard is tiny, 2 always
-    bool side_pdl = true; // DDC_SIDE_PDL: the scan of the neighbour counts launched programmatically behind the count kernel
-                          // (-4 us at C2, neutral elsewhere)
-    bool dev_join = false; // DDC_DEV_JOIN: the labelling kernel's last block waits for the neighbour kernels instead of an event join
-                           // (off: measured +13 us at C5, +2.5 us at C2 / C3, -1 us at C4 on one GPU)
-    bool row_flags = true; // DDC_ROW_FLAGS: exchange step 2 with one flag per block of the row-count kernel (default: 2 ranks
-                           // only -- measured -2.4 us on 2 GPUs, +4 us on 8, where a block has 8 flags to send)
-    int early = 17; // DDC_EARLY, bit mask (default 1 + 16): which kernels poll a flag / word instead of waiting for the previous kernel's
-                   // completion (ChainWord): 1 k_sum_cols, 2 K4, 4 labelling kernel, 8 row counts, 16 K2
+    DevBuf<unsigned> gate; // words polled in place of a kernel boundary (see ddc_create)
     DevBuf<Plan> plan;
     DevBuf<int> strips; // x0[P+1] x1[P+1] p0[P+2] S always
     DevBuf<int> boxes; // x0 y0 ex ey, P each
@@ -213,12 +198,8 @@ struct ddc_handle_s {
     // the plan the launches were sized for, and what it was assumed for (see enqueue_partition)
     int plan_nx = 0, plan_ny = 0, plan_P = 0, aix = 0, aiy = 0;
     bool pending = false, profiled = false; // a step is enqueued but not yet validated
-    int last_flags = 0, strip_k = 0;
-    // knobs (environment, read once in ddc_create): DDC_PDL=0 plain stream order between the kernels,
-    // DDC_FUSE_FIN=0
-    // k_finalize as a kernel of its own after the labelling kernel, DDC_DEBUG_TS=1 time stamps, DDC_SCAN_RPC / DDC_LABEL_RPC rows per CTA
-    bool use_pdl = true, fuse_fin = true, debug_ts = false;
-    int scan_rpc = 0, label_rpc = 0, scan_tail = 25;
+    int last_flags = 0;
+    bool debug_ts = false; // DDC_DEBUG_TS=1 (read in ddc_create): time stamps of every phase (Plan::ts)
     PeerSync fin_ps {}; // the exchange state of the last step, for a k_finalize launched from validate()
     size_t xcuts_static = 0, ycuts_static = 0; // static shared memory of the cut kernels (0: not yet asked)
     // what K2 (column counts, scalars) and the scan's last CTA (counters) left clean for a later step: k_init is
@@ -302,28 +283,6 @@ int fail(ddc_handle_t h, int code, const char* fmt, ...)
                 g_nccl.GetErrorString(r_), __FILE__, __LINE__);                                    \
     } while (0)
 
-NaiveParams naive_params(int P, int NX, int NY)
-{
-    // Grid.cpp:18-35 (find_factors) and Grid.cpp:153-155 (float ceil)
-    int fa = -1, fb = -1;
-    for (int i = 2; i * i <= P; i += 2)
-        if (P % i == 0) {
-            fa = i;
-            fb = P / fa;
-        }
-    NaiveParams nv;
-    if (fa == -1 || fb == -1) {
-        nv.np0 = P;
-        nv.np1 = 1;
-    } else {
-        nv.np0 = fa;
-        nv.np1 = fb;
-    }
-    nv.lx = (int)ceilf((float)NX / (float)nv.np0);
-    nv.ly = (int)ceilf((float)NY / (float)nv.np1);
-    return nv;
-}
-
 struct Tables {
     StripTable st;
     BoxTable bx;
@@ -391,12 +350,12 @@ int run_neighbours(ddc_handle_t h, int P, int nx, int ny, int px, int py)
     const int warps_per_cta = 8;
     const int grid = (std::max(P, 8) + warps_per_cta - 1) / warps_per_cta; // >= 8 * pad32(P) threads
     CUDA_TRY(h, launch_k(k_neighbours<false>, dim3(grid), dim3(256), 0, s, false, t.bx, P, nx, ny, px, py, t.st,
-        h->nbr_counts.p, nullptr, nullptr, h->nbr_cap, nullptr, nullptr, nullptr, h->sc.p, nullptr, ChainWord { nullptr, 0u }, nullptr));
+        h->nbr_counts.p, nullptr, nullptr, h->nbr_cap, nullptr, nullptr, nullptr, h->sc.p, nullptr));
     CUDA_TRY(h, launch_k(k_scan_counts, dim3(8), dim3(1024), 0, s, false, h->nbr_counts.p, P, h->nbr_offsets.p,
         h->nbr_totals.p, nullptr));
     CUDA_TRY(h, launch_k(k_neighbours<true>, dim3(grid), dim3(256), 0, s, false, t.bx, P, nx, ny, px, py, t.st,
         h->nbr_counts.p, h->nbr_offsets.p, h->nbr_totals.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p,
-        h->sc.p, nullptr, ChainWord { nullptr, 0u }, nullptr));
+        h->sc.p, nullptr));
     h->stats.gpu_launches += 3;
     CUDA_TRY(h, cudaGetLastError());
     h->totals_valid = false;
@@ -428,7 +387,7 @@ int fetch_totals(ddc_handle_t h)
         const int grid = (std::max(h->nparts, 8) + 7) / 8;
         CUDA_TRY(h, launch_k(k_neighbours<true>, dim3(grid), dim3(256), 0, h->stream, false, t.bx, h->nparts, h->nx, h->ny,
             h->px, h->py, t.st, h->nbr_counts.p, h->nbr_offsets.p, h->nbr_totals.p, h->nbr_cap, h->nbr_ids.p,
-            h->nbr_halos.p, h->nbr_starts.p, h->sc.p, nullptr, ChainWord { nullptr, 0u }, nullptr));
+            h->nbr_halos.p, h->nbr_starts.p, h->sc.p, nullptr));
         CUDA_TRY(h, cudaGetLastError());
         CUDA_TRY(h, cudaMemcpyAsync(&hs, h->sc.p, sizeof hs, cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
@@ -622,13 +581,11 @@ int ddc_create(ddc_handle_t* out, int device, int rank, int nranks, const void* 
     h->stream = h->own_stream;
     {
         // highest priority: the small neighbour kernels must get SM slots while the labelling
-        // kernel still has tens of thousands of CTAs queued
+        // kernel still has tens of thousands of CTAs queued (also on several GPUs, where every rank builds ALL
+        // neighbour tables beside a labelling kernel that has only 1 / G of the cells: DESIGN.md 5)
         int least = 0, greatest = 0;
         CREATE_TRY(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        // (DDC_SIDE_PRIO=0: the priority of a default stream -- on several GPUs every rank builds ALL neighbour tables
-        //  beside a labelling kernel that has only 1 / G of the cells, see DESIGN.md 5)
-        CREATE_TRY(cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking,
-            env_int("DDC_SIDE_PRIO", 1) ? greatest : least));
+        CREATE_TRY(cudaStreamCreateWithPriority(&h->side_stream, cudaStreamNonBlocking, greatest));
     }
     CREATE_TRY(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     CREATE_TRY(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
@@ -638,27 +595,10 @@ int ddc_create(ddc_handle_t* out, int device, int rank, int nranks, const void* 
     for (auto& ev : h->ev)
         CREATE_TRY(cudaEventCreate(&ev));
     h->ev_ok = true;
-    if (const char* e = getenv("DDC_STRIP_K")) { // tuning knob of the strip row-count kernel
-        const int v = atoi(e);
-        h->strip_k = (v == 1 || v == 2 || v == 4 || v == 8) ? v : 0;
-    }
-    if (const char* e = getenv("DDC_WALK_LANES")) { // tuning knob of the cut kernels
-        const int v = std::max(1, std::min(32, atoi(e)));
-        CREATE_TRY(cudaMemcpyToSymbol(g_walk_lanes, &v, sizeof v));
-    }
-    h->use_pdl = env_int("DDC_PDL", 1) != 0;
-    h->fuse_fin = env_int("DDC_FUSE_FIN", 1) != 0;
-    h->debug_ts = env_int("DDC_DEBUG_TS", 0) != 0;
-    h->scan_rpc = env_int("DDC_SCAN_RPC", 0);
-    h->scan_tail = std::max(0, std::min(90, env_int("DDC_SCAN_TAIL", 25)));
-    h->label_rpc = env_int("DDC_LABEL_RPC", 0);
-    h->use_gate = env_int("DDC_GATE", 1);
-    h->early = env_int("DDC_EARLY", 17);
-    h->dev_join = env_int("DDC_DEV_JOIN", 0) != 0;
-    h->side_pdl = env_int("DDC_SIDE_PDL", 1) != 0;
-    h->row_flags = env_int("DDC_ROW_FLAGS", nranks <= 2 ? 1 : 0) != 0;
-    CREATE_TRY(h->gate.ensure(4)); // [0] K4 -> labelling kernel / second stream, [1] k_sum_cols -> K2, [2] K2 -> K3 (ChainWord)
-    CREATE_TRY(cudaMemset(h->gate.p, 0, 4 * sizeof(unsigned)));
+    const char* ts = getenv("DDC_DEBUG_TS");
+    h->debug_ts = ts && *ts && atoi(ts) != 0;
+    CREATE_TRY(h->gate.ensure(2)); // [0] K4 -> second stream (BoxGate), [1] k_sum_cols -> K2 (ChainWord)
+    CREATE_TRY(cudaMemset(h->gate.p, 0, 2 * sizeof(unsigned)));
     CREATE_TRY(h->sc.ensure(1));
     CREATE_TRY(h->plan.ensure(1));
     CREATE_TRY(cudaMemset(h->plan.p, 0, sizeof(Plan)));
@@ -743,11 +683,10 @@ int ddc_destroy(ddc_handle_t h)
     return DDC_OK;
 }
 
-static void guess_plan_public(int P, int NX, int NY, int* ix, int* iy);
 static void peer_capacity(int nx, int ny, int nparts, int G, size_t* colcap, size_t* rowcap, size_t* flagcap)
 {
     int ix, iy;
-    guess_plan_public(nparts, nx, ny, &ix, &iy);
+    guess_plan(nparts, nx, ny, &ix, &iy);
     const size_t Scap = (size_t)std::min<long long>(nparts, 1LL << std::min(ix, 30));
     const size_t Rmax = ((size_t)ny + G - 1) / G;
     const size_t elems = iy > 0 ? Scap * ((Rmax + 31) & ~(size_t)31) : 0; // whole row blocks (row_count_index)
@@ -979,30 +918,6 @@ int ddc_synchronize(ddc_handle_t h)
 // the hot path
 // ------------------------------------------------------------------------------------------------
 namespace {
-// The numbers of x / y levels depend on the bounding box of the dots, i.e. on the data, and they
-// size the launches after K2 (strip count, row-count buffers, the all-gather).  Instead of reading
-// the plan back in the middle of the pipeline, the host ASSUMES a plan -- the one of the previous
-// call on the same geometry, else the one of a full-extent bounding box -- K2 compares it with the
-// real one, and on a mismatch every later kernel does nothing; the step is then run again with the
-// real plan (validate(), at the end of ddc_partition or, with DDC_ASYNC, in the first getter).
-void guess_plan(int P, int NX, int NY, int* ix, int* iy)
-{
-    double wx = (double)(NX - 1), wy = (double)(NY - 1);
-    *ix = *iy = 0;
-    for (int t = P; t > 1; t = (t + 1) / 2) {
-        if (wx > wy) {
-            (*ix)++;
-            wx /= 2.0;
-        } else {
-            (*iy)++;
-            wy /= 2.0;
-        }
-    }
-}
-
-} // namespace
-static void guess_plan_public(int P, int NX, int NY, int* ix, int* iy) { guess_plan(P, NX, NY, ix, iy); }
-namespace {
 // K5 (one block): `changes` of all ranks; when nothing moved, the naive blocks and the neighbour tables rebuilt
 // from them; the plan into the host's pinned copy.  Uses nparts / px / py / nx / ny of the handle.
 int launch_finalize(ddc_handle_t h, const PeerSync& ps, bool want_nbr)
@@ -1140,7 +1055,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
         return fail(h, DDC_ERR_STATE, "%d ranks but no exchange path: created without a NCCL id and %s", G,
             h->p2p ? "the decomposition exceeds the exported peer buffers" : "no peer buffers imported");
     const int par = (int)(h->step & 1u);
-    const bool pdl = h->use_pdl && !profile; // (event records between the kernels would break the chain anyway)
+    const bool pdl = !profile; // (event records between the kernels would break the chain anyway)
     unsigned long long* dbg = h->debug_ts
         ? reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(h->plan.p) + offsetof(Plan, ts))
         : nullptr;
@@ -1189,7 +1104,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     const int gridx = (NG + 7) / 8;
     // counters of the "last block" patterns: [0, gridx] mask scan, [gridx + 1] strip row counts, then the
     // 64-bit counter of the labelling kernel; all zero between steps (their last blocks reset them)
-    const int d_rows = gridx + 1, d_label = (gridx + 3) & ~1, d_ycuts = d_label + 2, d_sum = d_ycuts + 1, d_nbr = d_sum + 1, ndone = d_nbr + 1;
+    const int d_rows = gridx + 1, d_label = (gridx + 3) & ~1, d_ycuts = d_label + 2, d_sum = d_ycuts + 1, ndone = d_sum + 1;
     CUDA_TRY(h, h->done.ensure((size_t)ndone));
     ddc_handle_s::CleanSig sig;
     sig.col = colcount;
@@ -1213,17 +1128,15 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     const bool vec = (NX % 4 == 0) && (((uintptr_t)h->d_mask) % (u8 ? 4 : 16) == 0);
     int* yr = reinterpret_cast<int*>(colcount + yr_off + 2 * h->rank);
     if (rows > 0 || p2p) { // an empty shard still has to push its (empty) counts and raise its flag
-        int rpc = u8 ? (vec ? pick_rows_per_cta(k_scan_mask_u8<true>, std::max(rows, 1), gridx)
-                            : pick_rows_per_cta(k_scan_mask_u8<false>, std::max(rows, 1), gridx))
-                     : (vec ? pick_rows_per_cta(k_scan_mask<true>, std::max(rows, 1), gridx)
-                            : pick_rows_per_cta(k_scan_mask<false>, std::max(rows, 1), gridx));
-        if (h->scan_rpc >= 8)
-            rpc = h->scan_rpc & ~7;
-        // the last `scan_tail` percent of the rows go in chunks of a quarter of the size (see the kernel)
+        const int rpc = u8 ? (vec ? pick_rows_per_cta(k_scan_mask_u8<true>, std::max(rows, 1), gridx)
+                                  : pick_rows_per_cta(k_scan_mask_u8<false>, std::max(rows, 1), gridx))
+                           : (vec ? pick_rows_per_cta(k_scan_mask<true>, std::max(rows, 1), gridx)
+                                  : pick_rows_per_cta(k_scan_mask<false>, std::max(rows, 1), gridx));
+        // the last quarter of the rows go in chunks of a quarter of the size (see the kernel)
         const int small = std::max(8, (rpc / 4) & ~7);
         int nbig = (rows + rpc - 1) / rpc, nsmall = 0;
-        if (h->scan_tail > 0 && small < rpc && rows >= 4 * rpc) {
-            nbig = (int)((long long)rows * (100 - h->scan_tail) / 100) / rpc;
+        if (small < rpc && rows >= 4 * rpc) {
+            nbig = (int)((long long)rows * 75 / 100) / rpc;
             nsmall = (rows - nbig * rpc + small - 1) / small;
         }
         dim3 grid(gridx, std::max(1, nbig + nsmall));
@@ -1242,15 +1155,12 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     // several GPUs: a grid of blocks waits for the ranks' flags and sums their column-count slots into ONE buffer,
     // the x-cut block then reads global counts as on one GPU
     const bool presum = p2p;
-    // words polled in place of a kernel boundary (ChainWord; only between programmatic launches)
-    ChainWord w_none { nullptr, 0u }, w_sum = w_none, w_strips = w_none;
-    if (pdl && presum && (h->early & 16))
-        w_sum = ChainWord { h->gate.p + 1, h->step };
-    if (pdl && (h->early & 8))
-        w_strips = ChainWord { h->gate.p + 2, h->step };
+    // between programmatic launches k_sum_cols polls the scan's local flag, and K2 polls the word k_sum_cols publishes,
+    // in place of the kernel boundaries (ChainWord)
+    const ChainWord w_sum = pdl && presum ? ChainWord { h->gate.p + 1, h->step } : ChainWord { nullptr, 0u };
     if (presum) {
         CUDA_TRY(h, launch_k(k_sum_cols, dim3(gridx), dim3(256), 0, s, pdl, pc, ps, NX, yr_off, h->colsum.p, h->plan.p,
-            pdl && (h->early & 1) ? 1 : 0, h->done.p + d_sum, w_sum, dbg));
+            pdl ? 1 : 0, h->done.p + d_sum, w_sum, dbg));
         launches++;
         pc = PeerCols {};
         pc.col[0] = h->colsum.p;
@@ -1269,11 +1179,11 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
         CUDA_TRY(h, opt_in_smem(k_xcuts<true>, h->device, 0, std::max<size_t>(xneed, 48 * 1024)));
         CUDA_TRY(h, launch_k(k_xcuts<true>, dim3(1), dim3(1024), xneed, s, pdl, pc, ps_x, NX, NY, P, nullptr, yr_off, G, aix,
             aiy, h->plan.p, t.st, t.bx, h->loads.p, h->loadmm.p, h->sc.p, colcount, dbg ? 1 : 0,
-            h->pin_plan_dev, presum ? 1 : 0, reset_in_label ? 0 : 1, w_sum, ycuts ? w_strips : w_none));
+            h->pin_plan_dev, presum ? 1 : 0, reset_in_label ? 0 : 1, w_sum));
     } else
         CUDA_TRY(h, launch_k(k_xcuts<false>, dim3(1), dim3(1024), LEVEL_NODES_BYTES, s, pdl, pc, ps_x, NX, NY, P, h->colpfx.p, yr_off, G, aix,
             aiy, h->plan.p, t.st, t.bx, h->loads.p, h->loadmm.p, h->sc.p, colcount, dbg ? 1 : 0,
-            h->pin_plan_dev, presum ? 1 : 0, reset_in_label ? 0 : 1, w_sum, ycuts ? w_strips : w_none));
+            h->pin_plan_dev, presum ? 1 : 0, reset_in_label ? 0 : 1, w_sum));
     launches++;
     // the column -> strip table K6 reads: painted by K4's blocks; without y levels there is no K4
     if (!ycuts) {
@@ -1285,12 +1195,10 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     // the second stream (neighbour tables beside the labelling kernel) is forked by a device-side gate when K4 runs
     // and nothing else has to sit between K4 and the labelling kernel (no profiling events)
     // (not on tiny shards: there the neighbour kernels end the step, and starting them behind a polling kernel instead of
-    //  an event costs more than the programmatic launch of a 9 us labelling kernel saves -- 528 x 522: +3 us with the gate;
-    //  DDC_GATE=2 forces it)
-    const bool gated = h->use_gate && want_nbr && ycuts && !profile && (h->use_gate > 1 || (long long)rows * NX >= (1LL << 21));
-    const bool label_polls = pdl && ycuts && (h->early & 4); // the labelling kernel polls the same word
+    //  an event costs more than the programmatic launch of a 9 us labelling kernel saves -- 528 x 522: +3 us with the gate)
+    const bool gated = want_nbr && ycuts && !profile && (long long)rows * NX >= (1LL << 21);
     BoxGate gate {};
-    if (gated || label_polls) {
+    if (gated) {
         gate.word = h->gate.p;
         gate.done = h->done.p + d_ycuts;
         gate.step = h->step;
@@ -1306,14 +1214,14 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
             // (measured at C3 / C4 / one eighth of C5: two rows per warp beat one -- whole row in registers or not --
             //  by 2-4 us: half the blocks, each amortising its boundary table over twice the rows)
             int K = Rmax >= 32 * 4 * 148 ? 4 : 2;
-            if (h->strip_k) // DDC_STRIP_K: tuning knob (1, 2, 4: rows per warp; 8: one row per warp, whole row at once)
-                K = h->strip_k == 8 ? 1 : h->strip_k;
             while (K > 1 && sizeof(int) * strip_scan_smem_words(NG, Scap, K) > 48 * 1024)
                 K >>= 1;
             const size_t scan_smem = sizeof(int) * strip_scan_smem_words(NG, Scap, K);
             if (scan_smem <= 48 * 1024) { // the streaming kernel: boundary table in shared memory
                 const int grid = (Rmax + 8 * K - 1) / (8 * K);
-                if (p2p && h->row_flags && (size_t)grid <= h->x_flagcap) { // one flag per block (row_flags_raise)
+                // one flag per block (row_flags_raise) on 2 ranks: measured -2.4 us on 2 GPUs, but +4 us on 8, where a
+                // block has 8 flags to send
+                if (p2p && G <= 2 && (size_t)grid <= h->x_flagcap) {
                     const size_t off = peer_words(G, h->x_colcap, h->x_rowcap, 0);
                     for (int q = 0; q < G; q++)
                         ps_rows.rowflag[q] = h->xpeer[q] + off;
@@ -1321,36 +1229,30 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
                     ps_rows.rowblocks = grid;
                 }
                 rb_shift = K == 4 ? 5 : (K == 2 ? 4 : 3);
-#define LAUNCH_SCAN(CT, KK, FF)                                                                    \
-    CUDA_TRY(h, launch_k(k_strip_rows_scan<CT, KK, FF>, dim3(grid), dim3(256), scan_smem, s, pdl, h->bits.p, NB, NX, rows, \
-        t.st.x0, t.st.p0, h->plan.p, Scap, push_row, Rmax, ps_rows, h->done.p + d_rows, dbg, w_strips))
-                // small shards: one row per warp, the whole row requested at once (rows of <= 8 chunks)
-                const bool full = h->strip_k == 8 && K == 1 && NG <= 256;
+#define LAUNCH_SCAN(CT, KK)                                                                        \
+    CUDA_TRY(h, launch_k(k_strip_rows_scan<CT, KK>, dim3(grid), dim3(256), scan_smem, s, pdl, h->bits.p, NB, NX, rows, \
+        t.st.x0, t.st.p0, h->plan.p, Scap, push_row, Rmax, ps_rows, h->done.p + d_rows, dbg))
                 if (narrow) {
                     if (K == 4)
-                        LAUNCH_SCAN(uint16_t, 4, false);
+                        LAUNCH_SCAN(uint16_t, 4);
                     else if (K == 2)
-                        LAUNCH_SCAN(uint16_t, 2, false);
-                    else if (full)
-                        LAUNCH_SCAN(uint16_t, 1, true);
+                        LAUNCH_SCAN(uint16_t, 2);
                     else
-                        LAUNCH_SCAN(uint16_t, 1, false);
+                        LAUNCH_SCAN(uint16_t, 1);
                 } else {
                     if (K == 4)
-                        LAUNCH_SCAN(unsigned, 4, false);
+                        LAUNCH_SCAN(unsigned, 4);
                     else if (K == 2)
-                        LAUNCH_SCAN(unsigned, 2, false);
-                    else if (full)
-                        LAUNCH_SCAN(unsigned, 1, true);
+                        LAUNCH_SCAN(unsigned, 2);
                     else
-                        LAUNCH_SCAN(unsigned, 1, false);
+                        LAUNCH_SCAN(unsigned, 1);
                 }
 #undef LAUNCH_SCAN
             } else {
                 dim3 grid((Rmax + 31) / 32, (Scap + 7) / 8);
                 CUDA_TRY(h, launch_k(narrow ? k_strip_rows<uint16_t> : k_strip_rows<unsigned>, grid, dim3(256), 0, s, pdl,
                     h->bits.p, NB, rows, t.st.x0, t.st.x1, t.st.p0, h->plan.p, Scap, push_row, Rmax, ps, h->done.p + d_rows,
-                    dbg, w_strips));
+                    dbg));
             }
             launches++;
         }
@@ -1369,8 +1271,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
         if (SM)                                                                                    \
             CUDA_TRY(h, opt_in_smem(k_ycuts<CT, SM>, h->device, which, std::max<size_t>(yneed, 48 * 1024))); \
         CUDA_TRY(h, launch_k(k_ycuts<CT, SM>, dim3(ygrid), dim3(1024), SM ? yneed : LEVEL_NODES_BYTES, s, pdl, pr, ps_rows, rl, NY, t.st, \
-            h->ypfx.p, t.bx, h->loads.p, h->loadmm.p, h->plan.p, h->strip_of_col.p, dbg ? 1 : 0, gate, h->part_at.p, nchunk, \
-            pdl && p2p && (h->early & 2) ? 1 : 0)); \
+            h->ypfx.p, t.bx, h->loads.p, h->loadmm.p, h->plan.p, h->strip_of_col.p, dbg ? 1 : 0, gate, h->part_at.p, nchunk)); \
     } while (0)
         if (narrow) {
             if (y_smem)
@@ -1403,12 +1304,8 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     // a quarter of the warp-per-part grid that caller-supplied boxes need (run_neighbours)
     const int ngrid = std::max(1, (8 * ((P + 31) & ~31) + 255) / 256);
     // The labelling kernel's last block also ends the step (`changes`, exchange step 3, the plan into the host's
-    // pinned copy) unless there is no labelling kernel on this rank or the exchange goes through NCCL ...
-    const bool fuse = h->fuse_fin && label_runs && (G == 1 || p2p);
-    // ... and then it also waits for the neighbour kernels of the second stream (a word in device memory) instead of
-    // the host joining the streams with an event
-    const bool dev_join = h->dev_join && fuse && want_nbr;
-    const ChainWord w_nbr = dev_join ? ChainWord { h->gate.p + 3, h->step } : ChainWord { nullptr, 0u };
+    // pinned copy) unless there is no labelling kernel on this rank or the exchange goes through NCCL.
+    const bool fuse = label_runs && (G == 1 || p2p);
     if (want_nbr) {
         cudaStream_t q = h->side_stream;
         if (!gated) {
@@ -1416,25 +1313,23 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
             CUDA_TRY(h, cudaStreamWaitEvent(q, h->ev_fork, 0));
         }
         CUDA_TRY(h, launch_k(k_neighbours<false>, dim3(ngrid), dim3(256), 0, q, false, t.bx, P, NX, NY, px, py, t.st,
-            h->nbr_counts.p, nullptr, nullptr, h->nbr_cap, nullptr, nullptr, nullptr, h->sc.p, h->plan.p, ChainWord { nullptr, 0u }, nullptr));
-        CUDA_TRY(h, launch_k(k_scan_counts, dim3(8), dim3(1024), 0, q, pdl && h->side_pdl, h->nbr_counts.p, P, h->nbr_offsets.p,
+            h->nbr_counts.p, nullptr, nullptr, h->nbr_cap, nullptr, nullptr, nullptr, h->sc.p, h->plan.p));
+        CUDA_TRY(h, launch_k(k_scan_counts, dim3(8), dim3(1024), 0, q, pdl, h->nbr_counts.p, P, h->nbr_offsets.p,
             h->nbr_totals.p, h->plan.p));
         // (the fill kernel with a plain launch: its P / 8 blocks, resident and waiting on the high-priority stream while the
         //  8 blocks of the scan run, took the SMs from the labelling kernel -- +15 us at C5)
         CUDA_TRY(h, launch_k(k_neighbours<true>, dim3(ngrid), dim3(256), 0, q, false, t.bx, P, NX, NY, px, py, t.st,
             h->nbr_counts.p, h->nbr_offsets.p, h->nbr_totals.p, h->nbr_cap, h->nbr_ids.p, h->nbr_halos.p, h->nbr_starts.p,
-            h->sc.p, h->plan.p, w_nbr, h->done.p + d_nbr));
+            h->sc.p, h->plan.p));
         launches += 3;
         CUDA_TRY(h, cudaEventRecord(h->ev_join, q));
     }
     // ---- K6: labels + `changes` -----------------------------------------------------------------
-    // The labelling kernel's last block also ends the step (`changes`, exchange step 3, the plan into the host's
-    // pinned copy) unless there is no labelling kernel on this rank or the exchange goes through NCCL.
     h->fin_ps = ps;
     if (label_runs) {
         const bool vecp = want_pid && (NX % 4 == 0) && (((uintptr_t)h->pid.p) % 16 == 0);
         // no heavy per-CTA epilogue: many small CTAs keep more stores in flight
-        const int rpc = h->label_rpc >= 8 ? (h->label_rpc & ~7) : 32;
+        const int rpc = 32;
         const dim3 grid(gridx, (rows + rpc - 1) / rpc);
         LabelEnd fin {};
         fin.fuse = fuse ? 1 : 0;
@@ -1448,9 +1343,6 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
         fin.reset_col = reset_in_label ? colcount : nullptr;
         fin.reset_n = ncol;
         fin.yr_off = yr_off;
-        if (label_polls)
-            fin.prev = ChainWord { h->gate.p, h->step };
-        fin.nbr = w_nbr;
         auto kernel = !want_pid ? k_label<false, false> : (vecp ? k_label<true, true> : k_label<false, true>);
         // (behind K4 without a stream operation in between when the second stream is gated: programmatic launch)
         CUDA_TRY(h, launch_k(kernel, grid, dim3(256), 0, s, pdl && (gated || !want_nbr), h->bits.p, NX, rows, h->y_begin, NB, rpc, h->strip_of_col.p,
@@ -1460,7 +1352,7 @@ int enqueue_partition(ddc_handle_t h, int nparts, int px, int py, int flags)
     if (G > 1 && !p2p)
         NCCL_TRY(h, g_nccl.AllReduce(&h->sc.p->changes, &h->sc.p->changes, 1, nccl_Int32, nccl_Max, h->comm, s));
     mark(5);
-    if (want_nbr && !dev_join)
+    if (want_nbr)
         CUDA_TRY(h, cudaStreamWaitEvent(s, h->ev_join, 0)); // the step is over when the neighbour tables are, too
     // ---- K5 as a kernel of its own (see above; otherwise only from validate(), when nothing moved) ----
     if (!fuse) {

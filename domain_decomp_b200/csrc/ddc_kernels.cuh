@@ -33,6 +33,7 @@
 
 #include <algorithm>
 #include <climits>
+#include <cmath>
 #include <vector>
 
 #include "ddc_median.cuh"
@@ -73,6 +74,48 @@ constexpr int TS_SCAN = 11, TS_ROWS = 15, TS_LABEL = 17, TS_XLEV = 20, TS_YLEV =
 struct NaiveParams { // Grid.cpp:150-166
     int np0, np1, lx, ly;
 };
+inline NaiveParams naive_params(int P, int NX, int NY)
+{
+    // Grid.cpp:18-35 (find_factors) and Grid.cpp:153-155 (float ceil)
+    int fa = -1, fb = -1;
+    for (int i = 2; i * i <= P; i += 2)
+        if (P % i == 0) {
+            fa = i;
+            fb = P / fa;
+        }
+    NaiveParams nv;
+    if (fa == -1 || fb == -1) {
+        nv.np0 = P;
+        nv.np1 = 1;
+    } else {
+        nv.np0 = fa;
+        nv.np1 = fb;
+    }
+    nv.lx = (int)std::ceil((float)NX / (float)nv.np0);
+    nv.ly = (int)std::ceil((float)NY / (float)nv.np1);
+    return nv;
+}
+
+// The numbers of x / y levels depend on the bounding box of the dots, i.e. on the data, and they
+// size the launches after K2 (strip count, row-count buffers, the all-gather).  Instead of reading
+// the plan back in the middle of the pipeline, the host ASSUMES a plan -- the one of the previous
+// call on the same geometry, else the one of a full-extent bounding box -- K2 compares it with the
+// real one, and on a mismatch every later kernel does nothing; the step is then run again with the
+// real plan (validate() in ddc_api.cu, at the end of ddc_partition or, with DDC_ASYNC, in the first getter).
+inline void guess_plan(int P, int NX, int NY, int* ix, int* iy)
+{
+    double wx = (double)(NX - 1), wy = (double)(NY - 1);
+    *ix = *iy = 0;
+    for (int t = P; t > 1; t = (t + 1) / 2) {
+        if (wx > wy) {
+            (*ix)++;
+            wx /= 2.0;
+        } else {
+            (*iy)++;
+            wy /= 2.0;
+        }
+    }
+}
 
 // ------------------------------------------------------------------------------------------------
 // multi-GPU exchange over peer memory (NVLink / NVSwitch)
@@ -1107,10 +1150,9 @@ __device__ inline const RcbNode* rcb_levels(const Hist& H, RcbSet root, int leve
 }
 
 // threads that share one leaf's walk: the largest power of two <= 32 with lanes * leaves <= threads
-__device__ int g_walk_lanes = 32; // upper bound (tuning knob, set by the host)
 __device__ __forceinline__ int walk_lanes(int leaves, int threads)
 {
-    int lanes = g_walk_lanes;
+    int lanes = 32;
     while (lanes > 1 && (long long)lanes * leaves > threads)
         lanes >>= 1;
     return lanes;
@@ -1261,7 +1303,7 @@ __global__ void __launch_bounds__(1024) k_xcuts(PeerCols pc, PeerSync ps, int NX
     DevScalars* sc, unsigned* own_col /* this rank's column counts: reset here once they are consumed */,
     int dbg, Plan* host_plan, int presummed /* k_sum_cols ran: pc is ONE buffer of global counts */,
     int reset_own /* put this rank's column counts back to zero here (else: the labelling kernel does it) */,
-    ChainWord prev /* published by k_sum_cols */, ChainWord next /* polled by the row-count kernel */)
+    ChainWord prev /* published by k_sum_cols */)
 {
     DDC_DYN_SHARED(unsigned, smem_dyn);
     __shared__ unsigned wsum[PFX_WS];
@@ -1274,9 +1316,6 @@ __global__ void __launch_bounds__(1024) k_xcuts(PeerCols pc, PeerSync ps, int NX
     chain_wait(prev); // the mask scan (and k_sum_cols) is complete
     if (presummed && plan->mismatch == 3) { // a rank did not show up
         publish_plan(plan, host_plan);
-        __syncthreads();
-        if (tid == 0)
-            chain_signal(next);
         return;
     }
     if (tid == 0) {
@@ -1436,11 +1475,6 @@ __global__ void __launch_bounds__(1024) k_xcuts(PeerCols pc, PeerSync ps, int NX
         __syncthreads(); //   the host reads the real plan from its pinned copy and runs the step again
         publish_plan(plan, host_plan);
     }
-    if (next.word) { // strip table, leaf boxes and plan are written: the row-count kernel's blocks may go
-        __syncthreads();
-        if (tid == 0)
-            chain_signal(next);
-    }
 }
 
 // strip of every column (read by the labelling kernel), for decompositions WITHOUT y levels; with y levels K4
@@ -1570,13 +1604,13 @@ template <typename CT /* uint16_t when NX < 65536, else unsigned */>
 __global__ void __launch_bounds__(256) k_strip_rows(const uint8_t* __restrict__ bits, int NB, int rows,
     const int* __restrict__ st_x0, const int* __restrict__ st_x1, const int* __restrict__ st_p0,
     const Plan* __restrict__ plan, int Scap, PeerPush out, int Rmax, PeerSync ps, unsigned* __restrict__ done,
-    unsigned long long* dbg, ChainWord prev /* published by the x-cut block */)
+    unsigned long long* dbg)
 {
     __shared__ int s_last;
     pdl_trigger();
     if (threadIdx.x == 0)
         stamp_first(dbg, TS_RES + 2);
-    chain_wait(prev);
+    pdl_wait(); // the x-cut kernel is complete
     if (plan->mismatch) { // (the flag is raised all the same: the y-cut kernel may wait for it before it looks at the plan)
         rows_pushed(ps, done, gridDim.x * gridDim.y, &s_last);
         return;
@@ -1623,20 +1657,17 @@ __host__ __device__ inline size_t strip_scan_smem_words(int NG, int S, int K)
 {
     return (size_t)(NG + 1) + (size_t)(S + 1) + 8 * (size_t)K * (size_t)((S + 1) | 1);
 }
-// FULL (K == 1, rows of at most 8 chunks = 32768 columns): a lane requests ALL chunks of its row before
-// the boundary table is built, so that a block pays the memory latency once.
-template <typename CT, int K, bool FULL>
+template <typename CT, int K>
 __global__ void __launch_bounds__(256) k_strip_rows_scan(const uint8_t* __restrict__ bits, int NB, int NX, int rows,
     const int* __restrict__ st_x0, const int* __restrict__ st_p0, const Plan* __restrict__ plan, int Scap,
-    PeerPush out, int Rmax, PeerSync ps, unsigned* __restrict__ done, unsigned long long* dbg,
-    ChainWord prev /* published by the x-cut block */)
+    PeerPush out, int Rmax, PeerSync ps, unsigned* __restrict__ done, unsigned long long* dbg)
 {
     DDC_DYN_SHARED(int, sm_scan);
     __shared__ int s_last;
     pdl_trigger();
     if (threadIdx.x == 0)
         stamp_first(dbg, TS_RES + 2);
-    chain_wait(prev);
+    pdl_wait(); // the x-cut kernel is complete
     if (plan->mismatch) { // (the flag is raised all the same: the y-cut kernel may wait for it before it looks at the plan)
         if (ps.enabled && ps.rowflag[0])
             row_flags_raise(ps);
@@ -1646,10 +1677,8 @@ __global__ void __launch_bounds__(256) k_strip_rows_scan(const uint8_t* __restri
     }
     if (threadIdx.x == 0)
         stamp_first(dbg, TS_ROWS);
-    static_assert(!FULL || K == 1, "FULL holds one row per warp in registers");
     constexpr int RB = 8 * K; // rows per block
     constexpr int KP = (K + 1) / 2; // packed scan registers (two 16-bit running sums each)
-    constexpr int NCH = FULL ? 8 : 1; // chunks held in registers
     const int S = min(plan->S, Scap);
     const int NG = NB >> 4;
     const int PS = (S + 1) | 1;
@@ -1663,7 +1692,7 @@ __global__ void __launch_bounds__(256) k_strip_rows_scan(const uint8_t* __restri
     const uint4* rp[K];
     bool live[K];
     unsigned carry[K];
-    uint4 nxt[K], all[NCH];
+    uint4 nxt[K];
 #pragma unroll
     for (int k = 0; k < K; k++) {
         const int row = r_base + warp + 8 * k;
@@ -1671,16 +1700,8 @@ __global__ void __launch_bounds__(256) k_strip_rows_scan(const uint8_t* __restri
         rp[k] = reinterpret_cast<const uint4*>(bits + (size_t)(live[k] ? row : 0) * NB);
         carry[k] = 0u;
         nxt[k] = make_uint4(0u, 0u, 0u, 0u);
-        if (!FULL && live[k] && lane < NG)
+        if (live[k] && lane < NG)
             nxt[k] = __ldg(rp[k] + lane);
-    }
-    if (FULL) {
-#pragma unroll
-        for (int c = 0; c < NCH; c++) {
-            all[c] = make_uint4(0u, 0u, 0u, 0u);
-            if (live[0] && c * 32 + lane < NG)
-                all[c] = __ldg(rp[0] + c * 32 + lane);
-        }
     }
     for (int b = tid; b <= S; b += blockDim.x)
         xb[b] = b < S ? (st_x0[b] | (st_p0[b + 1] - st_p0[b] <= 1 ? (int)0x80000000 : 0)) : NX;
@@ -1700,25 +1721,18 @@ __global__ void __launch_bounds__(256) k_strip_rows_scan(const uint8_t* __restri
     __syncthreads();
     // The per-group popcounts (<= 128, their running sums over a chunk <= 4096) are scanned two to a register.
     const int nchunks = (NG + 31) >> 5;
-#pragma unroll(FULL ? NCH : 1)
-    for (int ch = 0; ch < (FULL ? NCH : nchunks); ch++) {
-        const int g0 = ch * 32;
-        if (FULL && g0 >= NG)
-            break;
-        const int g = g0 + lane;
+#pragma unroll 1
+    for (int ch = 0; ch < nchunks; ch++) {
+        const int g = ch * 32 + lane;
         const bool in = g < NG;
         unsigned long long wl[K], wh[K]; // columns 0-63 and 64-127 of my group, per row
 #pragma unroll
         for (int k = 0; k < K; k++) {
-            if (FULL)
-                nxt[k] = all[ch % NCH];
             wl[k] = (unsigned long long)nxt[k].x | ((unsigned long long)nxt[k].y << 32);
             wh[k] = (unsigned long long)nxt[k].z | ((unsigned long long)nxt[k].w << 32);
-            if (!FULL) {
-                nxt[k] = make_uint4(0u, 0u, 0u, 0u);
-                if (live[k] && g + 32 < NG)
-                    nxt[k] = __ldg(rp[k] + g + 32);
-            }
+            nxt[k] = make_uint4(0u, 0u, 0u, 0u);
+            if (live[k] && g + 32 < NG)
+                nxt[k] = __ldg(rp[k] + g + 32);
         }
         unsigned pc[K], ip[KP];
 #pragma unroll
@@ -1901,35 +1915,14 @@ template <typename CT, bool SMEM>
 __global__ void __launch_bounds__(1024) k_ycuts(PeerRows pr, PeerSync ps, RowLayout rl, int NY, StripTable st,
     unsigned* pfx_g, BoxTable bx, long long* loads, long long* loadmm, Plan* plan, int* __restrict__ strip_of_col,
     int dbg, BoxGate gate, int* __restrict__ part_at /* [S][nchunk]: the part of a strip owning row 32 j (PartAt) */,
-    int nchunk, int early /* the flags of exchange step 2 stand in for the completion of the row-count kernel */)
+    int nchunk)
 {
     DDC_DYN_SHARED(unsigned, smem_dyn);
     __shared__ unsigned wsum[PFX_WS];
     pdl_trigger(); // the labelling kernel may become resident
     if (dbg && blockIdx.x == 0 && threadIdx.x == 0)
         plan->ts[TS_RES + 3] = global_ns(); // (diagnostic only)
-    // Flags instead of a kernel boundary: a kernel that has stored into peer-mapped memory completes late -- the grid
-    // is only done once every posted NVLink store is acknowledged -- and its successor in the stream starts 6-8 us
-    // after its last block instead of 1.5 us.  This kernel needs nothing from that completion that the flags do not
-    // give: this rank's own flag is raised by the last block of ITS row-count kernel (release, cumulative over the
-    // block counter), which ran after the x-cut kernel had completed, so acquiring all G flags orders every input of
-    // this kernel before it.  (The blocks may then be resident, polling, while the row counts are still written.)
-    if (ps.enabled && early) {
-        bool ok = true;
-        unsigned seen;
-        if (ps.rowflag[0])
-            ok = row_flags_wait(ps);
-        else if (threadIdx.x < ps.G)
-            ok = peer_wait(ps, 1, &seen);
-        if (__syncthreads_or(!ok)) {
-            pdl_wait();
-            if (threadIdx.x == 0)
-                plan->mismatch = 3;
-            boxes_ready(gate);
-            return;
-        }
-    } else
-        pdl_wait(); // the strip row-count kernel (and with it everything before) is complete
+    pdl_wait(); // the strip row-count kernel (and with it everything before) is complete
     // everything the block needs to know about its first strip is requested at once: one trip to L2 instead of a chain
     // of four (mismatch -> S -> p0 -> x0) in front of the row counts
     const int mism = plan->mismatch, S = *st.S, ylevels = plan->iy;
@@ -1952,7 +1945,7 @@ __global__ void __launch_bounds__(1024) k_ycuts(PeerRows pr, PeerSync ps, RowLay
             strip_of_col[x] = s;
     }
     // exchange step 2: every rank's strip row counts are written (the last block of its row-count kernel said so)
-    if (ps.enabled && !early) {
+    if (ps.enabled) {
         bool ok = true;
         unsigned seen;
         if (ps.rowflag[0])
@@ -2299,8 +2292,6 @@ struct LabelEnd {
     PartAt part_at; // the row -> part table K4 left (table == nullptr: none)
     unsigned* reset_col; // != nullptr: this rank's column-count slot, consumed by k_sum_cols: zeroed here for the next step
     int reset_n, yr_off;
-    ChainWord prev; // the gate word the last block of K4 writes (boxes_ready), polled instead of the kernel boundary
-    ChainWord nbr; // published by the neighbour kernels on the second stream: the step ends when they have, too
 };
 
 template <bool VEC, bool WRITE>
@@ -2313,7 +2304,7 @@ __global__ void __launch_bounds__(256, 5) k_label(const uint8_t* __restrict__ bi
     pdl_trigger(); // the next step's mask scan may become resident behind the last blocks of this grid
     if (threadIdx.x == 0)
         stamp_first(fin.dbg, TS_RES + 4);
-    chain_wait(fin.prev);
+    pdl_wait(); // the cut kernels are complete
     if (plan->mismatch) { // the host runs the step again with the real plan (or reports the time-out)
         if (fin.fuse && blockIdx.x == 0 && blockIdx.y == 0)
             publish_plan(plan, fin.host_plan);
@@ -2354,28 +2345,6 @@ __global__ void __launch_bounds__(256, 5) k_label(const uint8_t* __restrict__ bi
         sc->changes = changes;
         sc->changes_all = changes;
         plan->fixup = (changes || fin.P <= 1) ? 0 : (fin.ps.enabled ? 2 : 1);
-        // The neighbour tables are built beside this kernel on a second stream.  Instead of joining the streams with
-        // an event (a stream operation between this kernel and the next step's scan: no programmatic launch there,
-        // and ~2 us more per step), this block waits for the word their last block publishes: when this grid has
-        // completed, the whole step has.
-        if (fin.nbr.word) {
-#ifndef DDC_HOST_EMU
-            const unsigned long long t0 = global_ns();
-            for (;;) {
-                unsigned v;
-                asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(fin.nbr.word) : "memory");
-                if (v == fin.nbr.step)
-                    break;
-                if (global_ns() - t0 > PEER_TIMEOUT_NS) {
-                    plan->mismatch = 3;
-                    break;
-                }
-            }
-#else
-            if (*fin.nbr.word != fin.nbr.step)
-                plan->mismatch = 3;
-#endif
-        }
         stamp_last(fin.dbg, TS_LABEL + 2);
     }
     __syncthreads();
@@ -2473,10 +2442,7 @@ template <bool FILL>
 __global__ void __launch_bounds__(256) k_neighbours(BoxTable bx, int P, int NX, int NY, int px, int py,
     StripTable st, int* __restrict__ counts, const int* __restrict__ offsets,
     const int* __restrict__ totals, int cap, int* __restrict__ ids, int* __restrict__ halos,
-    int* __restrict__ starts, DevScalars* sc, const Plan* __restrict__ plan,
-    ChainWord tables_done /* FILL: published by the last block on every path (the labelling kernel's last block waits
-                             for it: no join of the two streams between two steps) */,
-    unsigned* __restrict__ done_ctr)
+    int* __restrict__ starts, DevScalars* sc, const Plan* __restrict__ plan)
 {
     // (the scan of the counts is launched programmatically behind the count kernel; the count and the fill kernel
     //  themselves follow their predecessors with plain launches: P / 8 blocks waiting behind the gate kernel would hold
@@ -2509,16 +2475,6 @@ __global__ void __launch_bounds__(256) k_neighbours(BoxTable bx, int P, int NX, 
             if (t < 8LL * Ppad)
                 neighbours_structured<FILL>(bx, P, NX, NY, px, py, st, (int)(t / Ppad), (int)(t % Ppad), counts,
                     offsets, cap, ids, halos, starts, sc);
-        }
-    }
-    if (FILL && tables_done.word) {
-        __syncthreads(); // the block's entries are written ...
-        if (threadIdx.x == 0) {
-            __threadfence(); // ... and visible to the device before the block is counted
-            if (atomicAdd(done_ctr, 1u) == gridDim.x - 1u) {
-                *done_ctr = 0u;
-                chain_signal(tables_done);
-            }
         }
     }
 }

@@ -98,12 +98,6 @@ inline cudaError_t cudaMemset(void* p, int v, size_t n)
     return cudaSuccess;
 }
 inline cudaError_t cudaMemsetAsync(void* p, int v, size_t n, cudaStream_t) { return cudaMemset(p, v, n); }
-template <typename T>
-inline cudaError_t cudaMemcpyToSymbol(T& symbol, const void* src, size_t n)
-{
-    std::memcpy(&symbol, src, n);
-    return cudaSuccess;
-}
 inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned)
 {
     *s = reinterpret_cast<cudaStream_t>(std::malloc(1));

@@ -12,7 +12,6 @@
 #include "ddc_kernels.cuh"
 
 #include <climits>
-#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -24,41 +23,6 @@ using cuda_emu::Dim3;
 
 namespace {
 std::string g_err;
-
-NaiveParams naive_params(int P, int NX, int NY) // ddc_api.cu: Grid.cpp:18-35, 153-155
-{
-    int fa = -1, fb = -1;
-    for (int i = 2; i * i <= P; i += 2)
-        if (P % i == 0) {
-            fa = i;
-            fb = P / fa;
-        }
-    NaiveParams nv;
-    if (fa == -1 || fb == -1) {
-        nv.np0 = P;
-        nv.np1 = 1;
-    } else {
-        nv.np0 = fa;
-        nv.np1 = fb;
-    }
-    nv.lx = (int)std::ceil((float)NX / (float)nv.np0);
-    nv.ly = (int)std::ceil((float)NY / (float)nv.np1);
-    return nv;
-}
-void guess_plan(int P, int NX, int NY, int* ix, int* iy)
-{
-    double wx = (double)(NX - 1), wy = (double)(NY - 1);
-    *ix = *iy = 0;
-    for (int t = P; t > 1; t = (t + 1) / 2) {
-        if (wx > wy) {
-            (*ix)++;
-            wx /= 2.0;
-        } else {
-            (*iy)++;
-            wy /= 2.0;
-        }
-    }
-}
 
 struct Rank {
     int rank = 0, y_begin = 0, rows = 0;
@@ -74,8 +38,7 @@ struct Rank {
     std::vector<int> nbr_counts, nbr_offsets, nbr_totals, nbr_ids, nbr_halos, nbr_starts;
     DevScalars sc {};
     unsigned gate_word = 0;
-    unsigned nbr_word = 0; // published by the fill kernel's last block, awaited by the labelling kernel's
-    unsigned chain_words[2] = { 0u, 0u }; // k_sum_cols -> K2, K2 -> K3 (ChainWord)
+    unsigned sum_word = 0; // k_sum_cols -> K2 (ChainWord)
     Plan plan {}, host_plan {};
 };
 
@@ -88,10 +51,9 @@ struct Rank {
     } while (0)
 
 struct Options {
-    int strip_k = 0; // 0 auto, 1 / 2 / 4 rows per warp, 8 whole row in registers
+    int strip_k = 0; // 0 auto, 1 / 2 / 4 rows per warp, 16 the kernel for boundary tables beyond shared memory
     int scan_rpc = 64; // rows per CTA of the mask scan
     int smem_limit = 232448; // bytes of dynamic shared memory a block may use (B200: 227 KB)
-    bool row_flags = true; // exchange step 2 with one flag per block of the row-count kernel (DDC_ROW_FLAGS)
     bool collectives = false; // G > 1: the NCCL fallback of ddc_api.cu (all-reduce / all-gather between the kernels,
                               // emulated by host loops) instead of the slot exchange inside the kernels
 };
@@ -114,7 +76,7 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
     const bool x_smem = xneed + 1024 <= (size_t)opt.smem_limit, y_smem = yneed + 1024 <= (size_t)opt.smem_limit;
     const int ygrid = std::max(1, std::min(Scap, 148 * 2));
     const int gridx = (NG + 7) / 8;
-    const int d_rows = gridx + 1, d_label = (gridx + 3) & ~1, d_ycuts = d_label + 2, d_sum = d_ycuts + 1, d_nbr = d_sum + 1, ndone = d_nbr + 1; // ddc_api.cu: the "last block" counters
+    const int d_rows = gridx + 1, d_label = (gridx + 3) & ~1, d_ycuts = d_label + 2, d_sum = d_ycuts + 1, ndone = d_sum + 1; // ddc_api.cu: the "last block" counters
     const NaiveParams nv = naive_params(P, NX, NY);
     const int nchunk = (NY + 31) / 32;
     const int par = (int)(step & 1u);
@@ -209,10 +171,9 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
         for (Rank& r : R)
             std::copy(sum.begin(), sum.end(), colslot(r, r.rank));
     }
-    // every other step polls words in place of the kernel boundaries, as DDC_EARLY does on the device
+    // odd steps poll flags / words in place of the kernel boundaries between k_sum_cols and K2, as a step with
+    // programmatic launches does on the device; even steps wait for the boundaries, as a DDC_PROFILE step does
     const bool chained = (step & 1u) != 0u;
-    const ChainWord w_none { nullptr, 0u };
-    auto w_strips_of = [&](Rank& r) { return chained && ycuts ? ChainWord { &r.chain_words[1], step } : w_none; };
     // ---- K2: x cuts ----
     for (Rank& r : R) {
         StripTable st;
@@ -225,8 +186,7 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
         for (int q = 0; q < G; q++)
             pc.col[q] = colslot(r, p2p ? q : r.rank);
         PeerSync ps = sync_of(r);
-        const ChainWord w_sum = chained && p2p ? ChainWord { &r.chain_words[0], step } : w_none;
-        const ChainWord w_strips = w_strips_of(r);
+        const ChainWord w_sum = chained && p2p ? ChainWord { &r.sum_word, step } : ChainWord { nullptr, 0u };
         if (p2p) { // the ranks' slots summed by a grid of blocks first (k_sum_cols), K2 reads one buffer
             r.colsum.assign((size_t)ncol + 4, 0xdeadbeefu);
             LAUNCH(Dim3(gridx), Dim3(256), 0,
@@ -239,11 +199,11 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
         if (x_smem)
             LAUNCH(Dim3(1), Dim3(1024), xneed,
                 k_xcuts<true>(pc, ps, NX, NY, P, nullptr, yr_off, G, aix, aiy, &r.plan, st, bx, r.loads.data(), r.loadmm.data(),
-                    &r.sc, colslot(r, r.rank), 0, &r.host_plan, p2p ? 1 : 0, (p2p && r.rows > 0) ? 0 : 1, w_sum, w_strips));
+                    &r.sc, colslot(r, r.rank), 0, &r.host_plan, p2p ? 1 : 0, (p2p && r.rows > 0) ? 0 : 1, w_sum));
         else
             LAUNCH(Dim3(1), Dim3(1024), LEVEL_NODES_BYTES,
                 k_xcuts<false>(pc, ps, NX, NY, P, r.colpfx.data(), yr_off, G, aix, aiy, &r.plan, st, bx, r.loads.data(),
-                    r.loadmm.data(), &r.sc, colslot(r, r.rank), 0, &r.host_plan, p2p ? 1 : 0, (p2p && r.rows > 0) ? 0 : 1, w_sum, w_strips));
+                    r.loadmm.data(), &r.sc, colslot(r, r.rank), 0, &r.host_plan, p2p ? 1 : 0, (p2p && r.rows > 0) ? 0 : 1, w_sum));
         if (!ycuts) // with y levels K4 paints the column -> strip table
             LAUNCH(Dim3(std::max(1, std::min((Scap + 7) / 8, 148 * 4))), Dim3(256), 0,
                 k_paint_strips(st, &r.plan, r.strip_of_col.data()));
@@ -269,40 +229,35 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
             PeerSync ps = sync_of(r);
             int K = Rmax >= 32 * 4 * 148 ? 4 : 2;
             if (opt.strip_k)
-                K = opt.strip_k == 8 ? 1 : opt.strip_k;
+                K = opt.strip_k;
             while (K > 1 && sizeof(int) * strip_scan_smem_words(NG, Scap, K) > 48 * 1024)
                 K >>= 1;
             const size_t scan_smem = sizeof(int) * strip_scan_smem_words(NG, Scap, K);
             if (scan_smem <= 48 * 1024 && opt.strip_k != 16) {
                 const Dim3 grid((Rmax + 8 * K - 1) / (8 * K));
                 rb_shift = K == 4 ? 5 : (K == 2 ? 4 : 3);
-                if (p2p && opt.row_flags) { // one flag per block instead of one per rank (row_flags_raise)
+                if (p2p && G <= 2) { // one flag per block instead of one per rank (row_flags_raise), as on 2 GPUs
                     row_blocks = (int)grid.x;
                     row_sync(ps);
                 }
-                const bool full = opt.strip_k == 8 && K == 1 && NG <= 256;
-#define SCAN(CT, KK, FF)                                                                           \
+#define SCAN(CT, KK)                                                                               \
     LAUNCH(grid, Dim3(256), scan_smem,                                                             \
-        (k_strip_rows_scan<CT, KK, FF>(r.bits.data(), NB, NX, r.rows, st.x0, st.p0, &r.plan, Scap, out, Rmax, ps,      \
-            r.done.data() + d_rows, nullptr, w_strips_of(r))))
+        (k_strip_rows_scan<CT, KK>(r.bits.data(), NB, NX, r.rows, st.x0, st.p0, &r.plan, Scap, out, Rmax, ps,          \
+            r.done.data() + d_rows, nullptr)))
                 if (narrow) {
                     if (K == 4)
-                        SCAN(uint16_t, 4, false);
+                        SCAN(uint16_t, 4);
                     else if (K == 2)
-                        SCAN(uint16_t, 2, false);
-                    else if (full)
-                        SCAN(uint16_t, 1, true);
+                        SCAN(uint16_t, 2);
                     else
-                        SCAN(uint16_t, 1, false);
+                        SCAN(uint16_t, 1);
                 } else {
                     if (K == 4)
-                        SCAN(unsigned, 4, false);
+                        SCAN(unsigned, 4);
                     else if (K == 2)
-                        SCAN(unsigned, 2, false);
-                    else if (full)
-                        SCAN(unsigned, 1, true);
+                        SCAN(unsigned, 2);
                     else
-                        SCAN(unsigned, 1, false);
+                        SCAN(unsigned, 1);
                 }
 #undef SCAN
             } else { // strip_k == 16: the kernel for boundary tables that do not fit shared memory
@@ -311,11 +266,11 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
                 if (narrow)
                     LAUNCH(grid, Dim3(256), 0,
                         k_strip_rows<uint16_t>(r.bits.data(), NB, r.rows, st.x0, st.x1, st.p0, &r.plan, Scap, out, Rmax, ps,
-                            r.done.data() + d_rows, nullptr, w_strips_of(r)));
+                            r.done.data() + d_rows, nullptr));
                 else
                     LAUNCH(grid, Dim3(256), 0,
                         k_strip_rows<unsigned>(r.bits.data(), NB, r.rows, st.x0, st.x1, st.p0, &r.plan, Scap, out, Rmax, ps,
-                            r.done.data() + d_rows, nullptr, w_strips_of(r)));
+                            r.done.data() + d_rows, nullptr));
             }
         }
         std::vector<std::vector<unsigned>> gathered;
@@ -349,7 +304,7 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
 #define YCUTS(CT, SM)                                                                              \
     LAUNCH(Dim3(ygrid), Dim3(1024), SM ? yneed : LEVEL_NODES_BYTES,                                                \
         (k_ycuts<CT, SM>(pr, ps, rl, NY, st, r.ypfx.data(), bx, r.loads.data(), r.loadmm.data(), &r.plan,                    \
-            r.strip_of_col.data(), 0, gate, r.part_at.data(), nchunk, p2p ? (int)(step & 1u) : 0)))
+            r.strip_of_col.data(), 0, gate, r.part_at.data(), nchunk)))
             if (narrow) {
                 if (y_smem)
                     YCUTS(uint16_t, true);
@@ -380,13 +335,12 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
             }
             LAUNCH(Dim3(ngrid), Dim3(256), 0,
                 k_neighbours<false>(bx, P, NX, NY, px, py, st, r.nbr_counts.data(), nullptr, nullptr, cap, nullptr, nullptr,
-                    nullptr, &r.sc, &r.plan, ChainWord { nullptr, 0u }, nullptr));
+                    nullptr, &r.sc, &r.plan));
             LAUNCH(Dim3(8), Dim3(1024), 0,
                 k_scan_counts(r.nbr_counts.data(), P, r.nbr_offsets.data(), r.nbr_totals.data(), &r.plan));
             LAUNCH(Dim3(ngrid), Dim3(256), 0,
                 k_neighbours<true>(bx, P, NX, NY, px, py, st, r.nbr_counts.data(), r.nbr_offsets.data(), r.nbr_totals.data(),
-                    cap, r.nbr_ids.data(), r.nbr_halos.data(), r.nbr_starts.data(), &r.sc, &r.plan,
-                    ChainWord { &r.nbr_word, step }, r.done.data() + d_nbr));
+                    cap, r.nbr_ids.data(), r.nbr_halos.data(), r.nbr_starts.data(), &r.sc, &r.plan));
         }
         if (r.rows > 0) {
             const bool vecp = (NX % 4 == 0) && (((uintptr_t)r.pid.data()) % 16 == 0);
@@ -404,10 +358,6 @@ bool run_step(std::vector<Rank>& R, int NX, int NY, int P, int px, int py, int a
             fin.reset_col = p2p ? colslot(r, r.rank) : nullptr;
             fin.reset_n = ncol;
             fin.yr_off = yr_off;
-            if (chained && ycuts)
-                fin.prev = ChainWord { &r.gate_word, step };
-            if (fin.fuse && want_nbr)
-                fin.nbr = ChainWord { &r.nbr_word, step };
             if (vecp)
                 LAUNCH(grid, Dim3(256), 0,
                     (k_label<true, true>(r.bits.data(), NX, r.rows, r.y_begin, NB, rpc, r.strip_of_col.data(), st.p0, bx.y0,
@@ -464,7 +414,7 @@ __attribute__((visibility("default"))) const char* emu_last_error(void) { return
 // boxes[P*4] = x0 y0 ex ey; pid[NY*NX]; nbr_counts[8*P]; nbr_flat[3][sum of list totals] = ids, halos, starts of
 // the eight lists one after the other (list l = periodic * 4 + edge), nbr_cap = entries available per array;
 // out[0..7] = changes, median iterations, n_ocean, strips, x levels, y levels, load min, load max.
-// strip_k: 0 auto; 1 / 2 / 4 / 8 as DDC_STRIP_K; 16: the non-streaming row-count kernel.
+// strip_k: 0 the product's choice; 1 / 2 / 4 rows per warp of the streaming row-count kernel; 16: the non-streaming one.
 // smem_limit: 0 = B200's 227 KB; smaller values force the global-memory prefix paths of the cut kernels.
 // Returns 0, or -1 (emu_last_error()).  Every rank must end with identical boxes and tables (checked).
 __attribute__((visibility("default"))) int emu_partition(const int32_t* mask, int NX, int NY, int P, int px, int py, int G,
@@ -481,7 +431,8 @@ __attribute__((visibility("default"))) int emu_partition(const int32_t* mask, in
         cuda_emu::set_schedule_seed(std::strtoull(e, nullptr, 10));
     else
         cuda_emu::set_schedule_seed(0);
-    if (G < 1 || G > MAX_PEERS || NX < 1 || NY < 1 || P < 1) {
+    if (G < 1 || G > MAX_PEERS || NX < 1 || NY < 1 || P < 1
+        || !(strip_k == 0 || strip_k == 1 || strip_k == 2 || strip_k == 4 || strip_k == 16)) {
         g_err = "bad arguments";
         return -1;
     }
@@ -492,8 +443,6 @@ __attribute__((visibility("default"))) int emu_partition(const int32_t* mask, in
     if (smem_limit > 0)
         opt.smem_limit = smem_limit;
     opt.collectives = std::getenv("DDC_EMU_COLLECTIVES") != nullptr;
-    if (const char* e = std::getenv("DDC_ROW_FLAGS"))
-        opt.row_flags = std::atoi(e) != 0;
     // the masks of the ranks: 16-byte aligned copies of their row blocks (like a cudaMalloc'ed shard)
     std::vector<Rank> R(G);
     std::vector<std::vector<int32_t>> shard(G);

@@ -125,13 +125,19 @@ def test_nothing_moved_reports_naive_blocks(handle, oracle, n, P):
     T.test_nothing_moved_reports_naive_blocks(handle, oracle, n, P)
 
 
-@pytest.mark.parametrize("k", [1, 2, 4, 8])
-def test_strip_row_kernel_variants(capi, oracle, k, monkeypatch):
-    monkeypatch.setenv("DDC_STRIP_K", str(k))
+@pytest.mark.parametrize("case", [(260, 100, 24, 0.45, 4, "K2"), (8, 19000, 6, 0.45, 4, "K4"), (4096, 8, 1025, 0.4, 7, "K1"),
+                                  (4096, 8, 2049, 0.4, 7, "k_strip_rows")],
+                         ids=lambda c: "%dx%d-P%d-%s" % (c[0], c[1], c[2], c[5]))
+def test_strip_row_kernel_variants(capi, oracle, case):
+    """test_gpu_parity.test_strip_row_kernel_variants with shapes the emulation runs in seconds: the same four kernels,
+    the K = 1 and k_strip_rows ones through 1024 and 2048 strips of few columns"""
+    nx, ny, P, land, seed, kernel = case
     h = capi.Handle(0)
     try:
-        m = capi.generate_mask_host(260, 100, 4, 0.45)
-        T.assert_same(T.run_gpu(h, m, 24, True, False), oracle.partition(m, 24, True, False, use_hist=True), "k=%d" % k)
+        m = capi.generate_mask_host(nx, ny, seed, land)
+        g = T.run_gpu(h, m, P, True, False)
+        T.assert_same(g, oracle.partition(m, P, True, False, use_hist=True), case)
+        assert T.strip_row_kernel(nx, ny, P, g["stats"]) == kernel, (case, g["stats"])
     finally:
         h.close()
 

@@ -257,17 +257,40 @@ def test_nothing_moved_reports_naive_blocks(handle, oracle, n, P):
         assert_same(run_gpu(handle, m, P, px, py), o, "all ocean n=%d P=%d" % (n, P))
 
 
-@pytest.mark.parametrize("k", [1, 2, 4, 8])
-def test_strip_row_kernel_variants(capi, oracle, k, monkeypatch):
-    """every variant of the strip row-count kernel (rows per warp 1 / 2 / 4, whole row in registers),
-    forced through the DDC_STRIP_K knob that ddc_create() reads"""
-    monkeypatch.setenv("DDC_STRIP_K", str(k))
+def strip_row_kernel(nx, ny, P, stats, ranks=1):
+    """the strip row-count kernel ddc_api.cu launches for a decomposition, from its shape and settled plan: the
+    streaming kernel with K rows per warp ("K4", "K2", "K1"), or "k_strip_rows" when even the K = 1 boundary table
+    exceeds 48 KiB of shared memory; None without y levels.  K is 4 for shards of at least 32 x 4 x 148 rows, else 2,
+    halved while the table of Scap = min(P, 2^x_levels) strips does not fit."""
+    if stats["n_ylev"] == 0 or P == 1:
+        return None
+    ng, scap, rmax = (nx + 127) // 128, min(P, 1 << stats["n_xlev"]), -(-ny // ranks)
+    assert stats["nstrips"] <= scap, (stats["nstrips"], scap)
+    table = lambda k: 4 * ((ng + 1) + (scap + 1) + 8 * k * ((scap + 1) | 1))  # bytes (strip_scan_smem_words)
+    k = 4 if rmax >= 32 * 4 * 148 else 2
+    while k > 1 and table(k) > 48 * 1024:
+        k //= 2
+    return "K%d" % k if table(k) <= 48 * 1024 else "k_strip_rows"
+
+
+# (nx, ny, P, land, seed, the strip row-count kernel the shape reaches)
+STRIP_ROW_CASES = [(1024, 768, 96, 0.45, 4, "K2"), (777, 1033, 37, 0.6, 9, "K2"), (4096, 515, 64, 0.5, 2, "K2"),
+                   (1500, 19000, 300, 0.45, 3, "K4"),  # >= 18944 rows
+                   (20000, 40, 1200, 0.4, 7, "K1"),  # 1024 strips: the K = 2 table exceeds 48 KiB
+                   (40000, 24, 2049, 0.4, 7, "k_strip_rows")]  # 2048 strips: so does the K = 1 table
+
+
+@pytest.mark.parametrize("case", STRIP_ROW_CASES, ids=lambda c: "%dx%d-P%d-%s" % (c[0], c[1], c[2], c[5]))
+def test_strip_row_kernel_variants(capi, oracle, case):
+    """every variant of the strip row-count kernel (rows per warp 1 / 2 / 4, and the kernel for boundary tables beyond
+    shared memory), reached through the shape of the decomposition"""
+    nx, ny, P, land, seed, kernel = case
     h = capi.Handle(0)
     try:
-        for (nx, ny, P, land, seed) in [(1024, 768, 96, 0.45, 4), (777, 1033, 37, 0.6, 9), (4096, 515, 64, 0.5, 2)]:
-            m = capi.generate_mask_host(nx, ny, seed, land)
-            assert_same(run_gpu(h, m, P, True, False), oracle.partition(m, P, True, False, use_hist=True),
-                        "k=%d %dx%d" % (k, nx, ny))
+        m = capi.generate_mask_host(nx, ny, seed, land)
+        g = run_gpu(h, m, P, True, False)
+        assert_same(g, oracle.partition(m, P, True, False, use_hist=True), case)
+        assert strip_row_kernel(nx, ny, P, g["stats"]) == kernel, (case, g["stats"])
     finally:
         h.close()
 

@@ -99,9 +99,9 @@ def test_row_sharded_ranks_exchange_through_their_slots(oracle, ranks):
         assert_same(d, oracle.partition(mask, P, px, py, use_hist=True), (mask.shape, P, ranks))
 
 
-@pytest.mark.parametrize("strip_k", [1, 2, 4, 8, 16])
+@pytest.mark.parametrize("strip_k", [1, 2, 4, 16])
 def test_strip_row_count_kernel_variants(oracle, strip_k):
-    """rows per warp 1 / 2 / 4, whole row in registers (8), and the kernel for tables beyond shared memory (16)"""
+    """rows per warp 1 / 2 / 4, and the kernel for tables beyond shared memory (16)"""
     from domain_decomp_b200 import capi
     mask = capi.generate_mask_host(300, 90, 11, 0.45)
     for ranks in (1, 2):
@@ -153,25 +153,22 @@ def test_column_counts_travel_as_data_and_flag_words(oracle):
         assert_same(d, oracle.partition(mask, P, True, False, use_hist=True), (nx, ny, P, ranks))
 
 
-def test_row_counts_with_one_flag_per_rank_or_per_block(oracle, monkeypatch):
-    """exchange step 2: the row-count kernel's last block raises one flag per rank (block counter), or every block
-    raises its own and the y-cut kernel polls ranks x blocks flags (DDC_ROW_FLAGS); both on 2 and 3 ranks, with more
-    row blocks than one y-cut block has threads to poll them in one go"""
+def test_row_counts_with_one_flag_per_rank_or_per_block(oracle):
+    """exchange step 2: on 2 ranks every block of the row-count kernel raises its own flag and the y-cut kernel polls
+    ranks x blocks flags, with more row blocks than one y-cut block has threads to poll them in one go; on 3 ranks
+    the kernel's last block raises one flag per rank (block counter)"""
     from domain_decomp_b200 import capi
     for nx, ny, P, ranks in ((70, 9000, 6, 2), (150, 301, 12, 3)):
         mask = capi.generate_mask_host(nx, ny, 11, 0.4)
         o = oracle.partition(mask, P, False, True, use_hist=True)
-        for mode in ("0", "1"):
-            monkeypatch.setenv("DDC_ROW_FLAGS", mode)
-            for strip_k in (0, 1):
-                d, _ = oracle.emu_partition(mask, P, False, True, ranks=ranks, strip_k=strip_k)
-                assert_same(d, o, (nx, ny, P, ranks, mode, strip_k))
-    monkeypatch.delenv("DDC_ROW_FLAGS")
+        for strip_k in (0, 1):
+            d, _ = oracle.emu_partition(mask, P, False, True, ranks=ranks, strip_k=strip_k)
+            assert_same(d, o, (nx, ny, P, ranks, strip_k))
 
 
 def test_random_multi_rank_cases(oracle, monkeypatch):
-    """random shapes, part counts, periodic flags, 2-8 ranks (ragged and empty shards included), both ways of flagging
-    the row counts, random block / thread schedules: boxes, pid, neighbour tables and `changes` equal the oracle's"""
+    """random shapes, part counts, periodic flags, 2-8 ranks (ragged and empty shards included), random block / thread
+    schedules: boxes, pid, neighbour tables and `changes` equal the oracle's"""
     import random
     from domain_decomp_b200 import capi
     rng = random.Random(20261018)
@@ -180,12 +177,10 @@ def test_random_multi_rank_cases(oracle, monkeypatch):
         P, ranks = rng.randint(2, 24), rng.choice([2, 3, 4, 5, 8])
         px, py = rng.random() < .5, rng.random() < .5
         monkeypatch.setenv("DDC_EMU_SCHED_SEED", str(rng.randint(1, 2 ** 40)))
-        monkeypatch.setenv("DDC_ROW_FLAGS", rng.choice(["0", "1"]))
         mask = capi.generate_mask_host(nx, ny, rng.randint(1, 99), rng.choice([0.2, 0.5, 0.8]))
         d, _ = oracle.emu_partition(mask, P, px, py, ranks=ranks, scan_rpc=rng.choice([8, 16, 64]))
         assert_same(d, oracle.partition(mask, P, px, py, use_hist=True), (nx, ny, P, ranks, px, py))
     monkeypatch.delenv("DDC_EMU_SCHED_SEED")
-    monkeypatch.delenv("DDC_ROW_FLAGS")
 
 
 def test_results_do_not_depend_on_the_schedule(oracle, monkeypatch):
